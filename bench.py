@@ -7,7 +7,7 @@ reference's NeRFRenderer.render_rays pipeline (rays -> slab test -> stratified s
 the refine losses and the backward pass to the camera pose and both latent codes (weights frozen: refine mode).
 N>1: object-parallel, every rank renders its own 16 objects (weak scaling, no collective on the data path).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16|fp32]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16|fp32] [--dump-outputs DIR]
 
 `value`   : rays/s with every input already resident in HBM (device tensors in, loss stays on device).
 `e2e`     : the same through the public drop-in API NeRFRenderer.render_rays with HOST inputs (pinned img / mask /
@@ -118,6 +118,20 @@ def make_objects(seed0, n_obj, im_sz):
     return objs
 
 
+# what one step of the timed path hands its caller, per object, with the shape each is written in by --dump-outputs
+OUTPUTS = {"rgb": (N_OBJ, -1, 3), "depth": (N_OBJ, -1), "acc": (N_OBJ, -1), "loss": (N_OBJ,), "cam_pose_grad": (N_OBJ, 3, 4),
+           "shapecode_grad": (N_OBJ, -1), "texturecode_grad": (N_OBJ, -1)}
+
+
+def dump_outputs(path, last):
+    """DIR/<name>.npy (float32) for every output of the last timed step: 16 objects x 128 x 128 rays, 5.3 MB in all."""
+    os.makedirs(path, exist_ok=True)
+    for name, shape in OUTPUTS.items():
+        t = last[name]
+        t = torch.stack(t) if isinstance(t, list) else t
+        np.save(os.path.join(path, name + ".npy"), t.detach().reshape(shape).float().cpu().numpy())
+
+
 def refine_loss(rgb, acc, tgt, occ):
     """optimizer_nuscenes.py:729-736"""
     den = torch.sum(torch.abs(occ)) + 1e-9
@@ -200,6 +214,8 @@ def run_ours(args):
         h_shp = torch.cat([o["shapecode"] for o in objs]).pin_memory()
         h_tex = torch.cat([o["texturecode"] for o in objs]).pin_memory()
 
+    last = {}   # what the latest step_resident() handed its caller (written by --dump-outputs)
+
     def step_resident():
         """One pass over the batch through the public API with every input already resident in HBM; the losses and their backward
         to the poses + latents close the step."""
@@ -208,8 +224,10 @@ def run_ours(args):
             rgb, dep, acc = R.render_batch(model, batch, cams, shps, texs, fused_sampler=args.fused_sampler)
             loss, parts = snb.losses.refine_loss_batch(rgb, acc, batch.rgb_tgt, batch.occ_pixels, 0.1)
             loss.backward(gradient=ones_b)     # every object's own loss, upstream gradient 1 each
+            last.update(zip(OUTPUTS, (rgb, dep, acc, loss, cams.grad, shps.grad, texs.grad)))
             return parts
         fork()
+        outs = []
         for i, d in enumerate(dobjs):
             with torch.cuda.stream(streams[i % len(streams)]):
                 d["cam"].grad = d["shp"].grad = d["tex"].grad = None
@@ -217,7 +235,9 @@ def run_ours(args):
                                                         d["tex"], im_sz=IM_SZ)
                 loss = snb.losses.refine_loss(rgb, acc, tgt, occ, 0.1)[0]
                 loss.backward()
+                outs.append((rgb, dep, acc, loss, d["cam"].grad, d["shp"].grad, d["tex"].grad))
         join()
+        last.update(zip(OUTPUTS, (list(o) for o in zip(*outs))))
         return loss
 
     # pinned result buffers: per object the loss (1) + d cam_pose (12) + d shapecode (256) + d texturecode (256)
@@ -286,11 +306,16 @@ def run_ours(args):
 
     for _ in range(max(args.warmup, 3)):
         step_resident()
+    # the stratified-sampling jitter comes from the device generator: seeded here, the timed steps see the same jitter in every run
+    # with the same --steps, whatever ran before them
+    torch.cuda.manual_seed(0)
     launches0 = lib.snb_launch_count()
     with ClockSampler(local) as clk:
         ms_total = timed(step_resident, args.steps)
     launches = lib.snb_launch_count() - launches0
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     # Kernel-only pass for the roofline: the SAME step on ONE stream with CUDA events on the launch stream around the tcgen05
     # kernels alone.  (With several streams an event pair also spans the time a decoder kernel queues behind another stream's
     # decoder kernel -- the SMs hold one decoder CTA each -- so the multi-stream pass above is timed without them.)
@@ -1039,7 +1064,7 @@ def gpu_eager_baseline(dev, steps=3, warmup=2):
 def run_reference(args):
     if int(os.environ.get("RANK", 0)) != 0:
         return
-    steps, warmup = max(1, min(args.steps, 8)), max(1, min(args.warmup, 2))
+    steps, warmup = args.steps, args.warmup
     t0 = time.perf_counter()
     cpu = cpu_baseline(steps=steps, warmup=warmup)
     wall = time.perf_counter() - t0
@@ -1077,7 +1102,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary measurements (dense rows, fp32 mode, CPU / eager-CUDA reference baselines)")
     ap.add_argument("--skip-modes", action="store_true", help="skip the configs[3] / configs[4] collective-bearing modes")
     ap.add_argument("--streams", type=int, default=3, help="CUDA streams the independent objects alternate over (1 = one stream)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rendered rgb / depth / acc, losses, pose and code gradients) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

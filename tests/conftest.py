@@ -25,9 +25,32 @@ def pytest_collection_modifyitems(config, items):
             item.add_marker(skip)
 
 
+class Sampled:
+    """A golden array stored as every `stride`-th element of its flattened form (tools/make_golden.py samples the large gradient
+    arrays so that each fixture stays under 1 MB).  `absmax` is max|.| over the whole array."""
+
+    def __init__(self, values, shape, stride, absmax):
+        self.values, self.shape, self.stride, self.absmax = values, tuple(int(s) for s in shape), int(stride), float(absmax)
+
+    def take(self, t):
+        """The elements of a whole array `t` (of this array's shape) at the stored positions, as float64."""
+        t = torch.as_tensor(t).detach().double().cpu()
+        assert tuple(t.shape) == self.shape, (tuple(t.shape), self.shape)
+        return t.reshape(-1)[::self.stride]
+
+    def like(self, t):
+        """A whole array `t` reduced to the same positions."""
+        t = torch.as_tensor(t).detach().double().cpu()
+        return Sampled(self.take(t).numpy(), self.shape, self.stride, t.abs().max().item())
+
+
 def load_golden(name):
     z = np.load(os.path.join(GOLDEN, name + ".npz"))
-    return {k: z[k] for k in z.files}
+    g = {k: z[k] for k in z.files if "@" not in k}
+    for k in g:
+        if k + "@stride" in z.files:
+            g[k] = Sampled(g[k], z[k + "@shape"], z[k + "@stride"], z[k + "@absmax"])
+    return g
 
 
 def T(a, dtype=None, device=None):
@@ -40,7 +63,14 @@ def T(a, dtype=None, device=None):
 
 
 def rel_err(a, b):
-    """per-tensor max|a-b| / max|b|  (the metric SURVEY §8(d) fixes for every float comparison)."""
+    """per-tensor max|a-b| / max|b|  (the metric SURVEY §8(d) fixes for every float comparison).  With a `Sampled` golden on either
+    side the maximum runs over its stored elements; the denominator stays max|b| over the whole array."""
+    if isinstance(a, Sampled) or isinstance(b, Sampled):
+        s = a if isinstance(a, Sampled) else b
+        a, b = (x if isinstance(x, Sampled) else s.like(x) for x in (a, b))
+        assert (a.shape, a.stride) == (b.shape, b.stride)
+        d = np.abs(a.values.astype(np.float64) - b.values.astype(np.float64)).max()
+        return float(d) / (b.absmax if b.absmax > 0 else 1.0)
     a = torch.as_tensor(a).detach().double().cpu()
     b = torch.as_tensor(b).detach().double().cpu()
     den = b.abs().max().item()
@@ -53,6 +83,7 @@ def close_vs_truth(got, ref32, truth64, tol=1e-5, slack=None, name=None):
     `ref32` the fp32 reference (golden or fp32 oracle).  Pass iff the kernel is within `tol` of the fp32 reference, or within
     `tol` of the truth, or no further from it than `slack` x the fp32 reference's own distance.  Recorded in the parity ledger.
     Returns (ok, err_got_vs_truth, err_ref_vs_truth)."""
+    truth64 = _on_golden_elements(ref32, truth64)
     e_got = rel_err(got, truth64)
     e_ref = rel_err(ref32, truth64)
     try:
@@ -61,6 +92,14 @@ def close_vs_truth(got, ref32, truth64, tol=1e-5, slack=None, name=None):
     except AssertionError:
         ok = False
     return ok, e_got, e_ref
+
+
+def _on_golden_elements(ref, truth):
+    """A whole `truth` against a `Sampled` reference is reduced to the reference's stored elements, so that the kernel, the
+    reference and the truth are judged on the same elements."""
+    if isinstance(ref, Sampled) and truth is not None and not isinstance(truth, Sampled):
+        return ref.like(truth)
+    return truth
 
 
 _AUTO = {}
@@ -123,6 +162,7 @@ def parity(name, got, ref, tol, truth=None, slack=TRUTH_SLACK, rows=None, floor=
       orders and never come back -- the loss does not see it.  The error over ALL elements is recorded as `err_all_elements`.
     Returns the error that decided (so a test can print it)."""
     import json
+    truth = _on_golden_elements(ref, truth)
     e = rel_err(got, ref)
     rec = {"test": _current_test(), "tensor": name, "tol": tol, "err_vs_ref": e}
     if outliers > 0:

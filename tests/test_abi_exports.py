@@ -130,6 +130,9 @@ def test_reference_checkpoints_load_strict_and_round_trip():
         snb.CodeNeRF().load_state_dict({"bogus.weight": torch.zeros(1)})
 
 
+SHIPPED_CODE = (".py", ".sh", ".cu", ".cuh", ".h", ".hpp", ".c", ".cc", ".cpp", ".so", ".o", ".a", ".cubin", ".fatbin", ".ptx")
+
+
 def test_shipped_artefacts_do_not_name_batch_memcpy_entry_points():
     """ADVICE r1: a statically linked CUDA runtime embeds the names of every runtime entry point, including the batched memcpy
     calls the GPU pool refuses.  The library links the shared runtime; no binary that travels to the GPU box may carry the names."""
@@ -138,8 +141,24 @@ def test_shipped_artefacts_do_not_name_batch_memcpy_entry_points():
     from supnerf_b200.build import build
     build()
     banned = re.compile(rb"cu(da)?Memcpy(3D)?BatchAsync")
-    tracked = subprocess.run(["git", "ls-files"], cwd=ROOT, capture_output=True, text=True).stdout.split()
-    paths = [_lib.LIB_PATH] + [os.path.join(ROOT, p) for p in tracked]
+    try:
+        r = subprocess.run(["git", "ls-files", "-z"], cwd=ROOT, capture_output=True, text=True)
+        tracked = [os.path.join(ROOT, p) for p in r.stdout.split("\0") if p] if r.returncode == 0 else None
+    except OSError:
+        tracked = None
+    if tracked is None:   # a copy of the tree without git metadata: its source and script files and built binaries (notes, logs and
+        tracked = []      # data may quote the names)
+        for d, dirs, files in os.walk(ROOT):
+            dirs[:] = [x for x in dirs if not x.startswith(".") and x != "__pycache__"]
+            for f in files:
+                p = os.path.join(d, f)
+                if f.endswith(SHIPPED_CODE):
+                    tracked.append(p)
+                elif os.path.isfile(p):
+                    with open(p, "rb") as fh:
+                        if fh.read(4) == b"\x7fELF":   # executables built without a suffix (tools/ubench)
+                            tracked.append(p)
+    paths = [_lib.LIB_PATH] + tracked
     for p in paths:
         if not os.path.isfile(p) or p.endswith("test_abi_exports.py") or os.path.basename(p) in ("ADVICE.md", "VERDICT.md"):
             continue

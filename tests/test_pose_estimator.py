@@ -1,6 +1,8 @@
 """SURVEY 8f rank 2, the pose-estimator forward: supnerf_b200.pose_estimator / SUPNeRF.encode_img / pose_update against outputs of the
 UNMODIFIED reference (tests/golden/pose_estimator.npz, tools/make_golden.py:golden_pose_estimator).  The encoder is plain torch
-(cuDNN / CPU convolutions): its tests run on the CPU too; the joint training step needs the decoder kernels (-m gpu)."""
+(cuDNN / CPU convolutions): its tests run on the CPU too; the joint training step needs the decoder kernels (-m gpu).
+The image and weight gradients of the fixture are stored as a strided sample of 1/2 .. 1/17 of their elements (conftest.Sampled):
+they are judged on those elements, against max|.| of the whole array."""
 import numpy as np
 import pytest
 import torch

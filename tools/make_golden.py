@@ -10,6 +10,7 @@ against them; the -m gpu tests pin the CUDA kernels against the same files.
 Usage: python tools/make_golden.py            (rewrites tests/golden/*.npz)
 """
 import hashlib
+import math
 import os
 import sys
 import types
@@ -33,6 +34,8 @@ import utils as ref_utils  # noqa: E402
 
 from oracle import oracle  # noqa: E402
 
+SAMPLE_MAX = 8192   # arrays save() samples keep at most this many elements: every fixture stays under 1 MB
+
 
 def state_hash(sd):
     h = hashlib.sha256()
@@ -46,10 +49,31 @@ def npy(t):
     return t.detach().cpu().numpy() if isinstance(t, torch.Tensor) else np.asarray(t)
 
 
-def save(name, **arrs):
+def sample_stride(a):
+    """Smallest stride that keeps at most SAMPLE_MAX elements of the flattened array and is coprime with its last dimension, so
+    that the sample visits every row and every column."""
+    s = -(-a.size // SAMPLE_MAX)
+    while math.gcd(s, a.shape[-1]) != 1:
+        s += 1
+    return s
+
+
+def save(name, sample=(), **arrs):
+    """Arrays whose key starts with a prefix in `sample` and that hold more than SAMPLE_MAX elements are stored as every
+    sample_stride()-th element of their flattened form, beside their shape, the stride and max|.| of the whole array
+    (tests/conftest.py:load_golden reads them back as `Sampled`)."""
     os.makedirs(OUT, exist_ok=True)
     path = os.path.join(OUT, name + ".npz")
-    np.savez_compressed(path, **{k: npy(v) for k, v in arrs.items()})
+    out = {}
+    for k, v in arrs.items():
+        a = npy(v)
+        if k.startswith(tuple(sample)) and a.size > SAMPLE_MAX:
+            s = sample_stride(a)
+            out.update({k: a.reshape(-1)[::s].copy(), k + "@shape": np.asarray(a.shape, np.int64), k + "@stride": np.int64(s),
+                        k + "@absmax": np.float64(np.abs(a.astype(np.float64)).max())})
+        else:
+            out[k] = a
+    np.savez_compressed(path, **out)
     print(f"wrote {path}  ({os.path.getsize(path) / 1024:.1f} KiB)")
 
 
@@ -181,7 +205,7 @@ def golden_render_box():
     torch.manual_seed(100)
     xyz, vdr, zv, hit = r.prepare_sampled_rays(ro, vd, obj["wlh"])
     g = {k: p.grad for k, p in model.named_parameters()}
-    save("render_box_c1",
+    save("render_box_c1", sample=("gw_",),
          seed=seed, im_sz=im_sz, n_samples=S, weights_sha256=np.frombuffer(state_hash(sd).encode(), dtype=np.uint8),
          K=obj["K"], cam_pose=obj["cam_pose"], wlh=obj["wlh"], roi=obj["roi"], img=obj["img"], mask_occ=obj["mask_occ"],
          shapecode=shp, texturecode=tex, jitter=jitter,
@@ -241,7 +265,7 @@ def golden_decoder_batch():
     occ = torch.sign(torch.randn(B, n, 1, generator=g))
     loss = losses(rgb, acc, tgt, occ)
     loss.backward()
-    save("decoder_batch_c5",
+    save("decoder_batch_c5", sample=("gw_",),
          seed=seed, weights_sha256=np.frombuffer(state_hash(sd).encode(), dtype=np.uint8),
          xyz=xyz, viewdir=vd, z_vals=zv, shapecode=shp, texturecode=tex, rgb_tgt=tgt, occ_pixels=occ,
          sigmas=sig, rgbs=rgbs, rgb=rgb, depth=dep, acc=acc, loss=loss,
@@ -630,7 +654,7 @@ def golden_pose_estimator():
         torch.set_default_dtype(old_dt)
     for name in stubs:
         sys.modules.pop(name, None)
-    save("pose_estimator", **out)
+    save("pose_estimator", sample=("eval_g", "j_gw_", "j64_gw_"), **out)
 
 
 def golden_scene():
