@@ -10,7 +10,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(CSRC, "_build")
 LIB = os.path.join(HERE, "libsupnerf_b200.so")
-SOURCES = ["api.cu", "composite.cu", "sampler.cu", "latent.cu", "mlp_f32.cu", "mlp_tc.cu", "mlp_tc2.cu", "render.cu", "loss.cu",
+SOURCES = ["api.cu", "composite.cu", "sampler.cu", "latent.cu", "mlp_f32.cu", "mlp_tc.cu", "mlp_tc2.cu", "decoder.cu", "render.cu", "loss.cu",
            "compact.cu", "scene.cu", "refine.cu", "render_batch.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC"]  # no --use_fast_math: sinf/expf accuracy is part of parity

@@ -1,8 +1,7 @@
 // C-ABI entry points that are not tied to one kernel file: error text, device info, the per-model
-// handle and the precision dispatch of the decoder MLP.
+// handle, and the decoder MLP's entry points (argument checks; decoder.cu picks and runs the back end).
 #include "common.cuh"
-#include "handle.h"
-#include "rb_rows.cuh"
+#include "decoder.h"
 #include <stdarg.h>
 #include <string.h>
 #include <new>
@@ -30,24 +29,6 @@ int sm_count() {
   }
   return cached;
 }
-
-// bf16 / tcgen05 back end (mlp_tc.cu)
-size_t tc_packed_bytes(const snb_handle_s* h);
-int tc_pack_weights(snb_handle_s* h, void* packed, cudaStream_t st);
-void tc_timing_enable(snb_handle_s* h, int on);
-int tc_timing_read(snb_handle_s* h, int which, float* ms, int max_n);
-size_t tc_workspace_bytes(const snb_handle_s* h, int64_t M, int64_t B);
-size_t tc_bwd_scratch_bytes(const snb_handle_s* h, int64_t M, int64_t B);
-int tc_forward(const snb_handle_s* h, const float* xyz, const float* viewdir, int64_t M, int64_t B,
-               const float* shape_latent, const float* texture_latent, float* sigma, float* rgb, void* ws, cudaStream_t st, bool train,
-               const int64_t* m_dev, const int32_t* tile_start = nullptr, const rb::RowSrc* rs = nullptr, bool split = false);
-int tc_backward(const snb_handle_s* h, const float* xyz, const float* viewdir, int64_t M, int64_t B,
-                const float* shape_latent, const float* texture_latent, const float* sigma, const float* g_sigma,
-                const float* g_rgb, const void* ws, void* scratch, float* g_xyz, float* g_viewdir, float* g_shape_latent,
-                float* g_texture_latent, float* const* g_weights, cudaStream_t st, bool train, const int64_t* m_dev,
-                const int32_t* tile_start = nullptr, bool split = false);
-size_t tc_train_workspace_extra(const snb_handle_s* h, int64_t M);
-size_t tc_train_scratch_extra(const snb_handle_s* h, int64_t M);
 
 }  // namespace snb
 
@@ -141,18 +122,18 @@ extern "C" int snb_set_weights(snb_handle h, const float* const* tensors, int32_
 extern "C" int snb_tc_set_debug(snb_handle h, float* acts) { SNB_REQUIRE(h, "snb_tc_set_debug: null handle"); h->dbg_acts = acts; return 0; }
 extern "C" int snb_tc_set_trace(snb_handle h, long long* stamps) { SNB_REQUIRE(h, "snb_tc_set_trace: null handle"); h->trace = stamps; return 0; }
 extern "C" int snb_tc_set_cg2(snb_handle h, int32_t mode) { SNB_REQUIRE(h, "snb_tc_set_cg2: null handle"); h->cg2_mode = mode; return 0; }
-extern "C" int snb_kernel_timing_enable(snb_handle h, int32_t on) { SNB_REQUIRE(h, "snb_kernel_timing_enable: null handle"); tc_timing_enable(h, on); return 0; }
+extern "C" int snb_kernel_timing_enable(snb_handle h, int32_t on) { SNB_REQUIRE(h, "snb_kernel_timing_enable: null handle"); decoder_timing_enable(h, on); return 0; }
 extern "C" int snb_kernel_timing_read(snb_handle h, int32_t which, float* ms_host, int32_t max_n) {
   if (!h) return 0;
-  return tc_timing_read(h, which, ms_host, max_n);
+  return decoder_timing_read(h, which, ms_host, max_n);
 }
 
-extern "C" size_t snb_packed_bytes(snb_handle h) { return h ? tc_packed_bytes(h) : 0; }
+extern "C" size_t snb_packed_bytes(snb_handle h) { return h ? decoder_packed_bytes(h) : 0; }
 
 extern "C" int snb_pack_weights(snb_handle h, void* packed, void* stream) {
   SNB_REQUIRE(h && packed, "snb_pack_weights: null argument");
   SNB_REQUIRE(h->weights_set, "snb_pack_weights: call snb_set_weights first");
-  return tc_pack_weights(h, packed, (cudaStream_t)stream);
+  return decoder_pack_weights(h, packed, (cudaStream_t)stream);
 }
 
 static int check_mlp_args(snb_handle h, int32_t precision, int64_t M, int64_t B) {
@@ -166,17 +147,11 @@ static int check_mlp_args(snb_handle h, int32_t precision, int64_t M, int64_t B)
 }
 
 extern "C" size_t snb_mlp_workspace_bytes(snb_handle h, int64_t M, int64_t B, int32_t precision) {
-  if (!h) return 0;
-  if (precision == SNB_PREC_BF16 || precision == SNB_PREC_FP32_TC) return tc_workspace_bytes(h, M, B);
-  if (precision == SNB_PREC_BF16_TRAIN) return tc_workspace_bytes(h, M, B) + tc_train_workspace_extra(h, M);
-  return f32_workspace_floats(h, M, B) * sizeof(float);
+  return h ? decoder_workspace_bytes(h, precision, M, B) : 0;
 }
 
 extern "C" size_t snb_mlp_bwd_scratch_bytes(snb_handle h, int64_t M, int64_t B, int32_t precision) {
-  if (!h) return 0;
-  if (precision == SNB_PREC_BF16 || precision == SNB_PREC_FP32_TC) return tc_bwd_scratch_bytes(h, M, B);
-  if (precision == SNB_PREC_BF16_TRAIN) return tc_bwd_scratch_bytes(h, M, B) + tc_train_scratch_extra(h, M);
-  return f32_bwd_scratch_floats(h, M, B) * sizeof(float);
+  return h ? decoder_scratch_bytes(h, precision, M, B) : 0;
 }
 
 extern "C" int snb_mlp_fwd(snb_handle h, int32_t precision, const float* xyz, const float* viewdir, int64_t M, int64_t B,
@@ -185,10 +160,7 @@ extern "C" int snb_mlp_fwd(snb_handle h, int32_t precision, const float* xyz, co
   if (check_mlp_args(h, precision, M, B)) return 2;
   if (M == 0) return 0;
   SNB_REQUIRE(xyz && viewdir && shape_latent && texture_latent && sigma && rgb && workspace, "mlp_fwd: null pointer");
-  if (precision != SNB_PREC_FP32)
-    return tc_forward(h, xyz, viewdir, M, B, shape_latent, texture_latent, sigma, rgb, workspace, (cudaStream_t)stream,
-                      precision == SNB_PREC_BF16_TRAIN, nullptr, nullptr, nullptr, precision == SNB_PREC_FP32_TC);
-  return f32_forward(h, xyz, viewdir, M, B, shape_latent, texture_latent, sigma, rgb, (float*)workspace, (cudaStream_t)stream);
+  return decoder_forward(h, precision, xyz, viewdir, M, B, shape_latent, texture_latent, sigma, rgb, workspace, (cudaStream_t)stream);
 }
 
 extern "C" int snb_mlp_bwd(snb_handle h, int32_t precision, const float* xyz, const float* viewdir, int64_t M, int64_t B,
@@ -197,25 +169,11 @@ extern "C" int snb_mlp_bwd(snb_handle h, int32_t precision, const float* xyz, co
                            float* g_viewdir, float* g_shape_latent, float* g_texture_latent, float* const* g_weights,
                            void* stream) {
   if (check_mlp_args(h, precision, M, B)) return 2;
-  if (M == 0) {   // no samples: every gradient is zero
-    cudaStream_t st0 = (cudaStream_t)stream;
-    if (g_shape_latent) SNB_CHECK_CUDA(cudaMemsetAsync(g_shape_latent, 0, sizeof(float) * B * h->arch.latent_dim, st0));
-    if (g_texture_latent) SNB_CHECK_CUDA(cudaMemsetAsync(g_texture_latent, 0, sizeof(float) * B * h->arch.latent_dim, st0));
-    if (g_weights)
-      for (size_t i = 0; i < h->layers.size(); ++i) {
-        SNB_CHECK_CUDA(cudaMemsetAsync(g_weights[2 * i], 0, sizeof(float) * h->layers[i].out * h->layers[i].in, st0));
-        SNB_CHECK_CUDA(cudaMemsetAsync(g_weights[2 * i + 1], 0, sizeof(float) * h->layers[i].out, st0));
-      }
-    return 0;
-  }
+  if (M == 0) return decoder_zero_grads(h, B, g_shape_latent, g_texture_latent, g_weights, (cudaStream_t)stream);   // no samples
   SNB_REQUIRE(xyz && viewdir && shape_latent && texture_latent && sigma && g_sigma && g_rgb && workspace && scratch,
               "mlp_bwd: null pointer");
-  if (precision != SNB_PREC_FP32)
-    return tc_backward(h, xyz, viewdir, M, B, shape_latent, texture_latent, sigma, g_sigma, g_rgb, workspace, scratch, g_xyz,
-                       g_viewdir, g_shape_latent, g_texture_latent, g_weights, (cudaStream_t)stream,
-                       precision == SNB_PREC_BF16_TRAIN, nullptr, nullptr, precision == SNB_PREC_FP32_TC);
-  return f32_backward(h, xyz, viewdir, M, B, shape_latent, texture_latent, sigma, g_sigma, g_rgb, (const float*)workspace,
-                      (float*)scratch, g_xyz, g_viewdir, g_shape_latent, g_texture_latent, g_weights, (cudaStream_t)stream);
+  return decoder_backward(h, precision, xyz, viewdir, M, B, shape_latent, texture_latent, sigma, g_sigma, g_rgb, workspace, scratch,
+                          g_xyz, g_viewdir, g_shape_latent, g_texture_latent, g_weights, (cudaStream_t)stream);
 }
 
 // ---------------------------------------------------------------------------------------------------------------------

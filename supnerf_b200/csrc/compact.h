@@ -1,9 +1,7 @@
-// Miss-ray compaction helpers (compact.cu) and the internal tensor-core decoder entry points the fused render calls directly.
+// Miss-ray compaction helpers (compact.cu) and the box sampler's backward in compact row order.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include "handle.h"
-#include "rb_rows.cuh"
 
 namespace snb {
 
@@ -22,19 +20,5 @@ int sample_box_bwd_compact(const float* rays_o, const float* viewdir, const floa
                            int32_t n_samples, float half_diag, const float* h, const float* g_xyz_c, const float* g_vrep_c,
                            const float* g_z_vals, const int32_t* pos, const int64_t* counts, float* g_rays_o, float* g_viewdir,
                            cudaStream_t st);
-
-// mlp_tc.cu: m_dev (optional) = device-side number of rows actually present (a multiple of 128, <= M);
-// tile_start (optional, B + 1 device ints, ascending, even): object b owns the 128-row tiles [tile_start[b], tile_start[b+1]) -- the
-// batched render's objects own different numbers of rows (render_batch.cu)
-bool tc_two_tile_active(const snb_handle_s* h);
-bool tc_one_tile_supported(const snb_handle_s* h);   // the architecture the one-tile kernels (bf16 and split-precision) cover
-int tc_forward(const snb_handle_s* h, const float* xyz, const float* viewdir, int64_t M, int64_t B,
-               const float* shape_latent, const float* texture_latent, float* sigma, float* rgb, void* ws, cudaStream_t st, bool train,
-               const int64_t* m_dev, const int32_t* tile_start = nullptr, const rb::RowSrc* rs = nullptr, bool split = false);
-int tc_backward(const snb_handle_s* h, const float* xyz, const float* viewdir, int64_t M, int64_t B,
-                const float* shape_latent, const float* texture_latent, const float* sigma, const float* g_sigma,
-                const float* g_rgb, const void* ws, void* scratch, float* g_xyz, float* g_viewdir, float* g_shape_latent,
-                float* g_texture_latent, float* const* g_weights, cudaStream_t st, bool train, const int64_t* m_dev,
-                const int32_t* tile_start = nullptr, bool split = false);
 
 }  // namespace snb

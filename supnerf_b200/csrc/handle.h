@@ -11,6 +11,9 @@ struct snb_layer {
   int out = 0, in = 0;
 };
 
+// byte offsets of the two-tile and split-precision images behind the one-tile bf16 image at 0, and the buffer size (0: not built yet)
+struct snb_packed_layout { size_t two_tile = 0, split = 0, bytes = 0; };
+
 struct snb_handle_s {
   snb_arch arch;
   std::vector<snb_layer> layers;  // canonical (state_dict) order
@@ -19,8 +22,7 @@ struct snb_handle_s {
   const void* packed = nullptr;   // borrowed: caller-owned buffer filled by snb_pack_weights
   // per-handle caches of pure functions of the architecture (built on first use; a handle is used by one host thread at a time)
   mutable std::shared_ptr<void> tc2_programs;   // mlp_tc2.cu: the step programs of the two-tile kernels
-  mutable size_t v1_packed_bytes_cache = 0;     // mlp_tc.cu: size of the first-generation packed image
-  mutable size_t x3_packed_bytes_cache = 0;     // mlp_tc.cu: size of the split-precision (fp16 hi / lo) packed image
+  mutable snb_packed_layout packed_layout;      // decoder.cu: where each weight image sits in the packed buffer
   // test / tuning / measurement hooks, per handle (a handle is used by one host thread at a time; nothing here is process-global)
   float* dbg_acts = nullptr;                    // snb_tc_set_debug
   long long* trace = nullptr;                   // snb_tc_set_trace
@@ -36,36 +38,3 @@ struct snb_handle_s {
   int d_xyz() const { return 3 + 6 * arch.num_xyz_freq; }
   int d_dir() const { return 3 + 6 * arch.num_dir_freq; }
 };
-
-namespace snb {
-// fp32 back end (mlp_f32.cu)
-size_t f32_workspace_floats(const snb_handle_s* h, int64_t M, int64_t B);
-size_t f32_bwd_scratch_floats(const snb_handle_s* h, int64_t M, int64_t B);
-int f32_forward(const snb_handle_s* h, const float* xyz, const float* viewdir, int64_t M, int64_t B,
-                const float* shape_latent, const float* texture_latent, float* sigma, float* rgb, float* ws,
-                cudaStream_t st);
-int f32_backward(const snb_handle_s* h, const float* xyz, const float* viewdir, int64_t M, int64_t B,
-                 const float* shape_latent, const float* texture_latent, const float* sigma, const float* g_sigma,
-                 const float* g_rgb, const float* ws, float* scratch, float* g_xyz, float* g_viewdir,
-                 float* g_shape_latent, float* g_texture_latent, float* const* g_weights, cudaStream_t st);
-// per-object latent layers, shared by both back ends.  zlat / dz: [(Bs+Bt)][B][W] (shape slots first).
-int latent_forward(const snb_handle_s* h, int64_t B, const float* shape_latent, const float* texture_latent, float* zlat,
-                   cudaStream_t st);
-// ebias[slot][b][:] = bias + W z  of the layer that consumes latent slot `slot` (shape_layer_j / texture_layer_j): the
-// latent add folded through the layer, exact in fp32 (SURVEY 8(a')3).
-int latent_effective_bias(const snb_handle_s* h, int64_t B, const float* zlat, float* ebias, cudaStream_t st);
-// single-launch versions (latent.cu): forward of all slots (+ effective biases if ebias != NULL); backward to the latents only
-// eimg != NULL: also write every effective bias as a tcgen05 bias-stage row (32 B each, [(Bs+Bt)][B][W]; tc_ptx.cuh)
-int latent_forward_fused(const snb_handle_s* h, int64_t B, const float* shape_latent, const float* texture_latent, float* zlat,
-                         float* ebias, cudaStream_t st, uint8_t* eimg = nullptr);
-// fold_tmp != NULL: dz holds the column sums of the consuming layers' pre-activation gradients (two-tile tcgen05 backward);
-// they are first folded through W_layer^T into fold_tmp (same size as dz).
-int latent_backward_fused(const snb_handle_s* h, int64_t B, const float* zlat, const float* dz, float* g_shape_latent,
-                          float* g_texture_latent, cudaStream_t st, float* fold_tmp = nullptr);
-// dz[slot][b][i] = sum_o W_layer[o][i] s_lat[slot][b][o]  (the W^T fold of the two-tile backward's column sums)
-int latent_fold(const snb_handle_s* h, int64_t B, const float* s_lat, float* dz, cudaStream_t st);
-// dz holds d loss / d zlat (post-ReLU outputs) and is overwritten by the pre-activation gradient.
-int latent_backward(const snb_handle_s* h, int64_t B, const float* shape_latent, const float* texture_latent,
-                    const float* zlat, float* dz, float* g_shape_latent, float* g_texture_latent, float* const* g_weights,
-                    cudaStream_t st);
-}  // namespace snb

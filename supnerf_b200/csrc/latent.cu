@@ -4,7 +4,7 @@
 // that consumes z (the latent add folded through that layer, used by the tcgen05 back end).  One launch does
 // the backward (ReLU mask, then d latent = sum_slots W_lat^T d_pre).
 #include "common.cuh"
-#include "handle.h"
+#include "decoder.h"
 #include "tc_ptx.cuh"
 
 namespace snb {
@@ -163,15 +163,6 @@ int latent_forward_fused(const snb_handle_s* h, int64_t B, const float* shape_la
     latent_fwd_kernel<1><<<grid, 256, 0, st>>>(L, B, shape_latent, texture_latent, zlat, ebias, eimg);
     SNB_LAUNCH_CHECK();
   }
-  return 0;
-}
-
-int latent_fold(const snb_handle_s* h, int64_t B, const float* s_lat, float* dz, cudaStream_t st) {
-  LatentLayers L;
-  if (fill_layers(h, L)) return 2;
-  dim3 gridf(L.n_total, (unsigned)B, (unsigned)((L.W + 31) / 32));
-  latent_fold_kernel<<<gridf, 1024, 0, st>>>(L, B, s_lat, dz);
-  SNB_LAUNCH_CHECK();
   return 0;
 }
 

@@ -5,7 +5,7 @@
 // evaluated once per object and enter as a per-object row offset of the next GEMM's A operand; the
 // `cat([y, PE(viewdir)])` layer is two GEMMs accumulating into one output.
 #include "common.cuh"
-#include "handle.h"
+#include "decoder.h"
 #include "sgemm.cuh"
 #include <math.h>
 
@@ -597,51 +597,6 @@ static int autorf_backward(const snb_handle_s* h, const float* xyz, const float*
     SNB_LAUNCH_CHECK();
   }
   (void)shape_latent; (void)texture_latent;
-  return 0;
-}
-
-int latent_forward(const snb_handle_s* h, int64_t B, const float* shape_latent, const float* texture_latent, float* zlat,
-                   cudaStream_t st) {
-  const int W = h->arch.W, D = h->arch.latent_dim, Bs = h->arch.shape_blocks, Bt = h->arch.texture_blocks;
-  const auto& ly = h->layers;
-  for (int j = 1; j <= Bs; ++j)
-    TRY(fwd_linear(shape_latent, D, B, D, ly[h->iSL(j)].w, D, ly[h->iSL(j)].b, W, zlat + (int64_t)(j - 1) * B * W, W, 1, 0,
-                   nullptr, 0, st));
-  for (int j = 1; j <= Bt; ++j)
-    TRY(fwd_linear(texture_latent, D, B, D, ly[h->iTL(j)].w, D, ly[h->iTL(j)].b, W, zlat + (int64_t)(Bs + j - 1) * B * W, W, 1,
-                   0, nullptr, 0, st));
-  return 0;
-}
-
-int latent_effective_bias(const snb_handle_s* h, int64_t B, const float* zlat, float* ebias, cudaStream_t st) {
-  const int W = h->arch.W, Bs = h->arch.shape_blocks, Bt = h->arch.texture_blocks;
-  const auto& ly = h->layers;
-  for (int j = 1; j <= Bs + Bt; ++j) {
-    const int li = j <= Bs ? h->iS(j) : h->iT(j - Bs);
-    TRY(fwd_linear(zlat + (int64_t)(j - 1) * B * W, W, B, W, ly[li].w, W, ly[li].b, W, ebias + (int64_t)(j - 1) * B * W, W, 0, 0,
-                   nullptr, 0, st));
-  }
-  return 0;
-}
-
-int latent_backward(const snb_handle_s* h, int64_t B, const float* shape_latent, const float* texture_latent,
-                    const float* zlat, float* dz, float* g_shape_latent, float* g_texture_latent, float* const* gw,
-                    cudaStream_t st) {
-  const int W = h->arch.W, D = h->arch.latent_dim, Bs = h->arch.shape_blocks, Bt = h->arch.texture_blocks;
-  const auto& ly = h->layers;
-  if (g_shape_latent) TRY(zero(g_shape_latent, B * D, st));
-  if (g_texture_latent) TRY(zero(g_texture_latent, B * D, st));
-  for (int j = 1; j <= Bs + Bt; ++j) {
-    const bool shape = j <= Bs;
-    const int li = shape ? h->iSL(j) : h->iTL(j - Bs);
-    float* d = dz + (int64_t)(j - 1) * B * W;
-    const float* z = zlat + (int64_t)(j - 1) * B * W;
-    const float* lat = shape ? shape_latent : texture_latent;
-    float* glat = shape ? g_shape_latent : g_texture_latent;
-    TRY(mask_colsum(d, z, W, W, B, B, nullptr, st));
-    if (gw) TRY(bwd_weight(d, W, B, W, lat, D, D, gw[2 * li], D, gw[2 * li + 1], nullptr, 0, st));
-    if (glat) TRY(bwd_data(d, W, B, W, ly[li].w, D, D, glat, D, 1, st));
-  }
   return 0;
 }
 

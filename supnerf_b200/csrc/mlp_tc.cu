@@ -14,15 +14,18 @@
 //
 // Warp roles (320 threads): warps 0-7 epilogue (warp w owns TMEM lanes 32*(w%4).. and the column
 // half w/4 of every 64-column chunk), warp 8 weight producer (+ TMEM alloc), warp 9 MMA issuer.
+//
+// Host side: the step programs and weight-packing jobs (build_plan), the packing launches and one launch function per direction
+// (tc1_launch_fwd / tc1_launch_bwd).  Back-end selection, workspace and packed-buffer layout, the latent layers and the timing live in
+// decoder.cu.
 #include "common.cuh"
-#include "handle.h"
+#include "decoder.h"
 #include "tc_ptx.cuh"
 #include "rb_rows.cuh"
 #include <math.h>
 #include <algorithm>
 #include <stdlib.h>
 #include <initializer_list>
-#include <utility>
 #include <vector>
 
 namespace snb {
@@ -840,7 +843,7 @@ __global__ void __launch_bounds__(256) pack_kernel(const __grid_constant__ PackJ
 // ------------------------------------------------------------------------------------------ host side
 using namespace tc;
 
-static bool tc_supported(const snb_handle_s* h, const char** why) {
+bool tc1_supported(const snb_handle_s* h, const char** why) {
   const snb_arch& a = h->arch;
   if (a.arch != SNB_ARCH_CODENERF) { *why = "bf16 mode covers the CodeNeRF/AutoRFMix/SUPNeRF decoder only"; return false; }
   if (a.W != 256) { *why = "bf16 mode needs W == 256"; return false; }
@@ -980,286 +983,78 @@ static TcPlan build_plan(const snb_handle_s* h, bool split = false) {
   return pl;
 }
 
-// second-generation kernels (mlp_tc2.cu): two tiles in flight per CTA
-bool tc2_supported(const snb_handle_s* h);
-bool tc_two_tile_active(const snb_handle_s* h);
-size_t tc2_packed_bytes(const snb_handle_s* h);
-int tc2_pack_weights(const snb_handle_s* h, void* packed, cudaStream_t st);
-int tc2_launch_fwd(const snb_handle_s* h, const void* packed2, const float* xyz, const float* viewdir, int64_t M, int64_t B,
-                   const uint8_t* eimg, uint32_t* masks, float* sigma, float* rgb, float* dbg, uint8_t* save, cudaStream_t st,
-                   const int64_t* m_dev, const int32_t* tile_start, const rb::RowSrc* rs);
-int tc2_launch_bwd(const snb_handle_s* h, const void* packed2, const float* xyz, const float* viewdir, int64_t M, int64_t B,
-                   const uint32_t* masks, const float* sigma, const float* g_sigma, const float* g_rgb, float* g_xyz,
-                   float* g_viewdir, float* g_zlat, uint8_t* save, cudaStream_t st, const int64_t* m_dev, const int32_t* tile_start);
-size_t tc2_fwd_save_bytes(const snb_handle_s* h, int64_t M);
-size_t tc2_bwd_save_bytes(const snb_handle_s* h, int64_t M);
-int tc2_launch_wgrad(const snb_handle_s* h, int64_t M, int64_t B, const uint8_t* fsave, const uint8_t* bsave, const float* sigma,
-                     const float* g_sigma, const float* g_rgb, const float* s_lat, const float* zlat, float* const* gw,
-                     cudaStream_t st, const int64_t* m_dev);
-int tc2_launch_latent_wgrad(const snb_handle_s* h, int64_t B, const float* zlat, const float* dz, const float* shape_latent,
-                            const float* texture_latent, float* const* gw, cudaStream_t st);
+size_t tc1_image_bytes(const snb_handle_s* h, bool split) { return build_plan(h, split).total_bytes; }
 
-static size_t v1_packed_bytes(const snb_handle_s* h) {
-  if (h->v1_packed_bytes_cache == 0) h->v1_packed_bytes_cache = ((size_t)build_plan(h).total_bytes + 1024 + 1023) & ~size_t(1023);
-  return h->v1_packed_bytes_cache;
-}
-// split-precision images: behind the first- and second-generation ones
-static size_t x3_packed_bytes(const snb_handle_s* h) {
-  if (h->x3_packed_bytes_cache == 0) h->x3_packed_bytes_cache = ((size_t)build_plan(h, true).total_bytes + 1024 + 1023) & ~size_t(1023);
-  return h->x3_packed_bytes_cache;
-}
-static size_t x3_packed_off(const snb_handle_s* h) { return (v1_packed_bytes(h) + tc2_packed_bytes(h) + 1023) & ~size_t(1023); }
-static bool use_v2(const snb_handle_s* h) {
-  static const bool force_v1 = [] { const char* e = getenv("SNB_TC_V1"); return e && atoi(e) != 0; }();
-  return !force_v1 && tc2_supported(h);
-}
-
-bool tc_one_tile_supported(const snb_handle_s* h) { const char* why; return tc_supported(h, &why); }
-bool tc_two_tile_active(const snb_handle_s* h) { const char* why; return tc_supported(h, &why) && use_v2(h); }
-
-size_t tc_packed_bytes(const snb_handle_s* h) {
-  const char* why;
-  if (!tc_supported(h, &why)) return 16;
-  return x3_packed_off(h) + x3_packed_bytes(h);
-}
-
-int tc_pack_weights(snb_handle_s* h, void* packed, cudaStream_t st) {
-  const char* why = "";
-  SNB_REQUIRE(tc_supported(h, &why), "snb_pack_weights: %s", why);
-  SNB_REQUIRE(((uintptr_t)packed & 15) == 0, "snb_pack_weights: buffer must be 16-byte aligned");
-  for (int split = 0; split < 2; ++split) {   // the bf16 images, then the fp16 (hi, lo) images of the split-precision mode
-    TcPlan pl = build_plan(h, split != 0);
-    uint8_t* dst = (uint8_t*)packed + (split ? x3_packed_off(h) : 0);
-    for (size_t i = 0; i < pl.jobs.size(); i += kJobsPerLaunch) {
-      PackJobs jb;
-      jb.n = (int)std::min<size_t>(kJobsPerLaunch, pl.jobs.size() - i);
-      for (int k = 0; k < jb.n; ++k) jb.j[k] = pl.jobs[i + k];
-      pack_kernel<<<jb.n, 256, 0, st>>>(jb, dst);
-      SNB_LAUNCH_CHECK();
-    }
+int tc1_pack_weights(const snb_handle_s* h, bool split, void* packed, cudaStream_t st) {
+  TcPlan pl = build_plan(h, split);
+  for (size_t i = 0; i < pl.jobs.size(); i += kJobsPerLaunch) {
+    PackJobs jb;
+    jb.n = (int)std::min<size_t>(kJobsPerLaunch, pl.jobs.size() - i);
+    for (int k = 0; k < jb.n; ++k) jb.j[k] = pl.jobs[i + k];
+    pack_kernel<<<jb.n, 256, 0, st>>>(jb, (uint8_t*)packed);
+    SNB_LAUNCH_CHECK();
   }
-  if (tc2_supported(h) && tc2_pack_weights(h, (uint8_t*)packed + v1_packed_bytes(h), st)) return 1;
-  h->packed = packed;
   return 0;
 }
 
-static inline int64_t tiles_of(int64_t M) { return (M + kTileM - 1) / kTileM; }
-
-// workspace: [zlat (Bs+Bt)*B*256 fp32][masks tiles*slots*8*128 u32]
-static size_t ws_zlat_bytes(const snb_handle_s* h, int64_t B) {
-  return (size_t)(h->arch.shape_blocks + h->arch.texture_blocks) * B * 256 * sizeof(float);
-}
-// workspace: [zlat][effective biases fp32][effective-bias stage images, 32 B per unit][masks]
-static size_t ws_eimg_off(const snb_handle_s* h, int64_t B) { return (2 * ws_zlat_bytes(h, B) + 255) & ~size_t(255); }
-static size_t ws_masks_off(const snb_handle_s* h, int64_t B) { return (ws_eimg_off(h, B) + 8 * ws_zlat_bytes(h, B) + 255) & ~size_t(255); }
-size_t tc_workspace_bytes(const snb_handle_s* h, int64_t M, int64_t B) {
-  const int slots = h->arch.shape_blocks + h->arch.texture_blocks + 3;
-  return ws_masks_off(h, B) + (size_t)tiles_of(M) * slots * 8 * 128 * 4 + 256;
-}
-size_t tc_bwd_scratch_bytes(const snb_handle_s* h, int64_t, int64_t B) { return ((2 * ws_zlat_bytes(h, B) + 255) & ~size_t(255)) + 256; }   // column sums + their W^T fold
-// training mode (SNB_PREC_BF16_TRAIN): the operand tiles kept for the weight-gradient kernels live behind the normal
-// workspace (forward) / scratch (backward: + a d xyz / d viewdir dummy, since training runs the full backward program)
-size_t tc_train_workspace_extra(const snb_handle_s* h, int64_t M) { return tc2_supported(h) ? tc2_fwd_save_bytes(h, M) + 1024 : 0; }
-size_t tc_train_scratch_extra(const snb_handle_s* h, int64_t M) {
-  return tc2_supported(h) ? tc2_bwd_save_bytes(h, M) + (size_t)M * 24 + 1024 : 0;
-}
-static inline uint8_t* align1k(uint8_t* p) { return (uint8_t*)(((uintptr_t)p + 1023) & ~uintptr_t(1023)); }
-
-static int tc_common_checks(const snb_handle_s* h, int64_t M, int64_t B, const char* who, bool ragged = false) {
-  const char* why = "";
-  SNB_REQUIRE(tc_supported(h, &why), "%s: %s", who, why);
-  SNB_REQUIRE(h->packed != nullptr, "%s: weights not packed (call snb_pack_weights)", who);
-  SNB_REQUIRE(ragged || (M / B) % kTileM == 0, "%s: bf16 mode needs samples-per-object (%lld) to be a multiple of %d; use fp32 mode",
-              who, (long long)(M / B), kTileM);
-  return 0;
-}
-
-static void fill_common(Params& p, const snb_handle_s* h, const float* xyz, const float* viewdir, int64_t M, int64_t B,
-                        const float* zlat, uint32_t* masks) {
+static void fill_common(Params& p, const snb_handle_s* h, const void* packed, const float* xyz, const float* viewdir, int64_t M,
+                        int64_t B, const float* zlat, uint32_t* masks, const int64_t* m_dev, const int32_t* tile_start) {
   p = Params{};
   p.xyz = xyz; p.viewdir = viewdir; p.M = M; p.B = B; p.rows_per_obj = M / B;
-  p.packed = (const uint8_t*)h->packed; p.zlat = zlat; p.masks = masks;
+  p.packed = (const uint8_t*)packed; p.zlat = zlat; p.masks = masks;
   p.wsig = h->layers[h->iSG].w; p.bsig = h->layers[h->iSG].b;
   p.n_latent = h->arch.shape_blocks + h->arch.texture_blocks;
   p.ev_step = h->arch.shape_blocks + 2;  // forward step index of encoding_viewdir
   p.w2 = h->layers[h->iR2].w; p.b2 = h->layers[h->iR2].b;
+  p.m_dev = m_dev; p.tile_start = tile_start;
 }
 
 static int tc_grid(int64_t M) {
   static const int cap = [] { const char* e = getenv("SNB_TC_GRID_CAP"); return e ? atoi(e) : 0; }();   // tuning: fewer CTAs than SMs
   int sms = sm_count();
   if (cap > 0 && cap < sms) sms = cap;
-  const int64_t t = tiles_of(M);
+  const int64_t t = (M + kTileM - 1) / kTileM;
   return (int)(t < sms ? t : sms);
 }
 
-// optional kernel-only timing (bench.py roofline): CUDA events recorded on the launch stream around the tcgen05 kernels
-void tc_timing_enable(snb_handle_s* h, int on) {
-  h->timing_on = on != 0;
-  for (auto* v : {&h->ev_fwd, &h->ev_bwd}) {
-    for (auto& e : *v) { cudaEventDestroy((cudaEvent_t)e.first); cudaEventDestroy((cudaEvent_t)e.second); }
-    v->clear();
-  }
-}
-int tc_timing_read(snb_handle_s* h, int which, float* ms, int max_n) {   // call after a stream/device synchronize
-  auto& v = which == 0 ? h->ev_fwd : h->ev_bwd;
-  int n = 0;
-  for (auto& e : v) {
-    if (n >= max_n) break;
-    float t = 0.f;
-    if (cudaEventElapsedTime(&t, (cudaEvent_t)e.first, (cudaEvent_t)e.second) == cudaSuccess) ms[n++] = t;
-  }
-  return n;
-}
-struct ScopedKernelTimer {
-  cudaStream_t st; std::pair<cudaEvent_t, cudaEvent_t> ev; bool on;
-  ScopedKernelTimer(cudaStream_t s, bool enable) : st(s), on(enable) {
-    if (on) { cudaEventCreate(&ev.first); cudaEventCreate(&ev.second); cudaEventRecord(ev.first, st); }
-  }
-  void stop(std::vector<std::pair<void*, void*>>& into) { if (on) { cudaEventRecord(ev.second, st); into.push_back({(void*)ev.first, (void*)ev.second}); } }
-};
-
-
-int tc_forward(const snb_handle_s* h, const float* xyz, const float* viewdir, int64_t M, int64_t B,
-               const float* shape_latent, const float* texture_latent, float* sigma, float* rgb, void* ws, cudaStream_t st,
-               bool train, const int64_t* m_dev, const int32_t* tile_start, const rb::RowSrc* rs, bool split) {
-  if (tc_common_checks(h, M, B, "mlp_fwd(bf16)", tile_start != nullptr)) return 2;
-  if (split) {   // SNB_PREC_FP32_TC: fp16 (hi, lo) operands, three MMAs per product, on the one-tile kernels (frozen weights)
-    SNB_REQUIRE(!train && rs == nullptr && xyz != nullptr && viewdir != nullptr, "mlp_fwd(fp32_tc): frozen weights and explicit coordinates only");
-    SNB_REQUIRE(tile_start == nullptr || m_dev != nullptr, "mlp_fwd(fp32_tc): per-object tile offsets need a device-side row count");
-    float* ebias = (float*)((uint8_t*)ws + ws_zlat_bytes(h, B));
-    uint32_t* masks = (uint32_t*)((uint8_t*)ws + ws_masks_off(h, B));
-    if (latent_forward_fused(h, B, shape_latent, texture_latent, (float*)ws, ebias, st, nullptr)) return 1;
-    TcPlan pl = build_plan(h, true);
-    Params p;
-    fill_common(p, h, xyz, viewdir, M, B, ebias, masks);
-    p.packed = (const uint8_t*)h->packed + x3_packed_off(h);
-    p.m_dev = m_dev; p.tile_start = tile_start;
-    p.sigma = sigma; p.rgb = rgb; p.dbg = h->dbg_acts;
-    p.prog = pl.fwd;
-    SNB_CHECK_CUDA(cudaFuncSetAttribute(tc_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Map<true>::SM_ALLOC));
-    ScopedKernelTimer tm(st, h->timing_on);
-    tc_fwd_kernel<true><<<tc_grid(M), kThreads, Map<true>::SM_ALLOC, st>>>(p);
-    tm.stop(const_cast<snb_handle_s*>(h)->ev_fwd);
-    SNB_LAUNCH_CHECK();
-    return 0;
-  }
-  SNB_REQUIRE(rs == nullptr || (tile_start != nullptr && rs->rays8 && rs->box && rs->z_steps && rs->jitter && rs->order && rs->counts),
-              "mlp_fwd(bf16): a row source needs per-object tile offsets and all of its pointers");
-  SNB_REQUIRE(rs != nullptr || (xyz != nullptr && viewdir != nullptr), "mlp_fwd(bf16): null coordinates");
-  SNB_REQUIRE(m_dev == nullptr || B == 1 || tile_start != nullptr,
-              "mlp_fwd(bf16): a device-side row count needs one object (or per-object tile offsets)");
-  SNB_REQUIRE(tile_start == nullptr || (m_dev != nullptr && !train), "mlp_fwd(bf16): per-object tile offsets need frozen weights and a device-side row count");
-  SNB_REQUIRE(rs == nullptr || use_v2(h), "mlp_fwd(bf16): the fused sampler needs the two-tile kernels");
-  SNB_REQUIRE(!train || use_v2(h), "mlp_fwd(bf16, training): weight gradients need the two-tile tcgen05 kernels (W = 256, "
-                                    "shape_blocks + texture_blocks <= 4); use precision='fp32' for this architecture");
-  uint8_t* fsave = train ? align1k((uint8_t*)ws + tc_workspace_bytes(h, M, B)) : nullptr;
-  float* zlat = (float*)ws;
-  float* ebias = (float*)((uint8_t*)ws + ws_zlat_bytes(h, B));
-  uint32_t* masks = (uint32_t*)((uint8_t*)ws + ws_masks_off(h, B));
-  uint8_t* eimg = (uint8_t*)ws + ws_eimg_off(h, B);
-  if (latent_forward_fused(h, B, shape_latent, texture_latent, zlat, ebias, st, use_v2(h) ? eimg : nullptr)) return 1;
-  if (use_v2(h)) {
-    ScopedKernelTimer tm2(st, h->timing_on);
-    if (tc2_launch_fwd(h, (const uint8_t*)h->packed + v1_packed_bytes(h), xyz, viewdir, M, B, eimg, masks, sigma, rgb,
-                       h->dbg_acts, fsave, st, m_dev, tile_start, rs)) return 1;
-    tm2.stop(const_cast<snb_handle_s*>(h)->ev_fwd);
-    SNB_LAUNCH_CHECK();
-    return 0;
-  }
-  TcPlan pl = build_plan(h);
+// forward: zlat holds the per-object effective biases (latent_forward_fused's ebias)
+template <bool X>
+int tc1_launch_fwd(const snb_handle_s* h, const void* packed, const float* xyz, const float* viewdir, int64_t M, int64_t B,
+                   const float* ebias, uint32_t* masks, float* sigma, float* rgb, cudaStream_t st, const int64_t* m_dev,
+                   const int32_t* tile_start) {
+  TcPlan pl = build_plan(h, X);
   Params p;
-  fill_common(p, h, xyz, viewdir, M, B, ebias, masks);
-  p.m_dev = m_dev; p.tile_start = tile_start;
+  fill_common(p, h, packed, xyz, viewdir, M, B, ebias, masks, m_dev, tile_start);
   p.sigma = sigma; p.rgb = rgb; p.dbg = h->dbg_acts;
   p.prog = pl.fwd;
-  SNB_CHECK_CUDA(cudaFuncSetAttribute(tc_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Map<false>::SM_ALLOC));
-  ScopedKernelTimer tm(st, h->timing_on);
-  tc_fwd_kernel<false><<<tc_grid(M), kThreads, Map<false>::SM_ALLOC, st>>>(p);
-  tm.stop(const_cast<snb_handle_s*>(h)->ev_fwd);
-  SNB_LAUNCH_CHECK();
+  SNB_CHECK_CUDA(cudaFuncSetAttribute(tc_fwd_kernel<X>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Map<X>::SM_ALLOC));
+  tc_fwd_kernel<X><<<tc_grid(M), kThreads, Map<X>::SM_ALLOC, st>>>(p);
   return 0;
 }
 
-int tc_backward(const snb_handle_s* h, const float* xyz, const float* viewdir, int64_t M, int64_t B,
-                const float* shape_latent, const float* texture_latent, const float* sigma, const float* g_sigma,
-                const float* g_rgb, const void* ws, void* scratch, float* g_xyz, float* g_viewdir, float* g_shape_latent,
-                float* g_texture_latent, float* const* g_weights, cudaStream_t st, bool train, const int64_t* m_dev,
-                const int32_t* tile_start, bool split) {
-  if (tc_common_checks(h, M, B, "mlp_bwd(bf16)", tile_start != nullptr)) return 2;
-  if (split) {
-    SNB_REQUIRE(!train && g_weights == nullptr, "mlp_bwd(fp32_tc): frozen weights only (weight gradients: precision='fp32' runs the FFMA back end)");
-    SNB_REQUIRE((g_xyz == nullptr) == (g_viewdir == nullptr), "mlp_bwd(fp32_tc): request both g_xyz and g_viewdir or neither");
-    SNB_REQUIRE(tile_start == nullptr || m_dev != nullptr, "mlp_bwd(fp32_tc): per-object tile offsets need a device-side row count");
-    const float* zlat = (const float*)ws;
-    uint32_t* masks = (uint32_t*)((uint8_t*)ws + ws_masks_off(h, B));
-    float* g_zlat = (float*)scratch;
-    SNB_CHECK_CUDA(cudaMemsetAsync(g_zlat, 0, ws_zlat_bytes(h, B), st));
-    TcPlan pl = build_plan(h, true);
-    Params p;
-    fill_common(p, h, xyz, viewdir, M, B, zlat, masks);
-    p.packed = (const uint8_t*)h->packed + x3_packed_off(h);
-    p.m_dev = m_dev; p.tile_start = tile_start;
-    p.sigma_in = sigma; p.g_sigma = g_sigma; p.g_rgb = g_rgb; p.g_xyz = g_xyz; p.g_viewdir = g_viewdir; p.g_zlat = g_zlat;
-    p.r0_mask_slot = pl.r0_slot;
-    p.prog = g_xyz ? pl.bwd_full : pl.bwd_noxyz;
-    SNB_CHECK_CUDA(cudaFuncSetAttribute(tc_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Map<true>::SM_ALLOC));
-    ScopedKernelTimer tm(st, h->timing_on);
-    tc_bwd_kernel<true><<<tc_grid(M), kThreads, Map<true>::SM_ALLOC, st>>>(p);
-    tm.stop(const_cast<snb_handle_s*>(h)->ev_bwd);
-    SNB_LAUNCH_CHECK();
-    return latent_backward_fused(h, B, zlat, g_zlat, g_shape_latent, g_texture_latent, st);
-  }
-  SNB_REQUIRE(m_dev == nullptr || B == 1 || tile_start != nullptr,
-              "mlp_bwd(bf16): a device-side row count needs one object (or per-object tile offsets)");
-  SNB_REQUIRE(tile_start == nullptr || (m_dev != nullptr && !train), "mlp_bwd(bf16): per-object tile offsets need frozen weights and a device-side row count");
-  SNB_REQUIRE(g_weights == nullptr || (train && use_v2(h)),
-              "mlp_bwd(bf16): weight gradients need the forward to have run in training mode (SNB_PREC_BF16_TRAIN: the python "
-              "modules select it when a weight requires grad) on an architecture the two-tile kernels cover; otherwise freeze "
-              "the weights (requires_grad_(False)) or use precision='fp32'");
-  SNB_REQUIRE((g_xyz == nullptr) == (g_viewdir == nullptr), "mlp_bwd(bf16): request both g_xyz and g_viewdir or neither");
-  const float* zlat = (const float*)ws;
-  uint32_t* masks = (uint32_t*)((uint8_t*)ws + ws_masks_off(h, B));
-  float* g_zlat = (float*)scratch;
-  SNB_CHECK_CUDA(cudaMemsetAsync(g_zlat, 0, ws_zlat_bytes(h, B), st));
-  if (use_v2(h)) {
-    float* fold_tmp = (float*)((uint8_t*)scratch + ws_zlat_bytes(h, B));
-    uint8_t* bsave = nullptr;
-    const bool want_w = train && g_weights != nullptr;
-    if (want_w) {   // training: keep every step's d pre-activation tile, run the full program (d xyz into a dummy if unwanted)
-      bsave = align1k((uint8_t*)scratch + tc_bwd_scratch_bytes(h, M, B));
-      float* dummy = (float*)(bsave + tc2_bwd_save_bytes(h, M));
-      if (g_xyz == nullptr) { g_xyz = dummy; g_viewdir = dummy + 3 * M; }
-      for (size_t i = 0; i < h->layers.size(); ++i) {   // every weight gradient is accumulated (atomics / +=): zero first
-        SNB_CHECK_CUDA(cudaMemsetAsync(g_weights[2 * i], 0, sizeof(float) * h->layers[i].out * h->layers[i].in, st));
-        SNB_CHECK_CUDA(cudaMemsetAsync(g_weights[2 * i + 1], 0, sizeof(float) * h->layers[i].out, st));
-      }
-    }
-    ScopedKernelTimer tm2(st, h->timing_on);
-    if (tc2_launch_bwd(h, (const uint8_t*)h->packed + v1_packed_bytes(h), xyz, viewdir, M, B, masks, sigma, g_sigma, g_rgb, g_xyz,
-                       g_viewdir, g_zlat, bsave, st, m_dev, tile_start)) return 1;
-    tm2.stop(const_cast<snb_handle_s*>(h)->ev_bwd);
-    SNB_LAUNCH_CHECK();
-    if (!want_w) return latent_backward_fused(h, B, zlat, g_zlat, g_shape_latent, g_texture_latent, st, fold_tmp);
-    const uint8_t* fsave = align1k((uint8_t*)ws + tc_workspace_bytes(h, M, B));
-    if (tc2_launch_wgrad(h, M, B, fsave, bsave, sigma, g_sigma, g_rgb, g_zlat, zlat, g_weights, st, m_dev)) return 1;
-    // latent layers (per object): fold the column sums through W_layer^T (= d loss / d z), d latent, then their weight gradients
-    if (latent_backward_fused(h, B, zlat, g_zlat, g_shape_latent, g_texture_latent, st, fold_tmp)) return 1;
-    return tc2_launch_latent_wgrad(h, B, zlat, fold_tmp, shape_latent, texture_latent, g_weights, st);
-  }
-  TcPlan pl = build_plan(h);
+template <bool X>
+int tc1_launch_bwd(const snb_handle_s* h, const void* packed, const float* xyz, const float* viewdir, int64_t M, int64_t B,
+                   const float* zlat, uint32_t* masks, const float* sigma, const float* g_sigma, const float* g_rgb, float* g_xyz,
+                   float* g_viewdir, float* g_zlat, cudaStream_t st, const int64_t* m_dev, const int32_t* tile_start) {
+  TcPlan pl = build_plan(h, X);
   Params p;
-  fill_common(p, h, xyz, viewdir, M, B, zlat, masks);
-  p.m_dev = m_dev; p.tile_start = tile_start;
+  fill_common(p, h, packed, xyz, viewdir, M, B, zlat, masks, m_dev, tile_start);
   p.sigma_in = sigma; p.g_sigma = g_sigma; p.g_rgb = g_rgb; p.g_xyz = g_xyz; p.g_viewdir = g_viewdir; p.g_zlat = g_zlat;
   p.r0_mask_slot = pl.r0_slot;
   p.prog = g_xyz ? pl.bwd_full : pl.bwd_noxyz;
-  SNB_CHECK_CUDA(cudaFuncSetAttribute(tc_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Map<false>::SM_ALLOC));
-  ScopedKernelTimer tm(st, h->timing_on);
-  tc_bwd_kernel<false><<<tc_grid(M), kThreads, Map<false>::SM_ALLOC, st>>>(p);
-  tm.stop(const_cast<snb_handle_s*>(h)->ev_bwd);
-  SNB_LAUNCH_CHECK();
-  return latent_backward_fused(h, B, zlat, g_zlat, g_shape_latent, g_texture_latent, st);
+  SNB_CHECK_CUDA(cudaFuncSetAttribute(tc_bwd_kernel<X>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Map<X>::SM_ALLOC));
+  tc_bwd_kernel<X><<<tc_grid(M), kThreads, Map<X>::SM_ALLOC, st>>>(p);
+  return 0;
 }
+
+#define SNB_TC1_LAUNCHERS(X)                                                                                                       \
+  template int tc1_launch_fwd<X>(const snb_handle_s*, const void*, const float*, const float*, int64_t, int64_t, const float*,     \
+                                 uint32_t*, float*, float*, cudaStream_t, const int64_t*, const int32_t*);                         \
+  template int tc1_launch_bwd<X>(const snb_handle_s*, const void*, const float*, const float*, int64_t, int64_t, const float*,     \
+                                 uint32_t*, const float*, const float*, const float*, float*, float*, float*, cudaStream_t,        \
+                                 const int64_t*, const int32_t*);
+SNB_TC1_LAUNCHERS(false)
+SNB_TC1_LAUNCHERS(true)
+#undef SNB_TC1_LAUNCHERS
 
 }  // namespace snb

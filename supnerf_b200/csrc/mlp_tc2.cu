@@ -22,7 +22,7 @@
 //    arrivals, the peer's MMA warp relays its stage completions; in the forward encoding_viewdir is one step whose last stage
 //    multiplies a per-slot PE(viewdir) tile.  Same arithmetic, bit-identical sigma / rgb (tests/test_gpu_bf16.py).
 #include "common.cuh"
-#include "handle.h"
+#include "decoder.h"
 #include "tc_ptx.cuh"
 #include "rb_rows.cuh"
 #include <algorithm>

@@ -4,8 +4,8 @@
 // Every intermediate lives in ONE caller-provided workspace (no allocation, no synchronisation here), so a refine
 // iteration costs two host calls per object instead of ~50 autograd-node launches.
 #include "common.cuh"
-#include "handle.h"
 #include "compact.h"
+#include "decoder.h"
 #include <stdlib.h>
 
 using namespace snb;
@@ -17,13 +17,13 @@ inline size_t al(size_t bytes) { return (bytes + 255) & ~size_t(255); }
 // of the 128-row tile, so any ray / sample count works; without it the bf16 decoder needs N * S to be a multiple of 128 itself
 inline int64_t decoder_rows(snb_handle h, const snb_render_desc& d);
 
-// Miss-ray compaction (compact.cu) applies to the box render on the two-tile tensor-core decoder; SNB_NO_COMPACT=1 disables it.
+// Miss-ray compaction (compact.cu) applies to the box render on the tensor-core decoders: they take the device-side row count (the
+// FFMA back end runs dense rows); SNB_NO_COMPACT=1 disables it.
 bool use_compaction(snb_handle h, const snb_render_desc& d) {
   static const bool off = [] { const char* e = getenv("SNB_NO_COMPACT"); return e && atoi(e) != 0; }();
   if (off || d.mode != SNB_RENDER_BOX || d.n_rays <= 0) return false;
-  if (d.precision == SNB_PREC_FP32) return false;     // FFMA back end: dense rows
-  if (d.precision == SNB_PREC_BF16_TRAIN) return tc_two_tile_active(h);
-  return tc_one_tile_supported(h);                    // frozen weights: every tensor-core kernel takes the device-side row count
+  Backend be;
+  return select_backend(h, d.precision, &be) == nullptr && be != Backend::Ffma;
 }
 
 // forward workspace (kept for the backward): rays_o, viewdir (N,3) | xyz, vrep (M,3) | z_vals (M) | sigma (M) | rgb (M,3) | mlp ws
@@ -141,8 +141,8 @@ extern "C" int snb_render_fwd(snb_handle h, const snb_render_desc* d, const floa
     int64_t* counts = reinterpret_cast<int64_t*>(wsb + L.counts);
     if (compact_plan(wsb + L.hit, N, d->n_samples, order, pos, counts, st)) return 1;
     if (compact_gather(F(ws, L.xyz), F(ws, L.vrep), order, counts, N, d->n_samples, F(ws, L.xyz_c), F(ws, L.vrep_c), st)) return 1;
-    if (tc_forward(h, F(ws, L.xyz_c), F(ws, L.vrep_c), decoder_rows(h, *d), 1, shape_latent, texture_latent, F(ws, L.sigma_c), F(ws, L.rgb_c),
-                   wsb + L.mlp, st, d->precision == SNB_PREC_BF16_TRAIN, counts + 3, nullptr, nullptr, d->precision == SNB_PREC_FP32_TC)) return 1;
+    if (decoder_forward(h, d->precision, F(ws, L.xyz_c), F(ws, L.vrep_c), decoder_rows(h, *d), 1, shape_latent, texture_latent,
+                        F(ws, L.sigma_c), F(ws, L.rgb_c), wsb + L.mlp, st, {counts + 3})) return 1;
     if (compact_expand(F(ws, L.sigma_c), F(ws, L.rgb_c), wsb + L.hit, pos, counts, N, d->n_samples, F(ws, L.sigma), F(ws, L.rgb), st))
       return 1;
   } else if (snb_mlp_fwd(h, d->precision, F(ws, L.xyz), F(ws, L.vrep), M, 1, shape_latent, texture_latent, F(ws, L.sigma),
@@ -160,16 +160,7 @@ extern "C" int snb_render_bwd(snb_handle h, const snb_render_desc* d, const floa
   SNB_REQUIRE(g_shape_latent && g_texture_latent, "render_bwd: latent gradient outputs are required");
   cudaStream_t st = (cudaStream_t)stream;
   if (g_c2w) SNB_CHECK_CUDA(cudaMemsetAsync(g_c2w, 0, 12 * sizeof(float), st));
-  if (d->n_rays == 0) {   // nothing rendered: every gradient is zero
-    SNB_CHECK_CUDA(cudaMemsetAsync(g_shape_latent, 0, sizeof(float) * h->arch.latent_dim, st));
-    SNB_CHECK_CUDA(cudaMemsetAsync(g_texture_latent, 0, sizeof(float) * h->arch.latent_dim, st));
-    if (g_weights)
-      for (size_t i = 0; i < h->layers.size(); ++i) {
-        SNB_CHECK_CUDA(cudaMemsetAsync(g_weights[2 * i], 0, sizeof(float) * h->layers[i].out * h->layers[i].in, st));
-        SNB_CHECK_CUDA(cudaMemsetAsync(g_weights[2 * i + 1], 0, sizeof(float) * h->layers[i].out, st));
-      }
-    return 0;
-  }
+  if (d->n_rays == 0) return decoder_zero_grads(h, 1, g_shape_latent, g_texture_latent, g_weights, st);   // nothing rendered
   const bool shell = d->mode == SNB_RENDER_SHELL;
   SNB_REQUIRE(px && py && K && c2w && z_steps && (jitter || shell) && shape_latent && texture_latent && workspace && g_rgb &&
               g_depth && g_acc && scratch, "render_bwd: null pointer");
@@ -189,10 +180,10 @@ extern "C" int snb_render_bwd(snb_handle h, const snb_render_desc* d, const floa
     const int32_t* pos = reinterpret_cast<const int32_t*>(wsb + L.pos);
     const int64_t* counts = reinterpret_cast<const int64_t*>(wsb + L.counts);
     if (compact_reduce(F(sc, G.g_sigma), F(sc, G.g_rgbs), order, counts, N, d->n_samples, F(sc, G.g_sigma_c), F(sc, G.g_rgb_c), st)) return 1;
-    if (tc_backward(h, F(ws, L.xyz_c), F(ws, L.vrep_c), decoder_rows(h, *d), 1, shape_latent, texture_latent, F(ws, L.sigma_c), F(sc, G.g_sigma_c),
-                    F(sc, G.g_rgb_c), wsb + L.mlp, static_cast<uint8_t*>(sc) + G.mlp, pose ? F(sc, G.g_xyz_c) : nullptr,
-                    pose ? F(sc, G.g_vrep_c) : nullptr, g_shape_latent, g_texture_latent, g_weights, st,
-                    d->precision == SNB_PREC_BF16_TRAIN, counts + 3, nullptr, d->precision == SNB_PREC_FP32_TC)) return 1;
+    if (decoder_backward(h, d->precision, F(ws, L.xyz_c), F(ws, L.vrep_c), decoder_rows(h, *d), 1, shape_latent, texture_latent,
+                         F(ws, L.sigma_c), F(sc, G.g_sigma_c), F(sc, G.g_rgb_c), wsb + L.mlp, static_cast<uint8_t*>(sc) + G.mlp,
+                         pose ? F(sc, G.g_xyz_c) : nullptr, pose ? F(sc, G.g_vrep_c) : nullptr, g_shape_latent, g_texture_latent, g_weights,
+                         st, {counts + 3})) return 1;
     if (!pose) return 0;
     if (sample_box_bwd_compact(F(ws, L.rays_o), F(ws, L.viewdir), z_steps, jitter, N, d->n_samples, d->half_diag, d->aabb_half,
                                F(sc, G.g_xyz_c), F(sc, G.g_vrep_c), F(sc, G.g_z), pos, counts, F(sc, G.g_rays_o), F(sc, G.g_viewdir), st))

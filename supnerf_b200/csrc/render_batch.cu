@@ -17,8 +17,7 @@
 //
 // plus the batched refine losses (one launch per direction for all objects).  Frozen weights, bf16 decoder (two-tile kernels).
 #include "common.cuh"
-#include "handle.h"
-#include "compact.h"
+#include "decoder.h"
 #include "sampler.cuh"
 #include "composite.cuh"
 #include "rb_rows.cuh"
@@ -733,13 +732,12 @@ __global__ void __launch_bounds__(256) rb_loss_bwd_kernel(const float* __restric
 
 }  // namespace rb
 
-// mlp_tc.cu
-size_t tc_workspace_bytes(const snb_handle_s* h, int64_t M, int64_t B);
-size_t tc_bwd_scratch_bytes(const snb_handle_s* h, int64_t M, int64_t B);
-
 namespace {
 
 inline size_t al(size_t bytes) { return (bytes + 255) & ~size_t(255); }
+
+// the decoder precision of a batched render: frozen weights, bf16 or (SNB_BATCH_FP32_TC) split precision
+inline int32_t batch_precision(const snb_batch_desc& d) { return (d.flags & SNB_BATCH_FP32_TC) ? SNB_PREC_FP32_TC : SNB_PREC_BF16; }
 
 // forward workspace (kept for the backward).  Mmax = B * pad256(N * S): every object's rows if all of its rays hit.  With the fused
 // sampler (SNB_BATCH_FUSED_SAMPLER) the forward keeps NO per-row coordinates: the decoder computes them from rays8 + jitter (K1), the
@@ -765,7 +763,7 @@ struct BatchLayout {
     z_c = o; o += al(Mc * 4);
     sigma_c = o; o += al(M * 4);
     rgb_c = o; o += al(M * 12);
-    mlp = o; o += al(tc_workspace_bytes(h, Mmax, (int64_t)B));
+    mlp = o; o += al(decoder_workspace_bytes(h, batch_precision(d), Mmax, (int64_t)B));
     total = o;
   }
 };
@@ -788,7 +786,7 @@ struct BatchScratch {
     g_vrep_c = o; o += al(M * 12);
     acc64 = o; o += al(B * 12 * 8);
     tickets = o; o += al(B * 4);
-    mlp = o; o += al(tc_bwd_scratch_bytes(h, Mmax, (int64_t)B));
+    mlp = o; o += al(decoder_scratch_bytes(h, batch_precision(d), Mmax, (int64_t)B));
     total = o;
   }
 };
@@ -800,12 +798,13 @@ int check_batch(snb_handle h, const snb_batch_desc* d, const char* who) {
               "%s: the batched render needs n_samples in {4, 8, ..., 128} (vectorised compositing)", who);
   SNB_REQUIRE(d->rays_per_obj < ((int64_t)1 << 30) && d->rays_per_obj * d->n_samples < ((int64_t)1 << 31) &&
               (int64_t)d->n_objs * d->rays_per_obj < ((int64_t)1 << 31), "%s: too many rays", who);
-  SNB_REQUIRE(tc_one_tile_supported(h), "%s: the batched render runs on the tcgen05 decoder kernels (CodeNeRF family, W = 256, "
-                                        "shape_blocks + texture_blocks <= 10); render the objects one by one for this architecture", who);
+  Backend be;
+  SNB_REQUIRE(select_backend(h, batch_precision(*d), &be) == nullptr, "%s: the batched render runs on the tcgen05 decoder kernels "
+              "(CodeNeRF family, W = 256, shape_blocks + texture_blocks <= 10); render the objects one by one for this architecture", who);
   if (d->flags & SNB_BATCH_FP32_TC)
     SNB_REQUIRE(!(d->flags & SNB_BATCH_FUSED_SAMPLER), "%s: SNB_BATCH_FP32_TC and SNB_BATCH_FUSED_SAMPLER exclude each other", who);
   if (d->flags & SNB_BATCH_FUSED_SAMPLER)
-    SNB_REQUIRE(tc_two_tile_active(h), "%s: the fused sampler needs the two-tile kernels (shape_blocks + texture_blocks <= 4)", who);
+    SNB_REQUIRE(be == Backend::TwoTile, "%s: the fused sampler needs the two-tile kernels (shape_blocks + texture_blocks <= 4)", who);
   return 0;
 }
 
@@ -866,8 +865,9 @@ extern "C" int snb_render_batch_fwd(snb_handle h, const snb_batch_desc* d, const
     rb::RowSrc rs;
     rs.rays8 = at<float>(ws, L.rays8); rs.box = box; rs.z_steps = z_steps; rs.jitter = jitter; rs.order = at<int32_t>(ws, L.order);
     rs.counts = at<rb::ObjCounts>(ws, L.counts); rs.N = N; rs.S = S;
-    if (tc_forward(h, nullptr, nullptr, L.Mmax, B, shape_latent, texture_latent, at<float>(ws, L.sigma_c), at<float>(ws, L.rgb_c),
-                   at<uint8_t>(ws, L.mlp), st, false, &at<rb::Meta>(ws, L.meta)->total_rows, at<int32_t>(ws, L.tile_start), &rs))
+    if (decoder_forward(h, SNB_PREC_BF16, nullptr, nullptr, L.Mmax, B, shape_latent, texture_latent, at<float>(ws, L.sigma_c),
+                        at<float>(ws, L.rgb_c), at<uint8_t>(ws, L.mlp), st,
+                        {&at<rb::Meta>(ws, L.meta)->total_rows, at<int32_t>(ws, L.tile_start), &rs}))
       return 1;
   } else {
     // default: the stratified samples of the EXECUTED rows are written once (28 B per row) and read back by the decoder -- measured
@@ -876,9 +876,9 @@ extern "C" int snb_render_batch_fwd(snb_handle h, const snb_batch_desc* d, const
                                                             at<rb::ObjCounts>(ws, L.counts), at<rb::Meta>(ws, L.meta), B, N, S,
                                                             at<float>(ws, L.xyz_c), at<float>(ws, L.vrep_c), at<float>(ws, L.z_c));
     SNB_LAUNCH_CHECK();
-    if (tc_forward(h, at<float>(ws, L.xyz_c), at<float>(ws, L.vrep_c), L.Mmax, B, shape_latent, texture_latent, at<float>(ws, L.sigma_c),
-                   at<float>(ws, L.rgb_c), at<uint8_t>(ws, L.mlp), st, false, &at<rb::Meta>(ws, L.meta)->total_rows,
-                   at<int32_t>(ws, L.tile_start), nullptr, (d->flags & SNB_BATCH_FP32_TC) != 0))
+    if (decoder_forward(h, batch_precision(*d), at<float>(ws, L.xyz_c), at<float>(ws, L.vrep_c), L.Mmax, B, shape_latent, texture_latent,
+                        at<float>(ws, L.sigma_c), at<float>(ws, L.rgb_c), at<uint8_t>(ws, L.mlp), st,
+                        {&at<rb::Meta>(ws, L.meta)->total_rows, at<int32_t>(ws, L.tile_start)}))
       return 1;
     zsrc.z_c = at<float>(ws, L.z_c);
   }
@@ -937,10 +937,10 @@ extern "C" int snb_render_batch_bwd(snb_handle h, const snb_batch_desc* d, const
   if (lpr == 8) SNB_RBB(8); else if (lpr == 16) SNB_RBB(16); else SNB_RBB(32);
 #undef SNB_RBB
   SNB_LAUNCH_CHECK();
-  if (tc_backward(h, xyz_c, vrep_c, L.Mmax, B, shape_latent, texture_latent, at<float>(ws, L.sigma_c),
-                  at<float>(sc, G.g_sigma_c), at<float>(sc, G.g_rgb_c), at<uint8_t>(ws, L.mlp), at<uint8_t>(sc, G.mlp),
-                  pose ? at<float>(sc, G.g_xyz_c) : nullptr, pose ? at<float>(sc, G.g_vrep_c) : nullptr, g_shape_latent, g_texture_latent,
-                  nullptr, st, false, &at<rb::Meta>(ws, L.meta)->total_rows, at<int32_t>(ws, L.tile_start), (d->flags & SNB_BATCH_FP32_TC) != 0))
+  if (decoder_backward(h, batch_precision(*d), xyz_c, vrep_c, L.Mmax, B, shape_latent, texture_latent, at<float>(ws, L.sigma_c),
+                       at<float>(sc, G.g_sigma_c), at<float>(sc, G.g_rgb_c), at<uint8_t>(ws, L.mlp), at<uint8_t>(sc, G.mlp),
+                       pose ? at<float>(sc, G.g_xyz_c) : nullptr, pose ? at<float>(sc, G.g_vrep_c) : nullptr, g_shape_latent, g_texture_latent,
+                       nullptr, st, {&at<rb::Meta>(ws, L.meta)->total_rows, at<int32_t>(ws, L.tile_start)}))
     return 1;
   if (!pose) return 0;
   SNB_CHECK_CUDA(cudaMemsetAsync(at<uint8_t>(sc, G.acc64), 0, G.mlp - G.acc64, st));   // fp64 sums + tickets
