@@ -198,6 +198,8 @@ int decoder_backward(const snb_handle_s* h, int32_t precision, const float* xyz,
     return f32_backward(h, xyz, viewdir, M, B, shape_latent, texture_latent, sigma, g_sigma, g_rgb, (const float*)ws, (float*)scratch,
                         g_xyz, g_viewdir, g_shape_latent, g_texture_latent, g_weights, st);
   if (tc_checks(h, M, B, "mlp_bwd(bf16)", r)) return 2;
+  SNB_REQUIRE(r.live == nullptr || (r.n_live != nullptr && r.tile_start != nullptr && g_weights == nullptr),
+              "mlp_bwd: a list of live super tiles needs its count, per-object tile offsets and frozen weights");
   const TcLayout L(h, precision, M, B);
   if (be == Backend::OneTileSplit) {
     SNB_REQUIRE(g_weights == nullptr, "mlp_bwd(fp32_tc): frozen weights only (weight gradients: precision='fp32' runs the FFMA back end)");
@@ -232,13 +234,13 @@ int decoder_backward(const snb_handle_s* h, int32_t precision, const float* xyz,
   int rc;
   if (be == Backend::TwoTile)
     rc = tc2_launch_bwd(h, packed + packed_layout(h).two_tile, xyz, viewdir, M, B, masks, sigma, g_sigma, g_rgb, g_xyz, g_viewdir,
-                        g_zlat, bsave, st, r.m_dev, r.tile_start);
+                        g_zlat, bsave, st, r.m_dev, r.tile_start, r.live, r.n_live);
   else if (be == Backend::OneTileSplit)
     rc = tc1_launch_bwd<true>(h, packed + packed_layout(h).split, xyz, viewdir, M, B, zlat, masks, sigma, g_sigma, g_rgb, g_xyz,
-                              g_viewdir, g_zlat, st, r.m_dev, r.tile_start);
+                              g_viewdir, g_zlat, st, r.m_dev, r.tile_start, r.live, r.n_live);
   else
     rc = tc1_launch_bwd<false>(h, packed, xyz, viewdir, M, B, zlat, masks, sigma, g_sigma, g_rgb, g_xyz, g_viewdir, g_zlat, st,
-                               r.m_dev, r.tile_start);
+                               r.m_dev, r.tile_start, r.live, r.n_live);
   if (rc) return 1;
   tm.stop(const_cast<snb_handle_s*>(h)->ev_bwd);
   SNB_LAUNCH_CHECK();

@@ -21,6 +21,11 @@ struct DeviceRows {
   const int64_t* m_dev = nullptr;       // number of rows actually present (a multiple of 128, <= M)
   const int32_t* tile_start = nullptr;  // B + 1 ascending, even ints: object b owns the 128-row tiles [tile_start[b], tile_start[b+1])
   const rb::RowSrc* rs = nullptr;       // forward only: the two-tile kernels compute each row's sample (xyz / viewdir unused)
+  // backward only (frozen weights, per-object tile offsets): the 256-row super tiles to run, ascending, and their count.  A super tile
+  // left out has upstream gradients that are exactly zero: its rows' d xyz / d viewdir are not written and it adds nothing to the
+  // latent gradients.  Null: every super tile.
+  const int32_t* live = nullptr;
+  const int32_t* n_live = nullptr;
 };
 
 size_t decoder_workspace_bytes(const snb_handle_s* h, int32_t precision, int64_t M, int64_t B);
@@ -75,7 +80,8 @@ int tc1_launch_fwd(const snb_handle_s* h, const void* packed, const float* xyz, 
 template <bool X>
 int tc1_launch_bwd(const snb_handle_s* h, const void* packed, const float* xyz, const float* viewdir, int64_t M, int64_t B,
                    const float* zlat, uint32_t* masks, const float* sigma, const float* g_sigma, const float* g_rgb, float* g_xyz,
-                   float* g_viewdir, float* g_zlat, cudaStream_t st, const int64_t* m_dev, const int32_t* tile_start);
+                   float* g_viewdir, float* g_zlat, cudaStream_t st, const int64_t* m_dev, const int32_t* tile_start,
+                   const int32_t* live, const int32_t* n_live);
 
 // ---- two-tile tensor-core back end (mlp_tc2.cu).  Same launch-count convention for tc2_launch_fwd / tc2_launch_bwd.
 bool tc2_supported(const snb_handle_s* h);
@@ -86,7 +92,8 @@ int tc2_launch_fwd(const snb_handle_s* h, const void* packed2, const float* xyz,
                    const int64_t* m_dev, const int32_t* tile_start, const rb::RowSrc* rs);
 int tc2_launch_bwd(const snb_handle_s* h, const void* packed2, const float* xyz, const float* viewdir, int64_t M, int64_t B,
                    const uint32_t* masks, const float* sigma, const float* g_sigma, const float* g_rgb, float* g_xyz,
-                   float* g_viewdir, float* g_zlat, uint8_t* save, cudaStream_t st, const int64_t* m_dev, const int32_t* tile_start);
+                   float* g_viewdir, float* g_zlat, uint8_t* save, cudaStream_t st, const int64_t* m_dev, const int32_t* tile_start,
+                   const int32_t* live, const int32_t* n_live);
 // training mode: bytes of the operand tiles the forward / backward keep for the weight-gradient kernels
 size_t tc2_fwd_save_bytes(const snb_handle_s* h, int64_t M);
 size_t tc2_bwd_save_bytes(const snb_handle_s* h, int64_t M);

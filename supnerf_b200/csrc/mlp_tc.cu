@@ -114,6 +114,8 @@ struct Params {
   const int64_t* m_dev;         // device-side row count (a multiple of 128, <= M) or null
   const int32_t* tile_start;    // per-object first tile (B + 1 ints) or null = M / B rows per object
   Program prog;
+  const int32_t* live;          // backward: the 256-row super tiles to run (ascending) or null = every tile (decoder.h: DeviceRows)
+  const int32_t* n_live;        // ... and their count, on the device
 };
 
 template <bool X> struct SmemT {
@@ -138,6 +140,10 @@ __device__ __forceinline__ int64_t obj_of_tile(const Params& p, int64_t tile) {
     if ((int64_t)__ldg(p.tile_start + mid) <= tile) lo = mid; else hi = mid - 1;
   }
   return lo;
+}
+// tile of the backward's j-th work item: its 128-row half of live super tile j / 2, or tile j without a list
+__device__ __forceinline__ int64_t work_tile(const Params& p, int64_t j) {
+  return p.live ? 2 * (int64_t)__ldg(p.live + (j >> 1)) + (j & 1) : j;
 }
 // barrier indices
 constexpr int BAR_WFULL = 0, BAR_WEMPTY = 4, BAR_AREADY = 8, BAR_ACC = 13;
@@ -665,7 +671,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bwd_kernel(const __grid_consta
   }
   kernel_prologue(sm, smem_raw, tid, warp, tmem_base);
   const int64_t M = rows_present(p);
-  const int64_t n_tiles = (M + kTileM - 1) / kTileM;
+  const int64_t n_tiles = p.live ? 2 * (int64_t)__ldg(p.n_live) : (M + kTileM - 1) / kTileM;   // work items (work_tile)
 
   if (warp == 8) {
     producer_loop<X>(p, sm, n_tiles, lane);
@@ -680,7 +686,8 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bwd_kernel(const __grid_consta
     const float* w2_s = sm.tab(MP::TAB_W2);
     uint32_t gstep = 0, acc_cnt[2] = {0, 0};
     const int nslots = p.prog.n_mask_slots;
-    for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+    for (int64_t j = blockIdx.x; j < n_tiles; j += gridDim.x) {
+      const int64_t tile = work_tile(p, j);
       e.grow = tile * kTileM + e.row;
       e.valid = e.grow < M;
       const int64_t crow = e.valid ? e.grow : M - 1;
@@ -786,8 +793,8 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bwd_kernel(const __grid_consta
         tc_fence_before();
       }
       // ---- tile end: d xyz, and flush the latent column sums when the next tile belongs to another object
-      const int64_t next = tile + gridDim.x;
-      const bool flush = next >= n_tiles || obj_of_tile(p, next) != obj;
+      const int64_t next = j + gridDim.x;
+      const bool flush = next >= n_tiles || obj_of_tile(p, work_tile(p, next)) != obj;
       epi_bar_sync();
       if (p.g_xyz != nullptr && e.hh == 0 && e.valid) {
 #pragma unroll
@@ -1035,10 +1042,12 @@ int tc1_launch_fwd(const snb_handle_s* h, const void* packed, const float* xyz, 
 template <bool X>
 int tc1_launch_bwd(const snb_handle_s* h, const void* packed, const float* xyz, const float* viewdir, int64_t M, int64_t B,
                    const float* zlat, uint32_t* masks, const float* sigma, const float* g_sigma, const float* g_rgb, float* g_xyz,
-                   float* g_viewdir, float* g_zlat, cudaStream_t st, const int64_t* m_dev, const int32_t* tile_start) {
+                   float* g_viewdir, float* g_zlat, cudaStream_t st, const int64_t* m_dev, const int32_t* tile_start,
+                   const int32_t* live, const int32_t* n_live) {
   TcPlan pl = build_plan(h, X);
   Params p;
   fill_common(p, h, packed, xyz, viewdir, M, B, zlat, masks, m_dev, tile_start);
+  p.live = live; p.n_live = n_live;
   p.sigma_in = sigma; p.g_sigma = g_sigma; p.g_rgb = g_rgb; p.g_xyz = g_xyz; p.g_viewdir = g_viewdir; p.g_zlat = g_zlat;
   p.r0_mask_slot = pl.r0_slot;
   p.prog = g_xyz ? pl.bwd_full : pl.bwd_noxyz;
@@ -1052,7 +1061,7 @@ int tc1_launch_bwd(const snb_handle_s* h, const void* packed, const float* xyz, 
                                  uint32_t*, float*, float*, cudaStream_t, const int64_t*, const int32_t*);                         \
   template int tc1_launch_bwd<X>(const snb_handle_s*, const void*, const float*, const float*, int64_t, int64_t, const float*,     \
                                  uint32_t*, const float*, const float*, const float*, float*, float*, float*, cudaStream_t,        \
-                                 const int64_t*, const int32_t*);
+                                 const int64_t*, const int32_t*, const int32_t*, const int32_t*);
 SNB_TC1_LAUNCHERS(false)
 SNB_TC1_LAUNCHERS(true)
 #undef SNB_TC1_LAUNCHERS

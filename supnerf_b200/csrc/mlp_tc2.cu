@@ -103,6 +103,8 @@ struct Params {
   const int64_t* m_dev;   // optional: the number of rows actually present (<= M), read on the device -- the fused render compacts
                           // the samples of rays that miss the box on the GPU and never learns the count on the host
   const int32_t* tile_start;   // optional (batched render): B + 1 ascending even tile offsets, object b owns tiles [tile_start[b], tile_start[b+1])
+  const int32_t* live;         // optional, backward: the 256-row super tiles to run, ascending (decoder.h: DeviceRows) ...
+  const int32_t* n_live;       // ... and their count, on the device
   rb::RowSrc rs;               // forward, batched render (K1): rs.rays8 != NULL -> the epilogue warps compute their rows' sample
                                // coordinates from the rays (32 B per ray + 4 B of jitter per row) instead of reading xyz / viewdir
   uint8_t* save;      // training mode (weight gradients wanted): [tile][Program::save_tile_bytes] copies of every step's A operand
@@ -859,7 +861,8 @@ __global__ void __launch_bounds__(kThreads, 1) tc2_bwd_kernel(const __grid_const
   kernel_prologue<CG2>(sm, tid, warp, tmem_base);
   const int64_t M_eff = rows_present(p);
   const int64_t n_tiles = (M_eff + kTileM - 1) / kTileM;
-  const int64_t n_pairs = (n_tiles + 1) / 2;
+  // work list: super tile q of the persistent loop is live[q] (every role of a cluster walks the same list), or q without a list
+  const int64_t n_pairs = p.live ? (int64_t)__ldg(p.n_live) : (n_tiles + 1) / 2;
 
   if (warp == 16) {
     producer_loop<CG2>(p, sm, n_pairs);
@@ -871,18 +874,24 @@ __global__ void __launch_bounds__(kThreads, 1) tc2_bwd_kernel(const __grid_const
     EpiCtx e;
     e.lane = lane; e.hh = gw >> 2; e.row = (gw & 3u) * 32u + lane; e.lane_field = ((gw & 3u) * 32u) << 16;
     e.tmem = tmem_base + slot * 256u; e.slot = slot;
+    const uint32_t crank = cluster_ctarank();
+    // tile_index with the list: this thread's 128-row half of list entry q (pair index p0 + its slot / rank); past the list's end
+    // n_tiles (never processed, never stored)
+    auto work_tile = [&](int64_t p0) -> int64_t {
+      if (!p.live) return tile_index<CG2>(p0, crank, slot);
+      const int64_t q = p0 + (CG2 ? slot : crank);
+      return q < n_pairs ? 2 * (int64_t)__ldg(p.live + q) + (CG2 ? crank : slot) : n_tiles;
+    };
     float* colsum = sm.tab(TAB_LAT) + slot * kMaxLat * 256;
     // tile-end scratch outside the A chunks: the hh == 1 half of every row leaves its partial d xyz here.  [128][4] floats per slot.
     float* part = sm.tab(TAB_BIAS) + slot * 512u;
     const float* w2_s = sm.tab(TAB_W2);
     const int nslots = p.prog.n_mask_slots;
     uint32_t acc_cnt = 0;
-    const uint32_t crank = cluster_ctarank();
     const int64_t pair_first = (int64_t)blockIdx.x - crank;
     // upstream gradients of one tile row: d softplus-input of sigma, d rgb, and the rgb.0 ReLU mask words of this thread's columns
     const uint32_t ready_leader = CG2 ? mapa_u32(sm.bar(BAR_READY + slot), 0u) : 0u;
-    auto load_upstream = [&](int64_t p0, float& gsp_o, float (&g3o)[3], uint32_t (&mwo)[2]) {
-      const int64_t t = tile_index<CG2>(p0, crank, slot);
+    auto load_upstream = [&](int64_t t, float& gsp_o, float (&g3o)[3], uint32_t (&mwo)[2]) {
       const bool ok = t < n_tiles;
       const int64_t r = t * kTileM + e.row;
       const bool valid = ok && r < M_eff;
@@ -920,12 +929,13 @@ __global__ void __launch_bounds__(kThreads, 1) tc2_bwd_kernel(const __grid_const
     float gsp = 0.f;
     if (pair_first < n_pairs) {   // first tile of this CTA
       float g3[3]; uint32_t mw2[2];
-      load_upstream(pair_first, gsp, g3, mw2);
+      load_upstream(work_tile(pair_first), gsp, g3, mw2);
       prologue(g3, mw2);
       publish<CG2>(sm, slot, lane, ready_leader);
     }
+    int64_t tile = work_tile(pair_first);
     for (int64_t pair0 = pair_first; pair0 < n_pairs; pair0 += gridDim.x) {
-      const int64_t tile = tile_index<CG2>(pair0, crank, slot);
+      const int64_t next = work_tile(pair0 + gridDim.x);   // this slot's next tile: one list lookup per tile
       const bool tile_ok = tile < n_tiles;
       const bool has_next = pair0 + (int64_t)gridDim.x < n_pairs;   // cluster-uniform
       e.grow = tile * kTileM + e.row;
@@ -943,7 +953,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc2_bwd_kernel(const __grid_const
           for (int c = 0; c < 4; ++c) mw[c] = mask_word(mask_tile, st.mask_slot, c * 2 + (int)e.hh, e.row);
         }
         const bool last = si + 1 == p.prog.n_steps;
-        if (last && has_next) load_upstream(pair0 + gridDim.x, gsp_n, g3n, mwn);   // global latency hides behind the last MMAs
+        if (last && has_next) load_upstream(next, gsp_n, g3n, mwn);   // global latency hides behind the last MMAs
 #ifndef SNB_EXP_NO_COLSUM   // (timing experiment builds only: upper bound of what the column-sum pass costs; wrong latent gradients)
         if (st.colsum) {   // column sums of this step's A operand (published by the whole group last step), while its MMAs run
           group_bar(slot);
@@ -1014,7 +1024,6 @@ __global__ void __launch_bounds__(kThreads, 1) tc2_bwd_kernel(const __grid_const
         if (p.trace && blockIdx.x == 0 && gtid == 0) p.trace[(((pair0 / gridDim.x) * p.prog.n_steps + si) * 2 + slot) * 4 + 3] = clock64();
       }
       // ---- tile end: d xyz, and flush the latent column sums when this slot's next tile belongs to another object
-      const int64_t next = tile + 2 * (int64_t)gridDim.x;
       const bool flush = tile_ok && (next >= n_tiles || obj_of_tile(p, next) != obj);
       if (p.g_xyz != nullptr && e.hh == 1) *reinterpret_cast<float4*>(part + 4 * e.row) = make_float4(gx[0], gx[1], gx[2], 0.f);
       group_bar(slot);
@@ -1033,6 +1042,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc2_bwd_kernel(const __grid_const
         }
         group_bar(slot);
       }
+      tile = next;
     }
   }
   tc_fence_before();
@@ -1383,7 +1393,8 @@ int tc2_launch_fwd(const snb_handle_s* h, const void* packed2, const float* xyz,
 
 int tc2_launch_bwd(const snb_handle_s* h, const void* packed2, const float* xyz, const float* viewdir, int64_t M, int64_t B,
                    const uint32_t* masks, const float* sigma, const float* g_sigma, const float* g_rgb, float* g_xyz,
-                   float* g_viewdir, float* g_zlat, uint8_t* save, cudaStream_t st, const int64_t* m_dev, const int32_t* tile_start) {
+                   float* g_viewdir, float* g_zlat, uint8_t* save, cudaStream_t st, const int64_t* m_dev, const int32_t* tile_start,
+                   const int32_t* live, const int32_t* n_live) {
   const Tc2Plan& pl = cached_plan2(h);
   tc2::Params p;
   fill_common2(p, h, packed2, xyz, viewdir, M, B, nullptr, const_cast<uint32_t*>(masks));
@@ -1392,6 +1403,7 @@ int tc2_launch_bwd(const snb_handle_s* h, const void* packed2, const float* xyz,
   p.save = save;
   p.m_dev = m_dev;
   p.tile_start = tile_start;
+  p.live = live; p.n_live = n_live;
   SNB_REQUIRE(save == nullptr || g_xyz != nullptr, "tc2 backward: training mode runs the full program (g_xyz scratch required)");
   p.prog = g_xyz ? pl.bwd_full : pl.bwd_noxyz;
   if (tc2_init_device()) return 1;

@@ -12,8 +12,9 @@
 //             latent layers + tcgen05 decoder over all objects' rows (mlp_tc2.cu: per-tile object lookup through tile_start)
 //             rb_composite_fwd           compositing straight on the compact rows (hit rays: S-sample scan; miss rays: their single
 //                                         sample in closed form) -> rgb / depth / acc per ray
-//   backward  rb_composite_bwd -> decoder backward -> rb_rays_bwd (per-ray fold of d xyz / d viewdir / d z through the sampler, the
-//             slab test and get_rays; per-object fp64 block sums -> d cam_pose (B,3,4))
+//   backward  rb_composite_bwd (+ the list of live super tiles) -> decoder backward over the live super tiles only -> rb_rays_bwd
+//             (per-ray fold of d xyz / d viewdir / d z through the sampler, the slab test and get_rays; per-object fp64 block sums
+//             -> d cam_pose (B,3,4))
 //
 // plus the batched refine losses (one launch per direction for all objects).  Frozen weights, bf16 decoder (two-tile kernels).
 #include "common.cuh"
@@ -162,6 +163,50 @@ __global__ void __launch_bounds__(256) rb_gather_kernel(const float* __restrict_
   }
 }
 
+// --------------------------------------------------------------------------------------------------------------- live super tiles
+// The decoder backward is linear in (g_sigma, g_rgb) of a row: a 256-row super tile whose rows all have exactly zero upstream
+// gradients (rays the loss gives no weight, e.g. occ == 0 in the refine loss; pad rows) has exactly zero outputs.  The compositing
+// backward sets one flag byte per super tile that has a nonzero (or NaN) upstream gradient; its last block lists the flagged super
+// tiles in ascending order for the decoder backward, which runs only those.  All on the device: a captured graph replays it as is.
+struct LiveHdr { int32_t n_live; unsigned int ticket; };
+
+// rows `row` of the calling lanes: flag their super tiles where nz; one store per warp and super tile
+__device__ __forceinline__ void mark_live(uint8_t* __restrict__ live, int64_t row, bool nz) {
+  const unsigned am = __activemask();
+  const unsigned lv = __ballot_sync(am, nz);
+  if (lv == 0u) return;
+  const unsigned sup = (unsigned)(row >> 8);
+  const unsigned peers = __match_any_sync(am, sup) & lv;
+  if (nz && (unsigned)(__ffs(peers) - 1) == (threadIdx.x & 31u)) live[sup] = 1;
+}
+
+// one block of 256 threads: the flagged super tiles of [0, total_rows / 256), ascending -> list, their count -> hdr->n_live.  Each
+// thread counts a contiguous run of 4-flag words (a flag byte is 0 or 1), one block scan, then each thread writes its run's entries.
+__device__ void build_live_list(const uint8_t* __restrict__ live, int64_t total_rows, int32_t* __restrict__ list, LiveHdr* hdr) {
+  __shared__ int warp_tot[8];
+  const int n_words = (int)(((total_rows >> 8) + 3) >> 2);
+  const int per = (n_words + 255) / 256;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int w0 = tid * per, w1 = min(w0 + per, n_words);
+  const unsigned int* words = reinterpret_cast<const unsigned int*>(live);
+  int cnt = 0;
+  for (int w = w0; w < w1; ++w) cnt += __popc(__ldcg(words + w));
+  int incl = cnt;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) { const int u = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += u; }
+  if (lane == 31) warp_tot[warp] = incl;
+  __syncthreads();
+  int before = incl - cnt, total = 0;
+  for (int k = 0; k < 8; ++k) { if (k < warp) before += warp_tot[k]; total += warp_tot[k]; }
+  for (int w = w0; w < w1; ++w) {
+    const unsigned int f = __ldcg(words + w);
+#pragma unroll
+    for (int b = 0; b < 4; ++b)
+      if ((f >> (8 * b)) & 1u) list[before++] = 4 * w + b;
+  }
+  if (tid == 0) hdr->n_live = total;
+}
+
 // --------------------------------------------------------------------------------------------------------------- compositing
 // z_vals of a lane's 4 samples (+ the next one) recomputed from the ray: the forward keeps no per-row coordinates or depths in HBM
 __device__ __forceinline__ void lane_z_from_ray(const float* __restrict__ r8, const float* __restrict__ jit_row, const float* __restrict__ z_steps,
@@ -263,7 +308,9 @@ __global__ void __launch_bounds__(256) rb_composite_bwd_kernel(const float* __re
                                                               const ObjCounts* __restrict__ counts, int64_t N, int S, int flags,
                                                               const float* __restrict__ g_rgb, const float* __restrict__ g_depth,
                                                               const float* __restrict__ g_acc, float* __restrict__ g_sigma_c,
-                                                              float* __restrict__ g_rgb_c, float* __restrict__ g_z_c) {
+                                                              float* __restrict__ g_rgb_c, float* __restrict__ g_z_c,
+                                                              const int64_t* __restrict__ total_rows, uint8_t* __restrict__ live,
+                                                              int32_t* __restrict__ live_list, LiveHdr* __restrict__ live_hdr) {
   constexpr int RPW = 32 / LPR;
   const int b = blockIdx.y;
   const ObjCounts c = counts[b];
@@ -321,6 +368,10 @@ __global__ void __launch_bounds__(256) rb_composite_bwd_kernel(const float* __re
     }
     float gprev = __shfl_up_sync(0xffffffffu, gdel[3], 1, LPR);
     if (sl == 0) gprev = 0.f;
+    bool nz = false;   // the lane's 4 rows (one super tile: rows start at multiples of 4) feed the decoder a nonzero gradient
+#pragma unroll
+    for (int j = 0; j < 4; ++j) nz |= (gs[j] != 0.f) | (gcol[j][0] != 0.f) | (gcol[j][1] != 0.f) | (gcol[j][2] != 0.f);
+    mark_live(live, row0 + k0, nz && L.valid && rv);
     if (L.valid && rv) {
       *reinterpret_cast<float4*>(g_sigma_c + row0 + k0) = make_float4(gs[0], gs[1], gs[2], gs[3]);
       float* gr = g_rgb_c + (row0 + k0) * 3;
@@ -356,6 +407,19 @@ __global__ void __launch_bounds__(256) rb_composite_bwd_kernel(const float* __re
     g_sigma_c[row] = gs;
     g_rgb_c[3 * row] = r0; g_rgb_c[3 * row + 1] = r1; g_rgb_c[3 * row + 2] = r2;
     if (g_z_c != nullptr) g_z_c[row] = gz;
+    mark_live(live, row, (gs != 0.f) | (r0 != 0.f) | (r1 != 0.f) | (r2 != 0.f));
+  }
+  // the last block lists the live super tiles (every block's flags are visible: bar.sync, then a cumulative fence before the ticket)
+  __shared__ bool last;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence();
+    last = atomicAdd(&live_hdr->ticket, 1u) == gridDim.x * gridDim.y - 1;
+  }
+  __syncthreads();
+  if (last) {
+    __threadfence();
+    build_live_list(live, *total_rows, live_list, live_hdr);
   }
 }
 
@@ -373,8 +437,9 @@ __global__ void __launch_bounds__(256) rb_rays_bwd_kernel(const float* __restric
                                                          const ObjCounts* __restrict__ counts, const float* __restrict__ z_steps,
                                                          const float* __restrict__ jitter, int64_t N, int S,
                                                          const float* __restrict__ g_xyz_c, const float* __restrict__ g_vrep_c,
-                                                         const float* __restrict__ g_z_c, double* __restrict__ acc64,
-                                                         unsigned int* __restrict__ tickets, float* __restrict__ g_c2w) {
+                                                         const float* __restrict__ g_z_c, const uint8_t* __restrict__ live,
+                                                         double* __restrict__ acc64, unsigned int* __restrict__ tickets,
+                                                         float* __restrict__ g_c2w) {
   const int b = blockIdx.y;
   const ObjCounts c = counts[b];
   const float* Kb = K + 9 * b;
@@ -410,11 +475,15 @@ __global__ void __launch_bounds__(256) rb_rays_bwd_kernel(const float* __restric
             const float zs = __fadd_rn(__ldg(z_steps + k), __fmul_rn(__ldg(jitter + gi * S + k), fstep));
             const float zc = __fadd_rn(__fmul_rn(near, __fsub_rn(1.f, zs)), __fmul_rn(far, zs));
             const int64_t gidx = c.row_start + (int64_t)p * S + k;
-            const float gx[3] = {__ldg(g_xyz_c + 3 * gidx), __ldg(g_xyz_c + 3 * gidx + 1), __ldg(g_xyz_c + 3 * gidx + 2)};
+            // a row of a super tile the decoder skipped has d xyz = d viewdir = 0 (its scratch rows hold an older call's values);
+            // d z comes from the compositing backward and is always read.  Per row: a ray can span two super tiles.
+            const bool lv = __ldg(live + (gidx >> 8)) != 0;
+            const float gx[3] = {lv ? __ldg(g_xyz_c + 3 * gidx) : 0.f, lv ? __ldg(g_xyz_c + 3 * gidx + 1) : 0.f,
+                                 lv ? __ldg(g_xyz_c + 3 * gidx + 2) : 0.f};
             float gz = gx[0] * d[0] + gx[1] * d[1] + gx[2] * d[2];
 #pragma unroll
             for (int a = 0; a < 3; ++a) { v[a] += gx[a]; v[3 + a] += zc * gx[a]; }
-            v[3] += __ldg(g_vrep_c + 3 * gidx); v[4] += __ldg(g_vrep_c + 3 * gidx + 1); v[5] += __ldg(g_vrep_c + 3 * gidx + 2);
+            if (lv) { v[3] += __ldg(g_vrep_c + 3 * gidx); v[4] += __ldg(g_vrep_c + 3 * gidx + 1); v[5] += __ldg(g_vrep_c + 3 * gidx + 2); }
             if (g_z_c != nullptr) {
               const float gv = __ldg(g_z_c + gidx);
               const float sgn = (zc > 0.f) ? 1.f : ((zc < 0.f) ? -1.f : 0.f);
@@ -430,11 +499,13 @@ __global__ void __launch_bounds__(256) rb_rays_bwd_kernel(const float* __restric
           const float zs = __fadd_rn(__ldg(z_steps + k), __fmul_rn(__ldg(jitter + gi * S + k), fstep));
           const float zc = __fadd_rn(__fmul_rn(near, __fsub_rn(1.f, zs)), __fmul_rn(far, zs));
           const int64_t gidx = c.row_start + c.n_hit * S + p;
-          const float gx[3] = {__ldg(g_xyz_c + 3 * gidx), __ldg(g_xyz_c + 3 * gidx + 1), __ldg(g_xyz_c + 3 * gidx + 2)};
+          const bool lv = __ldg(live + (gidx >> 8)) != 0;
+          const float gx[3] = {lv ? __ldg(g_xyz_c + 3 * gidx) : 0.f, lv ? __ldg(g_xyz_c + 3 * gidx + 1) : 0.f,
+                               lv ? __ldg(g_xyz_c + 3 * gidx + 2) : 0.f};
           float gz = gx[0] * d[0] + gx[1] * d[1] + gx[2] * d[2];
 #pragma unroll
           for (int a = 0; a < 3; ++a) { v[a] = gx[a]; v[3 + a] = zc * gx[a]; }
-          v[3] += __ldg(g_vrep_c + 3 * gidx); v[4] += __ldg(g_vrep_c + 3 * gidx + 1); v[5] += __ldg(g_vrep_c + 3 * gidx + 2);
+          if (lv) { v[3] += __ldg(g_vrep_c + 3 * gidx); v[4] += __ldg(g_vrep_c + 3 * gidx + 1); v[5] += __ldg(g_vrep_c + 3 * gidx + 2); }
           if (g_z_c != nullptr) {
             const float gv = __ldg(g_z_c + gidx);
             const float sgn = (zc > 0.f) ? 1.f : ((zc < 0.f) ? -1.f : 0.f);
@@ -769,9 +840,10 @@ struct BatchLayout {
 };
 
 // backward scratch: the executed rows' coordinates and depths are re-materialised here (rb_gather_kernel: the decoder backward folds
-// d PE through sin / cos of the coordinates), then the gradients
+// d PE through sin / cos of the coordinates), then the gradients, the live super tiles (header + one flag byte each, zeroed together;
+// the list)
 struct BatchScratch {
-  size_t xyz_c, vrep_c, z_c, g_sigma_c, g_rgb_c, g_z_c, g_xyz_c, g_vrep_c, acc64, tickets, mlp, total;
+  size_t xyz_c, vrep_c, z_c, g_sigma_c, g_rgb_c, g_z_c, g_xyz_c, g_vrep_c, live_hdr, live, live_end, live_list, acc64, tickets, mlp, total;
   BatchScratch(snb_handle h, const snb_batch_desc& d, int64_t Mmax) {
     const size_t M = (size_t)Mmax, B = (size_t)d.n_objs;
     size_t o = 0;
@@ -784,6 +856,11 @@ struct BatchScratch {
     g_z_c = o; o += al(M * 4);
     g_xyz_c = o; o += al(M * 12);
     g_vrep_c = o; o += al(M * 12);
+    const size_t n_super = M / 256;
+    live_hdr = o; o += al(sizeof(rb::LiveHdr));
+    live = o; o += al(n_super);
+    live_end = o;
+    live_list = o; o += al(n_super * 4);
     acc64 = o; o += al(B * 12 * 8);
     tickets = o; o += al(B * 4);
     mlp = o; o += al(decoder_scratch_bytes(h, batch_precision(d), Mmax, (int64_t)B));
@@ -931,16 +1008,19 @@ extern "C" int snb_render_batch_bwd(snb_handle h, const snb_batch_desc* d, const
     SNB_LAUNCH_CHECK();
     xyz_c = at<float>(sc, G.xyz_c); vrep_c = at<float>(sc, G.vrep_c); z_c = at<float>(sc, G.z_c);
   }
+  const int64_t* total_rows = &at<rb::Meta>(ws, L.meta)->total_rows;
+  SNB_CHECK_CUDA(cudaMemsetAsync(at<uint8_t>(sc, G.live_hdr), 0, G.live_end - G.live_hdr, st));   // count, ticket, flags
 #define SNB_RBB(LL) rb::rb_composite_bwd_kernel<LL><<<grid, 256, 0, st>>>(at<float>(ws, L.sigma_c), at<float>(ws, L.rgb_c), z_c, \
     at<int32_t>(ws, L.order), at<rb::ObjCounts>(ws, L.counts), N, S, d->flags, g_rgb, g_depth, g_acc, at<float>(sc, G.g_sigma_c), \
-    at<float>(sc, G.g_rgb_c), gz)
+    at<float>(sc, G.g_rgb_c), gz, total_rows, at<uint8_t>(sc, G.live), at<int32_t>(sc, G.live_list), at<rb::LiveHdr>(sc, G.live_hdr))
   if (lpr == 8) SNB_RBB(8); else if (lpr == 16) SNB_RBB(16); else SNB_RBB(32);
 #undef SNB_RBB
   SNB_LAUNCH_CHECK();
   if (decoder_backward(h, batch_precision(*d), xyz_c, vrep_c, L.Mmax, B, shape_latent, texture_latent, at<float>(ws, L.sigma_c),
                        at<float>(sc, G.g_sigma_c), at<float>(sc, G.g_rgb_c), at<uint8_t>(ws, L.mlp), at<uint8_t>(sc, G.mlp),
                        pose ? at<float>(sc, G.g_xyz_c) : nullptr, pose ? at<float>(sc, G.g_vrep_c) : nullptr, g_shape_latent, g_texture_latent,
-                       nullptr, st, {&at<rb::Meta>(ws, L.meta)->total_rows, at<int32_t>(ws, L.tile_start)}))
+                       nullptr, st, {total_rows, at<int32_t>(ws, L.tile_start), nullptr, at<int32_t>(sc, G.live_list),
+                                     &at<rb::LiveHdr>(sc, G.live_hdr)->n_live}))
     return 1;
   if (!pose) return 0;
   SNB_CHECK_CUDA(cudaMemsetAsync(at<uint8_t>(sc, G.acc64), 0, G.mlp - G.acc64, st));   // fp64 sums + tickets
@@ -949,7 +1029,7 @@ extern "C" int snb_render_batch_bwd(snb_handle h, const snb_batch_desc* d, const
   if (gr < 1) gr = 1;
   rb::rb_rays_bwd_kernel<<<dim3((unsigned)gr, (unsigned)B), 256, 0, st>>>(px, py, K, c2w, box, at<float>(ws, L.rays8), at<uint8_t>(ws, L.hit),
       at<int32_t>(ws, L.pos), at<rb::ObjCounts>(ws, L.counts), z_steps, jitter, N, S, at<float>(sc, G.g_xyz_c), at<float>(sc, G.g_vrep_c), gz,
-      at<double>(sc, G.acc64), at<unsigned int>(sc, G.tickets), g_c2w);
+      at<uint8_t>(sc, G.live), at<double>(sc, G.acc64), at<unsigned int>(sc, G.tickets), g_c2w);
   SNB_LAUNCH_CHECK();
   return 0;
 }
