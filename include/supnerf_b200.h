@@ -33,7 +33,7 @@ extern "C" {
 #define SNB_PREC_BF16 1 /* tcgen05 bf16 x bf16 -> fp32 TMEM accumulators: the 2e-2 throughput mode (weights frozen) */
 #define SNB_PREC_BF16_TRAIN 2 /* the same arithmetic; the forward/backward additionally keep every layer's operand tiles in the
                                  workspace / scratch so that snb_mlp_bwd can produce all weight gradients on the tensor core */
-#define SNB_PREC_FP32_TC 3 /* the 1e-5 parity mode on the tensor cores (weights frozen; CodeNeRF family, W = 256): every MMA operand
+#define SNB_PREC_FP32_TC 3 /* the 1e-5 parity mode on the tensor cores (weights frozen; CodeNeRF family, W = 128 or 256): every MMA operand
                               is held as two fp16 parts (x = hi + lo) and every product issued as three tcgen05 MMAs into fp32 TMEM
                               accumulators; biases, latent layers, heads and reductions stay fp32 FFMA.  Errors against the fp64
                               oracle on par with SNB_PREC_FP32; valid for |weight| < 255 and |activation| < 65504 (beyond: inf / NaN).

@@ -35,7 +35,7 @@ static inline size_t al1k(size_t b) { return (b + 1023) & ~size_t(1023); }
 static inline uint8_t* align1k(uint8_t* p) { return (uint8_t*)(((uintptr_t)p + 1023) & ~uintptr_t(1023)); }
 
 // Workspace and backward scratch of the tensor-core back ends (byte offsets):
-//   workspace  zlat (Bs+Bt)*B*256 fp32 | effective biases (same) | their bias-stage images, 32 B per unit | ReLU masks, 1 bit per unit
+//   workspace  zlat (Bs+Bt)*B*W fp32 | effective biases (same) | their bias-stage images, 32 B per unit | ReLU masks, 1 bit per unit
 //              | training: the forward's operand tiles (1 KB aligned in memory)
 //   scratch    latent column sums (zlat's shape) | their W^T fold | training: the backward's operand tiles (1 KB aligned), then a
 //              d xyz / d viewdir dummy (the training backward always runs the full program)
@@ -44,14 +44,14 @@ struct TcLayout {
   size_t fold, bsave, sc_bytes;
   bool train;
   TcLayout(const snb_handle_s* h, int32_t precision, int64_t M, int64_t B) {
-    const int slots = h->arch.shape_blocks + h->arch.texture_blocks;
+    const int slots = h->arch.shape_blocks + h->arch.texture_blocks, W = h->arch.W;
     const size_t tiles = (size_t)((M + tc::kTileM - 1) / tc::kTileM);
     train = precision == SNB_PREC_BF16_TRAIN && tc2_supported(h);
-    zlat_bytes = (size_t)slots * B * 256 * sizeof(float);
+    zlat_bytes = (size_t)slots * B * W * sizeof(float);
     ebias = zlat_bytes;
     eimg = al256(2 * zlat_bytes);
     masks = al256(eimg + 8 * zlat_bytes);
-    fsave = masks + tiles * (slots + 3) * 8 * 128 * 4 + 256;
+    fsave = masks + tiles * (slots + 3) * (W / 32) * 128 * 4 + 256;
     ws_bytes = fsave + (train ? tc2_fwd_save_bytes(h, M) + 1024 : 0);
     fold = zlat_bytes;
     bsave = al256(2 * zlat_bytes) + 256;

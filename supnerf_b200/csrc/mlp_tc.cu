@@ -7,7 +7,9 @@
 // images) is streamed from L2 by the bulk-copy engine (cp.async.bulk + mbarrier) through a 3-stage
 // ring.  Accumulators ping-pong between the two 256-column halves of TMEM so that the epilogue of
 // layer l (bias, ReLU, latent add, mask bits, bf16 pack) overlaps the MMAs of layer l+1 chunk by
-// chunk.  The 256->1 (sigma) and 128->3 (rgb) heads run on CUDA cores inside the epilogues.
+// chunk.  The W->1 (sigma) and W/2->3 (rgb) heads run on CUDA cores inside the epilogues.
+// The hidden width W (128 or 256) is a template parameter of the kernels: W / 64 K chunks per hidden layer, W / 32 ReLU-mask words
+// per layer.  Shared-memory tables keep a row stride of 256 at either width.
 // Backward: same machinery with transposed weight images; ReLU masks come back as 1 bit/unit;
 // latent gradients are per-object column sums reduced by warp butterflies; d(PE) is folded to
 // d xyz / d viewdir in the epilogue.
@@ -25,7 +27,6 @@
 #include <math.h>
 #include <algorithm>
 #include <stdlib.h>
-#include <initializer_list>
 #include <vector>
 
 namespace snb {
@@ -102,14 +103,14 @@ struct Params {
   const float* xyz; const float* viewdir;
   int64_t M, rows_per_obj, B;
   const uint8_t* packed;
-  const float* zlat;            // fwd: per-object effective biases b + W z, [(Bs+Bt)][B][256]; bwd: unused
+  const float* zlat;            // fwd: per-object effective biases b + W z, [(Bs+Bt)][B][W]; bwd: unused
   const float* wsig; const float* bsig; const float* w2; const float* b2;
-  uint32_t* masks;              // [tile][slot][8 words][128 rows]
+  uint32_t* masks;              // [tile][slot][W / 32 words][128 rows]
   // forward
   float* sigma; float* rgb; float* dbg;
   // backward
   const float* sigma_in; const float* g_sigma; const float* g_rgb;
-  float* g_xyz; float* g_viewdir; float* g_zlat;   // g_zlat [(Bs+Bt)][B][256], accumulated with atomics
+  float* g_xyz; float* g_viewdir; float* g_zlat;   // g_zlat [(Bs+Bt)][B][W], accumulated with atomics
   int r0_mask_slot, n_latent, ev_step;
   const int64_t* m_dev;         // device-side row count (a multiple of 128, <= M) or null
   const int32_t* tile_start;    // per-object first tile (B + 1 ints) or null = M / B rows per object
@@ -348,11 +349,11 @@ __device__ __forceinline__ void kernel_prologue(SmemT<X>& sm, uint8_t* smem_raw,
 // One layer's epilogue for this thread's row: TMEM -> (+bias, ReLU, mask bits, +latent) -> bf16 -> shared-memory A operand.
 // The TMEM load of chunk c+1 is in flight while chunk c is processed.  Split mode: accumulators carry the weight scale; the bias /
 // per-object effective bias is read through L1 from `bias_g` (every lane of a warp reads the same address).
-template <int EPI, bool LAT, bool DBG, bool X>
+template <int EPI, bool LAT, bool DBG, bool X, int W>
 __device__ __forceinline__ void fwd_epilogue(const Params& p, const SmemT<X>& sm, const Step& st, int si, uint32_t half, const EpiCtx& e,
                                              uint32_t* mask_tile, float& sig_acc, float (&rgb_acc)[3], const float* bias_g) {
   using MP = Map<X>;
-  constexpr int NC = (EPI == EPI_RGB_HEAD) ? 2 : 4;
+  constexpr int NC = (EPI == EPI_RGB_HEAD ? W / 2 : W) / 64;   // 64-column chunks of the layer's outputs
   // latent-conditioned layers read their per-object EFFECTIVE bias  b + W z_obj  (the latent add folded through the layer)
   const float* bias_s = X ? bias_g : (LAT ? sm.tab(MP::TAB_Z) + st.latent_slot * 256 : sm.tab(MP::TAB_BIAS) + si * 256);
   const float* wsig_s = sm.tab(MP::TAB_WSIG);
@@ -390,7 +391,7 @@ __device__ __forceinline__ void fwd_epilogue(const Params& p, const SmemT<X>& sm
       if (EPI == EPI_RGB_HEAD) {
 #pragma unroll
         for (int k = 0; k < 3; ++k) {
-          const float4 ww = *reinterpret_cast<const float4*>(w2_s + k * 128 + col0 + 4 * i4);
+          const float4 ww = *reinterpret_cast<const float4*>(w2_s + k * (W / 2) + col0 + 4 * i4);
           rgb_acc[k] += fmaxf(v[0], 0.f) * ww.x + fmaxf(v[1], 0.f) * ww.y + fmaxf(v[2], 0.f) * ww.z + fmaxf(v[3], 0.f) * ww.w;
         }
       }
@@ -410,7 +411,7 @@ __device__ __forceinline__ void fwd_epilogue(const Params& p, const SmemT<X>& sm
       }
     }
     const uint32_t mask = ~nmask;
-    if (EPI != EPI_LINEAR_SIGMA) mask_tile[((size_t)st.mask_slot * 8 + c * 2 + e.hh) * 128 + e.row] = mask;
+    if (EPI != EPI_LINEAR_SIGMA) mask_tile[((size_t)st.mask_slot * (W / 32) + c * 2 + e.hh) * 128 + e.row] = mask;
     if (EPI != EPI_RGB_HEAD) {
       rp.store(sm, c, e.row, e.hh);
       publish_chunk(sm, c, e.lane);
@@ -418,22 +419,22 @@ __device__ __forceinline__ void fwd_epilogue(const Params& p, const SmemT<X>& sm
   }
 }
 
-template <bool DBG, bool X>
+template <bool DBG, bool X, int W>
 __device__ __forceinline__ void fwd_epilogue_dispatch(const Params& p, const SmemT<X>& sm, const Step& st, int si, uint32_t half,
                                                       const EpiCtx& e, uint32_t* mask_tile, float& sig_acc, float (&rgb_acc)[3],
                                                       const float* bias_g) {
   if (st.epi == EPI_RELU) {
-    if (st.latent_slot >= 0) fwd_epilogue<EPI_RELU, true, DBG, X>(p, sm, st, si, half, e, mask_tile, sig_acc, rgb_acc, bias_g);
-    else fwd_epilogue<EPI_RELU, false, DBG, X>(p, sm, st, si, half, e, mask_tile, sig_acc, rgb_acc, bias_g);
+    if (st.latent_slot >= 0) fwd_epilogue<EPI_RELU, true, DBG, X, W>(p, sm, st, si, half, e, mask_tile, sig_acc, rgb_acc, bias_g);
+    else fwd_epilogue<EPI_RELU, false, DBG, X, W>(p, sm, st, si, half, e, mask_tile, sig_acc, rgb_acc, bias_g);
   } else if (st.epi == EPI_LINEAR_SIGMA) {
-    fwd_epilogue<EPI_LINEAR_SIGMA, false, DBG, X>(p, sm, st, si, half, e, mask_tile, sig_acc, rgb_acc, bias_g);
+    fwd_epilogue<EPI_LINEAR_SIGMA, false, DBG, X, W>(p, sm, st, si, half, e, mask_tile, sig_acc, rgb_acc, bias_g);
   } else {
-    fwd_epilogue<EPI_RGB_HEAD, false, DBG, X>(p, sm, st, si, half, e, mask_tile, sig_acc, rgb_acc, bias_g);
+    fwd_epilogue<EPI_RGB_HEAD, false, DBG, X, W>(p, sm, st, si, half, e, mask_tile, sig_acc, rgb_acc, bias_g);
   }
 }
 
 // ------------------------------------------------------------------------------------------ forward kernel
-template <bool X>
+template <bool X, int W>
 __global__ void __launch_bounds__(kThreads, 1) tc_fwd_kernel(const __grid_constant__ Params p) {
   using MP = Map<X>;
   extern __shared__ uint8_t smem_raw[];
@@ -452,9 +453,9 @@ __global__ void __launch_bounds__(kThreads, 1) tc_fwd_kernel(const __grid_consta
       }
     }
     float* wsig_s = reinterpret_cast<float*>(b + MP::SM_TAB + MP::TAB_WSIG);
-    for (int i = tid; i < 256; i += kThreads) wsig_s[i] = __ldg(p.wsig + i);
+    for (int i = tid; i < W; i += kThreads) wsig_s[i] = __ldg(p.wsig + i);
     float* w2_s = reinterpret_cast<float*>(b + MP::SM_TAB + MP::TAB_W2);
-    for (int i = tid; i < 384; i += kThreads) w2_s[i] = __ldg(p.w2 + i);
+    for (int i = tid; i < 3 * W / 2; i += kThreads) w2_s[i] = __ldg(p.w2 + i);
   }
   kernel_prologue(sm, smem_raw, tid, warp, tmem_base);
   const int64_t M = rows_present(p);
@@ -488,35 +489,39 @@ __global__ void __launch_bounds__(kThreads, 1) tc_fwd_kernel(const __grid_consta
       const int64_t crow = e.valid ? e.grow : M - 1;
       const int64_t next_tile = tile + gridDim.x;
       float xn[3] = {0.f, 0.f, 0.f};
-      if (next_tile < n_tiles) {  // prefetch the next tile's coordinates: consumed ~5 layers from now
+      // the next tile's coordinates, consumed by the encoding_viewdir epilogue.  W = 256: prefetched here, ~5 layers ahead.  W = 128:
+      // loaded while that layer's MMAs run (holding them from here made the split-precision forward spill 52 more bytes)
+      auto load_xn = [&] {
         int64_t rn = next_tile * kTileM + e.row;
         if (rn > M - 1) rn = M - 1;
         xn[0] = __ldg(p.xyz + 3 * rn); xn[1] = __ldg(p.xyz + 3 * rn + 1); xn[2] = __ldg(p.xyz + 3 * rn + 2);
-      }
+      };
+      if (W == 256 && next_tile < n_tiles) load_xn();
       const float dir[3] = {__ldg(p.viewdir + 3 * crow), __ldg(p.viewdir + 3 * crow + 1), __ldg(p.viewdir + 3 * crow + 2)};
       const int64_t obj = obj_of_tile(p, tile);   // tiles never straddle objects (checked on the host)
       if (obj != cur_obj) {  // (re)load the per-object effective biases; all epilogue warps are between tiles here
         cur_obj = obj;
         if (!X) {
-          for (int i = tid; i < p.n_latent * 256; i += 256)
-            z_s[i] = __ldg(p.zlat + ((size_t)(i >> 8) * p.B + obj) * 256 + (i & 255));
+          for (int i = tid; i < p.n_latent * 256; i += 256)   // [slot][256] in shared memory; column tid
+            if (W == 256 || tid < W) z_s[i] = __ldg(p.zlat + ((size_t)(i >> 8) * p.B + obj) * W + (i & 255));
         } else {   // split mode: into the latent-conditioned steps' rows of the bias table
           float* bias_tab = sm.tab(MP::TAB_BIAS);
           for (int si = 0; si < p.prog.n_steps && si < kSplitBiasSteps; ++si) {
             const int slot = p.prog.s[si].latent_slot;
-            if (slot >= 0) bias_tab[si * 256 + tid] = __ldg(p.zlat + ((size_t)slot * p.B + obj) * 256 + tid);
+            if (slot >= 0 && (W == 256 || tid < W)) bias_tab[si * 256 + tid] = __ldg(p.zlat + ((size_t)slot * p.B + obj) * W + tid);
           }
         }
         epi_bar_sync();
       }
-      uint32_t* mask_tile = p.masks + (size_t)tile * nslots * 8 * 128;
+      uint32_t* mask_tile = p.masks + (size_t)tile * nslots * (W / 32) * 128;
       float sig_acc = 0.f, rgb_acc[3] = {0.f, 0.f, 0.f};
       for (int si = 0; si < p.prog.n_steps; ++si, ++gstep) {
         const Step& st = p.prog.s[si];
         const uint32_t half = gstep & 1u;
         const float* bias_g = nullptr;   // split mode: the step's (effective) bias, from the shared-memory table or through L1
         if (X) bias_g = si < kSplitBiasSteps ? sm.tab(MP::TAB_BIAS) + si * 256
-                                             : (st.latent_slot >= 0 ? p.zlat + ((size_t)st.latent_slot * p.B + obj) * 256 : st.bias);
+                                             : (st.latent_slot >= 0 ? p.zlat + ((size_t)st.latent_slot * p.B + obj) * W : st.bias);
+        if (W == 128 && si == p.ev_step && next_tile < n_tiles) load_xn();
         mbar_wait(sm.bar(BAR_ACC + half), acc_cnt[half] & 1u);
         acc_cnt[half]++;
         tc_fence_after();
@@ -527,8 +532,8 @@ __global__ void __launch_bounds__(kThreads, 1) tc_fwd_kernel(const __grid_consta
           write_pe<10, X>(sm, e.row, e.hh, xn);
           publish_chunk(sm, 4, lane);
         }
-        if (p.dbg != nullptr) fwd_epilogue_dispatch<true, X>(p, sm, st, si, half, e, mask_tile, sig_acc, rgb_acc, bias_g);
-        else fwd_epilogue_dispatch<false, X>(p, sm, st, si, half, e, mask_tile, sig_acc, rgb_acc, bias_g);
+        if (p.dbg != nullptr) fwd_epilogue_dispatch<true, X, W>(p, sm, st, si, half, e, mask_tile, sig_acc, rgb_acc, bias_g);
+        else fwd_epilogue_dispatch<false, X, W>(p, sm, st, si, half, e, mask_tile, sig_acc, rgb_acc, bias_g);
         tc_fence_before();
       }
       sig_part[e.hh * 128 + e.row] = sig_acc;
@@ -551,8 +556,9 @@ __global__ void __launch_bounds__(kThreads, 1) tc_fwd_kernel(const __grid_consta
 }
 
 // ------------------------------------------------------------------------------------------ backward epilogues
+template <int W>
 __device__ __forceinline__ uint32_t mask_word(const uint32_t* mask_tile, int slot, int word, uint32_t row) {
-  return __ldg(mask_tile + ((size_t)slot * 8 + word) * 128 + row);
+  return __ldg(mask_tile + ((size_t)slot * (W / 32) + word) * 128 + row);
 }
 
 // acc = gradient w.r.t. the layer's input.  Optional: per-object column sums of it (latent gradient); then mask by the
@@ -561,10 +567,11 @@ __device__ __forceinline__ uint32_t mask_word(const uint32_t* mask_tile, int slo
 // shrink (or grow) by a factor per layer, and an fp16 pair only resolves 2^-25 absolutely, so every layer re-centres the row: both
 // threads of a row read the same 32 sample columns of the accumulator, take the power of two that brings their largest magnitude
 // to [4, 8) (13 bits of headroom above the sample for the other columns) and fold it into rexp -- exact, and identical in both threads.
-template <bool EV, bool COLSUM, bool MASK, bool PRODUCE, bool X>
+template <bool EV, bool COLSUM, bool MASK, bool PRODUCE, bool X, int W>
 __device__ __forceinline__ void bwd_epilogue(const SmemT<X>& sm, const Step& st, uint32_t half, const EpiCtx& e,
                                              const uint32_t* mask_tile, float gsp, int& rexp) {
   using MP = Map<X>;
+  constexpr int NC = W / 64;
   const float* wsig_s = sm.tab(MP::TAB_WSIG);
   float* colsum = sm.tab(MP::TAB_BIAS);
   const uint32_t t0 = e.tmem_base + half * 256u + e.hh * 32u + e.lane_field;
@@ -596,14 +603,14 @@ __device__ __forceinline__ void bwd_epilogue(const SmemT<X>& sm, const Step& st,
   }
   tmem_ld32_issue(t0, ra);
   uint32_t mw_next = 0xffffffffu;
-  if (MASK) mw_next = mask_word(mask_tile, st.mask_slot, (int)e.hh, e.row);
+  if (MASK) mw_next = mask_word<W>(mask_tile, st.mask_slot, (int)e.hh, e.row);
 #pragma unroll
-  for (int c = 0; c < 4; ++c) {
+  for (int c = 0; c < NC; ++c) {
     uint32_t (&r)[32] = (c & 1) ? rb : ra;
     tmem_ld_wait();
-    if (c + 1 < 4) tmem_ld32_issue(t0 + (uint32_t)(c + 1) * 64u, (c & 1) ? ra : rb);
+    if (c + 1 < NC) tmem_ld32_issue(t0 + (uint32_t)(c + 1) * 64u, (c & 1) ? ra : rb);
     const uint32_t mw = mw_next;
-    if (MASK && c + 1 < 4) mw_next = mask_word(mask_tile, st.mask_slot, (c + 1) * 2 + (int)e.hh, e.row);
+    if (MASK && c + 1 < NC) mw_next = mask_word<W>(mask_tile, st.mask_slot, (c + 1) * 2 + (int)e.hh, e.row);
     const int col0 = c * 64 + (int)e.hh * 32;
     float v[32];
 #pragma unroll
@@ -638,21 +645,21 @@ __device__ __forceinline__ void bwd_epilogue(const SmemT<X>& sm, const Step& st,
   }
 }
 
-template <bool X>
+template <bool X, int W>
 __device__ __forceinline__ void bwd_epilogue_dispatch(const SmemT<X>& sm, const Step& st, uint32_t half, const EpiCtx& e,
                                                       const uint32_t* mask_tile, float gsp, int& rexp) {
   if (st.epi == EPI_B_EV) {
-    bwd_epilogue<true, false, false, true, X>(sm, st, half, e, mask_tile, gsp, rexp);
+    bwd_epilogue<true, false, false, true, X, W>(sm, st, half, e, mask_tile, gsp, rexp);
   } else if (st.latent_slot >= 0) {
-    if (st.produce_a) bwd_epilogue<false, true, true, true, X>(sm, st, half, e, mask_tile, gsp, rexp);
-    else bwd_epilogue<false, true, false, false, X>(sm, st, half, e, mask_tile, gsp, rexp);
+    if (st.produce_a) bwd_epilogue<false, true, true, true, X, W>(sm, st, half, e, mask_tile, gsp, rexp);
+    else bwd_epilogue<false, true, false, false, X, W>(sm, st, half, e, mask_tile, gsp, rexp);
   } else {
-    bwd_epilogue<false, false, true, true, X>(sm, st, half, e, mask_tile, gsp, rexp);
+    bwd_epilogue<false, false, true, true, X, W>(sm, st, half, e, mask_tile, gsp, rexp);
   }
 }
 
 // ------------------------------------------------------------------------------------------ backward kernel
-template <bool X>
+template <bool X, int W>
 __global__ void __launch_bounds__(kThreads, 1) tc_bwd_kernel(const __grid_constant__ Params p) {
   using MP = Map<X>;
   extern __shared__ uint8_t smem_raw[];
@@ -665,9 +672,9 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bwd_kernel(const __grid_consta
     float* colsum0 = reinterpret_cast<float*>(b + MP::SM_TAB + MP::TAB_BIAS);
     for (uint32_t i = tid; i < kMaxLatentSlots * 256; i += kThreads) colsum0[i] = 0.f;
     float* wsig_s = reinterpret_cast<float*>(b + MP::SM_TAB + MP::TAB_WSIG);
-    for (int i = tid; i < 256; i += kThreads) wsig_s[i] = __ldg(p.wsig + i);
+    for (int i = tid; i < W; i += kThreads) wsig_s[i] = __ldg(p.wsig + i);
     float* w2_s = reinterpret_cast<float*>(b + MP::SM_TAB + MP::TAB_W2);
-    for (int i = tid; i < 384; i += kThreads) w2_s[i] = __ldg(p.w2 + i);
+    for (int i = tid; i < 3 * W / 2; i += kThreads) w2_s[i] = __ldg(p.w2 + i);
   }
   kernel_prologue(sm, smem_raw, tid, warp, tmem_base);
   const int64_t M = rows_present(p);
@@ -692,7 +699,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bwd_kernel(const __grid_consta
       e.valid = e.grow < M;
       const int64_t crow = e.valid ? e.grow : M - 1;
       const int64_t obj = obj_of_tile(p, tile);  // tiles never straddle objects (checked on the host)
-      const uint32_t* mask_tile = p.masks + (size_t)tile * nslots * 8 * 128;
+      const uint32_t* mask_tile = p.masks + (size_t)tile * nslots * (W / 32) * 128;
       const float gsg = e.valid ? __ldg(p.g_sigma + e.grow) : 0.f;
       float gsp = gsg * (-expm1f(-__ldg(p.sigma_in + crow)));   // d softplus = 1 - exp(-softplus)
       float g3[3] = {0.f, 0.f, 0.f};
@@ -711,18 +718,18 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bwd_kernel(const __grid_consta
           g3[0] *= inv; g3[1] *= inv; g3[2] *= inv;
         }
       }
-      // ---- prologue: d pre-activation of rgb.0 = (g_rgb W2) * mask -> A chunks 0,1 (128 columns)
+      // ---- prologue: d pre-activation of rgb.0 = (g_rgb W2) * mask -> A chunks 0 .. W / 128 - 1 (W / 2 columns)
       {
 #pragma unroll
-        for (int c = 0; c < 2; ++c) {
+        for (int c = 0; c < W / 128; ++c) {
           const int col0 = c * 64 + (int)e.hh * 32;
-          const uint32_t mw = mask_word(mask_tile, p.r0_mask_slot, c * 2 + e.hh, e.row);
+          const uint32_t mw = mask_word<W>(mask_tile, p.r0_mask_slot, c * 2 + e.hh, e.row);
           RowPack<X> rp;
 #pragma unroll
           for (int i4 = 0; i4 < 8; ++i4) {
             const float4 w0 = *reinterpret_cast<const float4*>(w2_s + col0 + 4 * i4);
-            const float4 w1 = *reinterpret_cast<const float4*>(w2_s + 128 + col0 + 4 * i4);
-            const float4 w2 = *reinterpret_cast<const float4*>(w2_s + 256 + col0 + 4 * i4);
+            const float4 w1 = *reinterpret_cast<const float4*>(w2_s + W / 2 + col0 + 4 * i4);
+            const float4 w2 = *reinterpret_cast<const float4*>(w2_s + W + col0 + 4 * i4);
             float v[4] = {g3[0] * w0.x + g3[1] * w1.x + g3[2] * w2.x, g3[0] * w0.y + g3[1] * w1.y + g3[2] * w2.y,
                           g3[0] * w0.z + g3[1] * w1.z + g3[2] * w2.z, g3[0] * w0.w + g3[1] * w1.w + g3[2] * w2.w};
 #pragma unroll
@@ -789,7 +796,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bwd_kernel(const __grid_consta
             p.g_viewdir[3 * e.grow] = g[0] * out_scale; p.g_viewdir[3 * e.grow + 1] = g[1] * out_scale; p.g_viewdir[3 * e.grow + 2] = g[2] * out_scale;
           }
         }
-        bwd_epilogue_dispatch<X>(sm, st, half, e, mask_tile, gsp, rexp);
+        bwd_epilogue_dispatch<X, W>(sm, st, half, e, mask_tile, gsp, rexp);
         tc_fence_before();
       }
       // ---- tile end: d xyz, and flush the latent column sums when the next tile belongs to another object
@@ -803,7 +810,7 @@ __global__ void __launch_bounds__(kThreads, 1) tc_bwd_kernel(const __grid_consta
       if (flush) {
         for (int sl = 0; sl < p.n_latent; ++sl) {
           const float v = colsum[sl * 256 + tid];
-          if (v != 0.f) atomicAdd(p.g_zlat + ((size_t)sl * p.B + obj) * 256 + tid, v);
+          if (v != 0.f && (W == 256 || tid < W)) atomicAdd(p.g_zlat + ((size_t)sl * p.B + obj) * W + tid, v);
           colsum[sl * 256 + tid] = 0.f;
         }
       }
@@ -853,7 +860,7 @@ using namespace tc;
 bool tc1_supported(const snb_handle_s* h, const char** why) {
   const snb_arch& a = h->arch;
   if (a.arch != SNB_ARCH_CODENERF) { *why = "bf16 mode covers the CodeNeRF/AutoRFMix/SUPNeRF decoder only"; return false; }
-  if (a.W != 256) { *why = "bf16 mode needs W == 256"; return false; }
+  if (a.W != 128 && a.W != 256) { *why = "the tensor-core back ends need W == 128 or W == 256"; return false; }
   if (a.num_xyz_freq != 10 || a.num_dir_freq != 4) { *why = "bf16 mode needs num_xyz_freq == 10 and num_dir_freq == 4"; return false; }
   if (a.shape_blocks + a.texture_blocks > kMaxLatentSlots) { *why = "the tensor-core back ends need shape_blocks + texture_blocks <= 10"; return false; }
   return true;
@@ -904,10 +911,11 @@ static void add_chunks(TcPlan& pl, const float* src, int ld, bool transposed, in
   add_chunk_list(pl, chunks, ld, transposed, n_valid, n_pad, first_off);
 }
 
-static Step make_step(int epi, int n_out, int n_chunks, std::initializer_list<int> chunks, int mask_slot, int latent_slot,
-                      int produce_a, const float* bias) {
+// chunks: the shared-memory A chunk of each K chunk, in order
+static Step make_step(int epi, int n_out, const std::vector<int>& chunks, int mask_slot, int latent_slot, int produce_a,
+                      const float* bias) {
   Step s{};
-  s.epi = (int8_t)epi; s.n_out = (uint16_t)n_out; s.n_chunks = (uint16_t)n_chunks; s.mask_slot = (int8_t)mask_slot;
+  s.epi = (int8_t)epi; s.n_out = (uint16_t)n_out; s.n_chunks = (uint16_t)chunks.size(); s.mask_slot = (int8_t)mask_slot;
   s.latent_slot = (int8_t)latent_slot; s.produce_a = (int8_t)produce_a; s.bias = bias; s.n2_out = 0;
   int i = 0;
   for (int c : chunks) s.a_chunk[i++] = (uint8_t)c;
@@ -918,7 +926,13 @@ static Step make_step(int epi, int n_out, int n_chunks, std::initializer_list<in
 static TcPlan build_plan(const snb_handle_s* h, bool split = false) {
   TcPlan pl;
   pl.split = split;
-  const int Bs = h->arch.shape_blocks, Bt = h->arch.texture_blocks, W = 256, dv = h->d_dir(), dx = h->d_xyz();
+  const int Bs = h->arch.shape_blocks, Bt = h->arch.texture_blocks, W = h->arch.W, dv = h->d_dir(), dx = h->d_xyz();
+  const int KC = W / 64;                           // K chunks of a hidden layer
+  std::vector<int> hid(KC);                        // ... held in A chunks 0 .. KC - 1
+  for (int c = 0; c < KC; ++c) hid[c] = c;
+  std::vector<int> ev_chunks = {4};                // encoding_viewdir: PE(viewdir) in the AUX chunk, then the hidden chunks
+  ev_chunks.insert(ev_chunks.end(), hid.begin(), hid.end());
+  const std::vector<int> r0_chunks(hid.begin(), hid.begin() + W / 128);   // backward through rgb.0: its W / 2 outputs
   const auto& ly = h->layers;
   const int slot_vv = Bs + 1, slot_r = Bs + Bt + 2;
   pl.r0_slot = slot_r;
@@ -926,59 +940,59 @@ static TcPlan build_plan(const snb_handle_s* h, bool split = false) {
   f.n_steps = 0; f.n_mask_slots = Bs + Bt + 3;
   auto push = [](Program& pr, const Step& s) { pr.s[pr.n_steps++] = s; };
   {  // ---------------- forward
-    Step s = make_step(EPI_RELU, 256, 1, {4}, 0, -1, 1, ly[h->iX].b);
-    add_chunks(pl, ly[h->iX].w, dx, false, 256, 256, dx, 1, &s.w_off);
+    Step s = make_step(EPI_RELU, W, {4}, 0, -1, 1, ly[h->iX].b);
+    add_chunks(pl, ly[h->iX].w, dx, false, W, W, dx, 1, &s.w_off);
     push(f, s);
     for (int j = 1; j <= Bs; ++j) {
-      s = make_step(EPI_RELU, 256, 4, {0, 1, 2, 3}, j, j - 1, 1, ly[h->iS(j)].b);   // effective bias slot j-1 = b + W zs_j
-      add_chunks(pl, ly[h->iS(j)].w, W, false, 256, 256, W, 4, &s.w_off);
+      s = make_step(EPI_RELU, W, hid, j, j - 1, 1, ly[h->iS(j)].b);   // effective bias slot j-1 = b + W zs_j
+      add_chunks(pl, ly[h->iS(j)].w, W, false, W, W, W, KC, &s.w_off);
       push(f, s);
     }
-    s = make_step(EPI_LINEAR_SIGMA, 256, 4, {0, 1, 2, 3}, -1, -1, 1, ly[h->iES].b);
-    add_chunks(pl, ly[h->iES].w, W, false, 256, 256, W, 4, &s.w_off);
+    s = make_step(EPI_LINEAR_SIGMA, W, hid, -1, -1, 1, ly[h->iES].b);
+    add_chunks(pl, ly[h->iES].w, W, false, W, W, W, KC, &s.w_off);
     push(f, s);
-    s = make_step(EPI_RELU, 256, 5, {4, 0, 1, 2, 3}, slot_vv, -1, 1, ly[h->iEV].b);
-    {  // chunk 0 = the PE(viewdir) columns [W, W+dv) of encoding_viewdir, chunks 1..4 = its first W columns
+    s = make_step(EPI_RELU, W, ev_chunks, slot_vv, -1, 1, ly[h->iEV].b);
+    {  // chunk 0 = the PE(viewdir) columns [W, W+dv) of encoding_viewdir, chunks 1..KC = its first W columns
       std::vector<ChunkSrc> chunks = {{ly[h->iEV].w + W, 0, dv}};
-      for (int c = 0; c < 4; ++c) chunks.push_back({ly[h->iEV].w, c * 64, W});
-      add_chunk_list(pl, chunks, W + dv, false, 256, 256, &s.w_off);
+      for (int c = 0; c < KC; ++c) chunks.push_back({ly[h->iEV].w, c * 64, W});
+      add_chunk_list(pl, chunks, W + dv, false, W, W, &s.w_off);
     }
     push(f, s);
     for (int j = 1; j <= Bt; ++j) {
-      s = make_step(EPI_RELU, 256, 4, {0, 1, 2, 3}, slot_vv + j, Bs + j - 1, 1, ly[h->iT(j)].b);
-      add_chunks(pl, ly[h->iT(j)].w, W, false, 256, 256, W, 4, &s.w_off);
+      s = make_step(EPI_RELU, W, hid, slot_vv + j, Bs + j - 1, 1, ly[h->iT(j)].b);
+      add_chunks(pl, ly[h->iT(j)].w, W, false, W, W, W, KC, &s.w_off);
       push(f, s);
     }
-    s = make_step(EPI_RGB_HEAD, 128, 4, {0, 1, 2, 3}, slot_r, -1, 0, ly[h->iR0].b);
-    add_chunks(pl, ly[h->iR0].w, W, false, 128, 128, W, 4, &s.w_off);
+    s = make_step(EPI_RGB_HEAD, W / 2, hid, slot_r, -1, 0, ly[h->iR0].b);
+    add_chunks(pl, ly[h->iR0].w, W, false, W / 2, W / 2, W, KC, &s.w_off);
     push(f, s);
   }
   {  // ---------------- backward (B operand = W^T: n = input unit, k = output unit)
     Program& b = pl.bwd_full;
     b.n_steps = 0; b.n_mask_slots = f.n_mask_slots;
-    Step s = make_step(EPI_B_MASK, 256, 2, {0, 1}, slot_vv + Bt, -1, 1, nullptr);          // through rgb.0 -> d T_Bt, mask of T_Bt
-    add_chunks(pl, ly[h->iR0].w, W, true, 256, 256, 128, 2, &s.w_off);
+    Step s = make_step(EPI_B_MASK, W, r0_chunks, slot_vv + Bt, -1, 1, nullptr);           // through rgb.0 -> d T_Bt, mask of T_Bt
+    add_chunks(pl, ly[h->iR0].w, W, true, W, W, W / 2, W / 128, &s.w_off);
     push(b, s);
     for (int j = Bt; j >= 1; --j) {                                                        // through texture_layer_j
-      s = make_step(EPI_B_MASK, 256, 4, {0, 1, 2, 3}, slot_vv + j - 1, Bs + j - 1, 1, nullptr);
-      add_chunks(pl, ly[h->iT(j)].w, W, true, 256, 256, W, 4, &s.w_off);
+      s = make_step(EPI_B_MASK, W, hid, slot_vv + j - 1, Bs + j - 1, 1, nullptr);
+      add_chunks(pl, ly[h->iT(j)].w, W, true, W, W, W, KC, &s.w_off);
       push(b, s);
     }
-    s = make_step(EPI_B_EV, 256, 4, {0, 1, 2, 3}, -1, -1, 1, nullptr);                     // through encoding_viewdir
-    add_chunks(pl, ly[h->iEV].w, W + dv, true, 256, 256, W, 4, &s.w_off);
-    add_chunks(pl, ly[h->iEV].w + W, W + dv, true, dv, 64, W, 4, &s.w2_off);
+    s = make_step(EPI_B_EV, W, hid, -1, -1, 1, nullptr);                                   // through encoding_viewdir
+    add_chunks(pl, ly[h->iEV].w, W + dv, true, W, W, W, KC, &s.w_off);
+    add_chunks(pl, ly[h->iEV].w + W, W + dv, true, dv, 64, W, KC, &s.w2_off);
     s.n2_out = 64;
     push(b, s);
-    s = make_step(EPI_B_MASK, 256, 4, {0, 1, 2, 3}, Bs, -1, 1, nullptr);                   // through encoding_shape, mask of H_Bs
-    add_chunks(pl, ly[h->iES].w, W, true, 256, 256, W, 4, &s.w_off);
+    s = make_step(EPI_B_MASK, W, hid, Bs, -1, 1, nullptr);                                 // through encoding_shape, mask of H_Bs
+    add_chunks(pl, ly[h->iES].w, W, true, W, W, W, KC, &s.w_off);
     push(b, s);
     for (int j = Bs; j >= 1; --j) {                                                        // through shape_layer_j
-      s = make_step(EPI_B_MASK, 256, 4, {0, 1, 2, 3}, j - 1, j - 1, 1, nullptr);
-      add_chunks(pl, ly[h->iS(j)].w, W, true, 256, 256, W, 4, &s.w_off);
+      s = make_step(EPI_B_MASK, W, hid, j - 1, j - 1, 1, nullptr);
+      add_chunks(pl, ly[h->iS(j)].w, W, true, W, W, W, KC, &s.w_off);
       push(b, s);
     }
-    s = make_step(EPI_B_XYZ, 64, 4, {0, 1, 2, 3}, -1, -1, 0, nullptr);                     // through encoding_xyz -> d PE(xyz)
-    add_chunks(pl, ly[h->iX].w, dx, true, dx, 64, W, 4, &s.w_off);
+    s = make_step(EPI_B_XYZ, 64, hid, -1, -1, 0, nullptr);                                 // through encoding_xyz -> d PE(xyz)
+    add_chunks(pl, ly[h->iX].w, dx, true, dx, 64, W, KC, &s.w_off);
     push(b, s);
     // variant without pose gradients: drop the last step and the d PE(viewdir) group; the new last step feeds nobody
     pl.bwd_noxyz = b;
@@ -1034,8 +1048,9 @@ int tc1_launch_fwd(const snb_handle_s* h, const void* packed, const float* xyz, 
   fill_common(p, h, packed, xyz, viewdir, M, B, ebias, masks, m_dev, tile_start);
   p.sigma = sigma; p.rgb = rgb; p.dbg = h->dbg_acts;
   p.prog = pl.fwd;
-  SNB_CHECK_CUDA(cudaFuncSetAttribute(tc_fwd_kernel<X>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Map<X>::SM_ALLOC));
-  tc_fwd_kernel<X><<<tc_grid(M), kThreads, Map<X>::SM_ALLOC, st>>>(p);
+  auto* kernel = h->arch.W == 128 ? tc_fwd_kernel<X, 128> : tc_fwd_kernel<X, 256>;   // tc1_supported: W is 128 or 256
+  SNB_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Map<X>::SM_ALLOC));
+  kernel<<<tc_grid(M), kThreads, Map<X>::SM_ALLOC, st>>>(p);
   return 0;
 }
 
@@ -1051,8 +1066,9 @@ int tc1_launch_bwd(const snb_handle_s* h, const void* packed, const float* xyz, 
   p.sigma_in = sigma; p.g_sigma = g_sigma; p.g_rgb = g_rgb; p.g_xyz = g_xyz; p.g_viewdir = g_viewdir; p.g_zlat = g_zlat;
   p.r0_mask_slot = pl.r0_slot;
   p.prog = g_xyz ? pl.bwd_full : pl.bwd_noxyz;
-  SNB_CHECK_CUDA(cudaFuncSetAttribute(tc_bwd_kernel<X>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Map<X>::SM_ALLOC));
-  tc_bwd_kernel<X><<<tc_grid(M), kThreads, Map<X>::SM_ALLOC, st>>>(p);
+  auto* kernel = h->arch.W == 128 ? tc_bwd_kernel<X, 128> : tc_bwd_kernel<X, 256>;
+  SNB_CHECK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Map<X>::SM_ALLOC));
+  kernel<<<tc_grid(M), kThreads, Map<X>::SM_ALLOC, st>>>(p);
   return 0;
 }
 

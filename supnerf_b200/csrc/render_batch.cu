@@ -877,7 +877,7 @@ int check_batch(snb_handle h, const snb_batch_desc* d, const char* who) {
               (int64_t)d->n_objs * d->rays_per_obj < ((int64_t)1 << 31), "%s: too many rays", who);
   Backend be;
   SNB_REQUIRE(select_backend(h, batch_precision(*d), &be) == nullptr, "%s: the batched render runs on the tcgen05 decoder kernels "
-              "(CodeNeRF family, W = 256, shape_blocks + texture_blocks <= 10); render the objects one by one for this architecture", who);
+              "(CodeNeRF family, W = 128 or 256, shape_blocks + texture_blocks <= 10); render the objects one by one for this architecture", who);
   if (d->flags & SNB_BATCH_FP32_TC)
     SNB_REQUIRE(!(d->flags & SNB_BATCH_FUSED_SAMPLER), "%s: SNB_BATCH_FP32_TC and SNB_BATCH_FUSED_SAMPLER exclude each other", who);
   if (d->flags & SNB_BATCH_FUSED_SAMPLER)

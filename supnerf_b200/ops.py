@@ -23,9 +23,9 @@ FP32_TC_MAX_WEIGHT = 255.0   # 256 * w must stay inside fp16's range (csrc/mlp_t
 
 
 def _fp32_tc(handle, prec, rows_per_obj=None, weights=None):
-    """fp32 mode with frozen weights -> the split-precision tensor-core kernels where they apply (CodeNeRF family, W = 256; dense row
-    counts a multiple of the 128-row tile; every |weight| < 255 -- checked once per weight version).  rows_per_obj None: the caller's
-    rows are compacted on the device (any count)."""
+    """fp32 mode with frozen weights -> the split-precision tensor-core kernels where they apply (CodeNeRF family, W = 128 or 256;
+    dense row counts a multiple of the 128-row tile; every |weight| < 255 -- checked once per weight version).  rows_per_obj None: the
+    caller's rows are compacted on the device (any count)."""
     if prec != PREC["fp32"] or not FP32_TENSOR_CORES or not handle.tc_ok:
         return prec
     if rows_per_obj is not None and (rows_per_obj <= 0 or rows_per_obj % 128 != 0):
@@ -695,7 +695,7 @@ def render_box_batch(handle, n_samples, white_bkgd, px, py, K, c2w, box, z_steps
     else:
         if fused_sampler or not handle.tc_ok or not handle.weights_in_fp16_range(weights):
             raise RuntimeError("render_box_batch(precision='fp32'): runs on the split-precision tensor-core decoder (CodeNeRF family, "
-                               "W = 256, |weights| < 255), without the fused sampler; render the objects one by one otherwise")
+                               "W = 128 or 256, |weights| < 255), without the fused sampler; render the objects one by one otherwise")
         flags |= BATCH_FP32_TC
         handle.use_frozen(weights, PREC_FP32_TC)
     return _RenderBoxBatch.apply(handle, n_samples, flags, px, py, K, c2w, box, z_steps, jitter, shape_latent, texture_latent)
