@@ -43,4 +43,14 @@ __device__ __forceinline__ float warp_sum(float v) {
 
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
+// gridDim.x of a grid-stride launch over n items, per_block items per block: ceil(n / per_block) blocks, at least one, at most
+// ceil(per_sm * SMs / n_objs) -- an equal share of per_sm blocks per SM for each of the n_objs objects a launch spreads over
+// gridDim.y.  <= 0 when there is no device.
+static inline int grid_1d(int64_t n, int64_t per_block, int per_sm, int n_objs = 1) {
+  const int sms = sm_count();
+  if (sms <= 0) return sms;
+  const int64_t blocks = ceil_div(n > 0 ? n : 1, per_block), cap = ceil_div((int64_t)per_sm * sms, n_objs);
+  return (int)(blocks < cap ? blocks : cap);
+}
+
 }  // namespace snb

@@ -10,72 +10,21 @@
 //   gather   dense xyz / viewdir (N,S,3) -> compact rows: hit rays S rows each, then one row per miss ray, then padding
 //   expand   compact sigma / rgb -> dense (N,S): miss rays replicated, so the unmodified compositing kernels run on them
 //   reduce   dense d sigma / d rgb -> compact: miss rays summed over their S samples (the decoder row is shared)
-//   scatter  compact d xyz / d viewdir -> dense: a miss ray's gradient goes to its last sample, zeros elsewhere -- the box sampler's
-//            backward only uses sum_k g_x_k (origin) and sum_k z_k g_x_k with z_k = -1 for every k (direction) on miss rays,
-//            both independent of which k holds it.
+// The box sampler's backward reads d xyz / d viewdir in compact row order (sampler.cu, sample_box_bwd_compact): a miss ray's row is
+// credited to its last sample -- the backward only uses sum_k g_x_k (origin) and sum_k z_k g_x_k with z_k = -1 for every k
+// (direction) on miss rays, both independent of which k holds it.
 // Exact: same per-row decoder arithmetic; gradients differ from the dense path only by fp32 summation order.
 #include "common.cuh"
 #include "compact.h"
 
 namespace snb {
 
+// one block: the rays ranked hit-first, then the row counts
 __global__ void __launch_bounds__(1024) compact_plan_kernel(const uint8_t* __restrict__ hit, int64_t n_rays, int S,
                                                            int32_t* __restrict__ order, int32_t* __restrict__ pos,
                                                            int64_t* __restrict__ counts) {
-  // One block.  Pre-pass: total number of hits (so the miss rays can be placed behind them).  Then super-chunks of 16 384 rays:
-  // warp w owns 512 consecutive rays as 16 coalesced 32-byte rows held in registers (16 independent loads = one memory
-  // latency), ballots give the in-row ranks, a 32-entry shared-memory scan the warp offsets, a running carry the rest.
-  __shared__ int warp_tot[32];
-  __shared__ int total_s;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const unsigned lt = (1u << lane) - 1u;
-  int local = 0;
-  for (int64_t i0 = 0; i0 < n_rays; i0 += 8 * 1024) {
-    int h[8];
-#pragma unroll
-    for (int k = 0; k < 8; ++k) { const int64_t i = i0 + (int64_t)k * 1024 + tid; h[k] = (i < n_rays && hit[i]) ? 1 : 0; }
-#pragma unroll
-    for (int k = 0; k < 8; ++k) local += h[k];
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) local += __shfl_xor_sync(0xffffffffu, local, o);
-  if (lane == 0) warp_tot[warp] = local;
-  __syncthreads();
-  if (tid == 0) { int t = 0; for (int w = 0; w < 32; ++w) t += warp_tot[w]; total_s = t; }
-  __syncthreads();
-  const int n_hit = total_s;
-  int carry = 0;   // hits in earlier super-chunks (identical in every thread)
-  for (int64_t sc = 0; sc < n_rays; sc += 16384) {
-    const int64_t wbase = sc + (int64_t)warp * 512;
-    unsigned m[16];
-    int wcnt = 0;
-#pragma unroll
-    for (int k = 0; k < 16; ++k) {
-      const int64_t i = wbase + k * 32 + lane;
-      m[k] = __ballot_sync(0xffffffffu, i < n_rays && hit[i]);
-    }
-#pragma unroll
-    for (int k = 0; k < 16; ++k) wcnt += __popc(m[k]);
-    __syncthreads();                       // warp_tot is free again
-    if (lane == 0) warp_tot[warp] = wcnt;
-    __syncthreads();
-    int before = carry, chunk_tot = 0;
-    for (int w = 0; w < 32; ++w) { const int t = warp_tot[w]; if (w < warp) before += t; chunk_tot += t; }
-#pragma unroll
-    for (int k = 0; k < 16; ++k) {
-      const int64_t i = wbase + k * 32 + lane;
-      const int h = (m[k] >> lane) & 1u;
-      const int hits_before = before + __popc(m[k] & lt);      // hit rays with a smaller index
-      if (i < n_rays) {
-        const int p = h ? hits_before : (int)(i - hits_before);   // rank inside its class
-        pos[i] = p;
-        order[h ? p : n_hit + p] = (int32_t)i;
-      }
-      before += __popc(m[k]);
-    }
-    carry += chunk_tot;
-  }
-  if (tid == 0) {
+  const int n_hit = rank_hits_first(hit, n_rays, order, pos);
+  if (threadIdx.x == 0) {
     const int64_t n_miss = n_rays - n_hit;
     const int64_t rows = (int64_t)n_hit * S + n_miss;
     counts[0] = n_hit; counts[1] = n_miss; counts[2] = rows; counts[3] = (rows + 127) / 128 * 128;
@@ -142,34 +91,6 @@ __global__ void __launch_bounds__(256) compact_reduce_kernel(const float* __rest
   }
 }
 
-__global__ void __launch_bounds__(256) compact_scatter_kernel(const float* __restrict__ g_xyz_c, const float* __restrict__ g_vrep_c,
-                                                             const uint8_t* __restrict__ hit, const int32_t* __restrict__ pos,
-                                                             const int64_t* __restrict__ counts, int64_t n_rays, int S,
-                                                             float* __restrict__ g_xyz, float* __restrict__ g_vrep) {
-  const int64_t n_hit = counts[0], total = n_rays * S;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
-    const int64_t ray = i / S;
-    const int k = (int)(i % S);
-    const bool h = hit[ray] != 0;
-    float x[3] = {0.f, 0.f, 0.f}, v[3] = {0.f, 0.f, 0.f};
-    if (h || k == S - 1) {
-      const int64_t r = compact_row(h, pos[ray], k, n_hit, S);
-#pragma unroll
-      for (int a = 0; a < 3; ++a) { x[a] = __ldg(g_xyz_c + 3 * r + a); v[a] = __ldg(g_vrep_c + 3 * r + a); }
-    }
-#pragma unroll
-    for (int a = 0; a < 3; ++a) { g_xyz[3 * i + a] = x[a]; g_vrep[3 * i + a] = v[a]; }
-  }
-}
-
-static int ew_grid(int64_t n) {
-  const int sms = sm_count();
-  if (sms <= 0) return -1;
-  const int64_t blocks = ceil_div(n > 0 ? n : 1, 256);
-  const int64_t cap = (int64_t)sms * 8;
-  return (int)(blocks < cap ? blocks : cap);
-}
-
 int compact_plan(const uint8_t* hit, int64_t n_rays, int S, int32_t* order, int32_t* pos, int64_t* counts, cudaStream_t st) {
   SNB_REQUIRE(n_rays < (int64_t)1 << 30, "compact_plan: too many rays");
   compact_plan_kernel<<<1, 1024, 0, st>>>(hit, n_rays, S, order, pos, counts);
@@ -178,7 +99,7 @@ int compact_plan(const uint8_t* hit, int64_t n_rays, int S, int32_t* order, int3
 }
 int compact_gather(const float* xyz, const float* vrep, const int32_t* order, const int64_t* counts, int64_t n_rays, int S,
                    float* xyz_c, float* vrep_c, cudaStream_t st) {
-  const int g = ew_grid(n_rays * S);
+  const int g = grid_1d(n_rays * S, 256, 8);
   SNB_REQUIRE(g > 0, "compact_gather: no CUDA device");
   compact_gather_kernel<<<g, 256, 0, st>>>(xyz, vrep, order, counts, S, xyz_c, vrep_c);
   SNB_LAUNCH_CHECK();
@@ -186,7 +107,7 @@ int compact_gather(const float* xyz, const float* vrep, const int32_t* order, co
 }
 int compact_expand(const float* sigma_c, const float* rgb_c, const uint8_t* hit, const int32_t* pos, const int64_t* counts,
                    int64_t n_rays, int S, float* sigma, float* rgb, cudaStream_t st) {
-  const int g = ew_grid(n_rays * S);
+  const int g = grid_1d(n_rays * S, 256, 8);
   SNB_REQUIRE(g > 0, "compact_expand: no CUDA device");
   compact_expand_kernel<<<g, 256, 0, st>>>(sigma_c, rgb_c, hit, pos, counts, n_rays, S, sigma, rgb);
   SNB_LAUNCH_CHECK();
@@ -194,19 +115,10 @@ int compact_expand(const float* sigma_c, const float* rgb_c, const uint8_t* hit,
 }
 int compact_reduce(const float* g_sigma, const float* g_rgb, const int32_t* order, const int64_t* counts, int64_t n_rays, int S,
                    float* g_sigma_c, float* g_rgb_c, cudaStream_t st) {
-  const int g = ew_grid(n_rays * S);
+  const int g = grid_1d(n_rays * S, 256, 8);
   SNB_REQUIRE(g > 0, "compact_reduce: no CUDA device");
   compact_reduce_kernel<<<g, 256, 0, st>>>(g_sigma, g_rgb, order, counts, S, g_sigma_c, g_rgb_c);
   SNB_LAUNCH_CHECK();
   return 0;
 }
-int compact_scatter(const float* g_xyz_c, const float* g_vrep_c, const uint8_t* hit, const int32_t* pos, const int64_t* counts,
-                    int64_t n_rays, int S, float* g_xyz, float* g_vrep, cudaStream_t st) {
-  const int g = ew_grid(n_rays * S);
-  SNB_REQUIRE(g > 0, "compact_scatter: no CUDA device");
-  compact_scatter_kernel<<<g, 256, 0, st>>>(g_xyz_c, g_vrep_c, hit, pos, counts, n_rays, S, g_xyz, g_vrep);
-  SNB_LAUNCH_CHECK();
-  return 0;
-}
-
 }  // namespace snb

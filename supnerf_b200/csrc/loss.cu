@@ -5,13 +5,14 @@
 //   loss_rgb = sum((rgb - tgt)^2 |occ|) / den            (the |occ| (N,1) broadcasts over the 3 channels)
 //   loss_occ = sum(exp(-occ (0.5 - acc)) |occ|) / den
 //   loss     = loss_rgb + coef * loss_occ
-// HBM-bound: reads 32 B/ray forward, reads 32 B + writes 16 B/ray backward.
+// HBM-bound: reads 32 B/ray forward, reads 32 B + writes 16 B/ray backward.  The per-object and the batched entry points (B objects
+// side by side, each over its own denominator) launch the same kernel pair, with gridDim.y = 1 and B.
 #include "common.cuh"
 #include "../../include/supnerf_b200.h"
 
 namespace snb {
 
-struct LossAcc {      // device scratch, 64 bytes
+struct LossAcc {      // device scratch, 40 bytes per object
   double num_rgb, num_occ, den;
   unsigned int ticket, pad;
   double den_final;   // den used by the forward (kept for the backward)
@@ -33,13 +34,18 @@ __device__ __forceinline__ double block_sum(double v, double* sh) {
   return t;   // valid in warp 0
 }
 
+// grid (chunks, objects): object b = blockIdx.y owns rays [b n, (b + 1) n), the record a[b] and out3[3 b .. 3 b + 2]
 __global__ void __launch_bounds__(256) refine_loss_fwd_kernel(const float* __restrict__ rgb, const float* __restrict__ acc,
                                                              const float* __restrict__ tgt, const float* __restrict__ occ,
                                                              int64_t n, float coef, const float* __restrict__ den_in,
-                                                             LossAcc* __restrict__ a, float* __restrict__ out3) {
+                                                             LossAcc* __restrict__ accs, float* __restrict__ out3) {
   __shared__ double sh[8];
+  const int b = blockIdx.y;
+  LossAcc* a = accs + b;
+  const int64_t base = (int64_t)b * n;
   double s_rgb = 0.0, s_occ = 0.0, s_den = 0.0;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+  for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t i = base + j;
     const float o = __ldg(occ + i), ao = fabsf(o);
     const float d0 = __ldg(rgb + 3 * i) - __ldg(tgt + 3 * i), d1 = __ldg(rgb + 3 * i + 1) - __ldg(tgt + 3 * i + 1),
                 d2 = __ldg(rgb + 3 * i + 2) - __ldg(tgt + 3 * i + 2);
@@ -56,28 +62,31 @@ __global__ void __launch_bounds__(256) refine_loss_fwd_kernel(const float* __res
     atomicAdd(&a->den, s_den);
     __threadfence();
     const unsigned int t = atomicAdd(&a->ticket, 1u);
-    if (t == gridDim.x - 1) {   // last block: every partial is visible
+    if (t == gridDim.x - 1) {   // the object's last block: every partial is visible
       __threadfence();
       const double nr = atomicAdd(&a->num_rgb, 0.0), no = atomicAdd(&a->num_occ, 0.0), dn = atomicAdd(&a->den, 0.0);
       // torch: den is an fp32 tensor (sum + 1e-9 in fp32); a caller-supplied den (ray-sharded mode) is used as is
-      const float den = den_in ? __ldg(den_in) : (float)dn + 1e-9f;
+      const float den = den_in ? __ldg(den_in + b) : (float)dn + 1e-9f;
       a->den_final = (double)den;
       const float lr = (float)(nr / (double)den), lo = (float)(no / (double)den);
-      out3[0] = lr + coef * lo;
-      out3[1] = lr;
-      out3[2] = lo;
+      out3[3 * b] = lr + coef * lo;
+      out3[3 * b + 1] = lr;
+      out3[3 * b + 2] = lo;
     }
   }
 }
 
 __global__ void __launch_bounds__(256) refine_loss_bwd_kernel(const float* __restrict__ rgb, const float* __restrict__ acc,
                                                              const float* __restrict__ tgt, const float* __restrict__ occ,
-                                                             int64_t n, float coef, const LossAcc* __restrict__ a,
+                                                             int64_t n, float coef, const LossAcc* __restrict__ accs,
                                                              const float* __restrict__ g_loss, float* __restrict__ g_rgb,
                                                              float* __restrict__ g_acc) {
-  const float g = g_loss ? __ldg(g_loss) : 1.f;
-  const float inv_den = (float)(1.0 / a->den_final);
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+  const int b = blockIdx.y;
+  const float g = g_loss ? __ldg(g_loss + b) : 1.f;
+  const float inv_den = (float)(1.0 / accs[b].den_final);
+  const int64_t base = (int64_t)b * n;
+  for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < n; j += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t i = base + j;
     const float o = __ldg(occ + i), ao = fabsf(o);
     const float s = 2.f * ao * inv_den * g;
     g_rgb[3 * i] = (__ldg(rgb + 3 * i) - __ldg(tgt + 3 * i)) * s;
@@ -85,6 +94,27 @@ __global__ void __launch_bounds__(256) refine_loss_bwd_kernel(const float* __res
     g_rgb[3 * i + 2] = (__ldg(rgb + 3 * i + 2) - __ldg(tgt + 3 * i + 2)) * s;
     g_acc[i] = g * coef * expf(-o * (0.5f - __ldg(acc + i))) * o * ao * inv_den;
   }
+}
+
+// one launch per direction for B objects of n rays each; the forward zeroes the B records first
+static int loss_fwd(const float* rgb, const float* acc, const float* tgt, const float* occ, int B, int64_t n, float coef, const float* den,
+                    float* out3, void* scratch, cudaStream_t st, const char* who) {
+  const int gx = grid_1d(n, 256, 2, B);
+  SNB_REQUIRE(gx > 0, "%s: no CUDA device (there is no CPU fallback)", who);
+  SNB_CHECK_CUDA(cudaMemsetAsync(scratch, 0, (size_t)B * sizeof(LossAcc), st));
+  refine_loss_fwd_kernel<<<dim3((unsigned)gx, (unsigned)B), 256, 0, st>>>(rgb, acc, tgt, occ, n, coef, den, (LossAcc*)scratch, out3);
+  SNB_LAUNCH_CHECK();
+  return 0;
+}
+
+static int loss_bwd(const float* rgb, const float* acc, const float* tgt, const float* occ, int B, int64_t n, float coef, const void* scratch,
+                    const float* g_loss, float* g_rgb, float* g_acc, cudaStream_t st, const char* who) {
+  const int gx = grid_1d(n, 256, 8, B);
+  SNB_REQUIRE(gx > 0, "%s: no CUDA device (there is no CPU fallback)", who);
+  refine_loss_bwd_kernel<<<dim3((unsigned)gx, (unsigned)B), 256, 0, st>>>(rgb, acc, tgt, occ, n, coef, (const LossAcc*)scratch, g_loss,
+                                                                         g_rgb, g_acc);
+  SNB_LAUNCH_CHECK();
+  return 0;
 }
 
 }  // namespace snb
@@ -97,15 +127,7 @@ extern "C" int snb_refine_loss_fwd(const float* rgb, const float* acc, const flo
                                    float occ_coef, const float* den, float* out3, void* scratch, void* stream) {
   SNB_REQUIRE(n_rays >= 0 && out3 && scratch, "refine_loss_fwd: bad arguments");
   SNB_REQUIRE(n_rays == 0 || (rgb && acc && tgt && occ), "refine_loss_fwd: null pointer");
-  const int sms = sm_count();
-  SNB_REQUIRE(sms > 0, "refine_loss_fwd: no CUDA device (there is no CPU fallback)");
-  cudaStream_t st = (cudaStream_t)stream;
-  SNB_CHECK_CUDA(cudaMemsetAsync(scratch, 0, sizeof(LossAcc), st));
-  int64_t blocks = ceil_div(n_rays > 0 ? n_rays : 1, 256);
-  const int grid = (int)(blocks < 2 * sms ? blocks : 2 * sms);
-  refine_loss_fwd_kernel<<<grid, 256, 0, st>>>(rgb, acc, tgt, occ, n_rays, occ_coef, den, (LossAcc*)scratch, out3);
-  SNB_LAUNCH_CHECK();
-  return 0;
+  return loss_fwd(rgb, acc, tgt, occ, 1, n_rays, occ_coef, den, out3, scratch, (cudaStream_t)stream, "refine_loss_fwd");
 }
 
 extern "C" int snb_refine_loss_bwd(const float* rgb, const float* acc, const float* tgt, const float* occ, int64_t n_rays,
@@ -114,12 +136,21 @@ extern "C" int snb_refine_loss_bwd(const float* rgb, const float* acc, const flo
   SNB_REQUIRE(n_rays >= 0 && scratch, "refine_loss_bwd: bad arguments");
   if (n_rays == 0) return 0;
   SNB_REQUIRE(rgb && acc && tgt && occ && g_rgb && g_acc, "refine_loss_bwd: null pointer");
-  const int sms = sm_count();
-  SNB_REQUIRE(sms > 0, "refine_loss_bwd: no CUDA device (there is no CPU fallback)");
-  int64_t blocks = ceil_div(n_rays, 256);
-  const int grid = (int)(blocks < 8 * sms ? blocks : 8 * sms);
-  refine_loss_bwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(rgb, acc, tgt, occ, n_rays, occ_coef, (const LossAcc*)scratch,
-                                                                g_loss, g_rgb, g_acc);
-  SNB_LAUNCH_CHECK();
-  return 0;
+  return loss_bwd(rgb, acc, tgt, occ, 1, n_rays, occ_coef, scratch, g_loss, g_rgb, g_acc, (cudaStream_t)stream, "refine_loss_bwd");
+}
+
+extern "C" size_t snb_refine_loss_batch_scratch_bytes(int32_t n_objs) { return n_objs > 0 ? (size_t)n_objs * sizeof(LossAcc) : 0; }
+
+extern "C" int snb_refine_loss_batch_fwd(const float* rgb, const float* acc, const float* tgt, const float* occ, int32_t n_objs,
+                                         int64_t rays_per_obj, float occ_coef, float* out3, void* scratch, void* stream) {
+  SNB_REQUIRE(n_objs >= 1 && rays_per_obj >= 1 && rgb && acc && tgt && occ && out3 && scratch, "refine_loss_batch_fwd: bad arguments");
+  return loss_fwd(rgb, acc, tgt, occ, n_objs, rays_per_obj, occ_coef, nullptr, out3, scratch, (cudaStream_t)stream, "refine_loss_batch_fwd");
+}
+
+extern "C" int snb_refine_loss_batch_bwd(const float* rgb, const float* acc, const float* tgt, const float* occ, int32_t n_objs,
+                                         int64_t rays_per_obj, float occ_coef, const void* scratch, const float* g_loss, float* g_rgb,
+                                         float* g_acc, void* stream) {
+  SNB_REQUIRE(n_objs >= 1 && rays_per_obj >= 1 && rgb && acc && tgt && occ && scratch && g_rgb && g_acc, "refine_loss_batch_bwd: bad arguments");
+  return loss_bwd(rgb, acc, tgt, occ, n_objs, rays_per_obj, occ_coef, scratch, g_loss, g_rgb, g_acc, (cudaStream_t)stream,
+                  "refine_loss_batch_bwd");
 }

@@ -16,8 +16,9 @@
 //             (per-ray fold of d xyz / d viewdir / d z through the sampler, the slab test and get_rays; per-object fp64 block sums
 //             -> d cam_pose (B,3,4))
 //
-// plus the batched refine losses (one launch per direction for all objects).  Frozen weights, bf16 decoder (two-tile kernels).
+// Frozen weights, bf16 decoder (two-tile kernels).
 #include "common.cuh"
+#include "compact.h"
 #include "decoder.h"
 #include "sampler.cuh"
 #include "composite.cuh"
@@ -37,24 +38,14 @@ __global__ void __launch_bounds__(256) rb_setup_kernel(const float* __restrict__
                                                       float* __restrict__ rays8, uint8_t* __restrict__ hit) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
     const int64_t b = i / N;
-    const float* Kb = K + 9 * b;
     const float* P = c2w + 12 * b;
     const float* bx = box + 4 * b;
-    const float cx = __ldg(Kb + 2), cy = __ldg(Kb + 5), fx = __ldg(Kb), fy = __ldg(Kb + 4);
-    // utils.get_rays: dirs = ((i - cx) / fx, (j - cy) / fy, 1); rays_d = sum(dirs * R, -1); viewdir = rays_d / |rays_d|
-    const float p0 = __fdiv_rn(__fsub_rn(__ldg(px + i), cx), fx), p1 = __fdiv_rn(__fsub_rn(__ldg(py + i), cy), fy), p2 = 1.f;
-    float r[3], o[3], d[3];
-#pragma unroll
-    for (int a = 0; a < 3; ++a)
-      r[a] = __fadd_rn(__fadd_rn(__fmul_rn(p0, __ldg(P + 4 * a)), __fmul_rn(p1, __ldg(P + 4 * a + 1))), __fmul_rn(p2, __ldg(P + 4 * a + 2)));
-    const float nrm = sqrtf(__fadd_rn(__fadd_rn(__fmul_rn(r[0], r[0]), __fmul_rn(r[1], r[1])), __fmul_rn(r[2], r[2])));
+    float o[3], d[3];
+    pixel_dir(K + 9 * b, P, __ldg(px + i), __ldg(py + i), d);
     const float half_diag = __ldg(bx);
     const float half[3] = {__ldg(bx + 1), __ldg(bx + 2), __ldg(bx + 3)};
 #pragma unroll
-    for (int a = 0; a < 3; ++a) {
-      d[a] = __fdiv_rn(r[a], nrm);
-      o[a] = __fdiv_rn(__ldg(P + 4 * a + 3), half_diag);   // rays_o / (obj_diag / 2), renderer.py:102
-    }
+    for (int a = 0; a < 3; ++a) o[a] = __fdiv_rn(__ldg(P + 4 * a + 3), half_diag);   // rays_o / (obj_diag / 2), renderer.py:102
     const Slab sl = slab_test(o, d, half);
     float4* dst = reinterpret_cast<float4*>(rays8 + 8 * i);
     dst[0] = make_float4(o[0], o[1], o[2], d[0]);
@@ -64,67 +55,17 @@ __global__ void __launch_bounds__(256) rb_setup_kernel(const float* __restrict__
 }
 
 // --------------------------------------------------------------------------------------------------------------- plan
-// block b: object b's rays ranked hit-first (the body of compact.cu's compact_plan_kernel); the last block to finish makes the
-// row offsets: object b owns rows [row_start, row_start + rows) of the decoder's input, padded to 256 (one cta_group::2 super tile)
+// block b: object b's rays ranked hit-first (compact.h); the last block to finish makes the row offsets: object b owns rows
+// [row_start, row_start + rows) of the decoder's input, padded to 256 (one cta_group::2 super tile)
 __global__ void __launch_bounds__(1024) rb_plan_kernel(const uint8_t* __restrict__ hit_all, int64_t N, int S, int B,
                                                       int32_t* __restrict__ order_all, int32_t* __restrict__ pos_all,
                                                       ObjCounts* __restrict__ counts, int32_t* __restrict__ tile_start,
                                                       Meta* __restrict__ meta) {
-  __shared__ int warp_tot[32];
-  __shared__ int total_s;
   const int b = blockIdx.x;
-  const uint8_t* hit = hit_all + (int64_t)b * N;
-  int32_t* order = order_all + (int64_t)b * N;
-  int32_t* pos = pos_all + (int64_t)b * N;
-  const int64_t n_rays = N;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const unsigned lt = (1u << lane) - 1u;
-  int local = 0;
-  for (int64_t i0 = 0; i0 < n_rays; i0 += 8 * 1024) {
-#pragma unroll
-    for (int k = 0; k < 8; ++k) { const int64_t i = i0 + (int64_t)k * 1024 + tid; local += (i < n_rays && hit[i]) ? 1 : 0; }
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) local += __shfl_xor_sync(0xffffffffu, local, o);
-  if (lane == 0) warp_tot[warp] = local;
+  const int n_hit = rank_hits_first(hit_all + (int64_t)b * N, N, order_all + (int64_t)b * N, pos_all + (int64_t)b * N);
   __syncthreads();
-  if (tid == 0) { int t = 0; for (int w = 0; w < 32; ++w) t += warp_tot[w]; total_s = t; }
-  __syncthreads();
-  const int n_hit = total_s;
-  int carry = 0;
-  for (int64_t sc = 0; sc < n_rays; sc += 16384) {
-    const int64_t wbase = sc + (int64_t)warp * 512;
-    unsigned m[16];
-    int wcnt = 0;
-#pragma unroll
-    for (int k = 0; k < 16; ++k) {
-      const int64_t i = wbase + k * 32 + lane;
-      m[k] = __ballot_sync(0xffffffffu, i < n_rays && hit[i]);
-    }
-#pragma unroll
-    for (int k = 0; k < 16; ++k) wcnt += __popc(m[k]);
-    __syncthreads();
-    if (lane == 0) warp_tot[warp] = wcnt;
-    __syncthreads();
-    int before = carry, chunk_tot = 0;
-    for (int w = 0; w < 32; ++w) { const int t = warp_tot[w]; if (w < warp) before += t; chunk_tot += t; }
-#pragma unroll
-    for (int k = 0; k < 16; ++k) {
-      const int64_t i = wbase + k * 32 + lane;
-      const int h = (m[k] >> lane) & 1u;
-      const int hits_before = before + __popc(m[k] & lt);
-      if (i < n_rays) {
-        const int p = h ? hits_before : (int)(i - hits_before);
-        pos[i] = p;
-        order[h ? p : n_hit + p] = (int32_t)i;
-      }
-      before += __popc(m[k]);
-    }
-    carry += chunk_tot;
-  }
-  __syncthreads();
-  if (tid == 0) {
-    const int64_t n_miss = n_rays - n_hit;
+  if (threadIdx.x == 0) {
+    const int64_t n_miss = N - n_hit;
     counts[b].n_hit = n_hit; counts[b].n_miss = n_miss; counts[b].rows = (int64_t)n_hit * S + n_miss;
     __threadfence();
     const unsigned t = atomicAdd(&meta->done, 1u);
@@ -424,6 +365,36 @@ __global__ void __launch_bounds__(256) rb_composite_bwd_kernel(const float* __re
 }
 
 // --------------------------------------------------------------------------------------------------------------- rays backward
+// Object b's pose gradient from the per-thread fp64 sums acc (c2w layout) of a 256-thread block: one block reduction and one atomic
+// per entry into acc64[12 b ..]; the object's last block (tickets[b]) writes the totals to g_c2w[12 b ..].
+__device__ __forceinline__ void flush_pose_grad(const double acc[12], int b, double* __restrict__ acc64, unsigned int* __restrict__ tickets,
+                                                float* __restrict__ g_c2w) {
+  __shared__ double red[8][12];
+  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+#pragma unroll
+  for (int i = 0; i < 12; ++i) {
+    double v = acc[i];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    if (lane == 0) red[wib][i] = v;
+  }
+  __syncthreads();
+  if (threadIdx.x < 12) {
+    double v = 0.0;
+    for (int k = 0; k < (int)(blockDim.x >> 5); ++k) v += red[k][threadIdx.x];
+    atomicAdd(acc64 + 12 * b + threadIdx.x, v);
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    __threadfence();
+    const unsigned t = atomicAdd(tickets + b, 1u);
+    if (t == gridDim.x - 1) {     // the object's last block: every partial is visible
+      __threadfence();
+      for (int i = 0; i < 12; ++i) g_c2w[12 * b + i] = (float)atomicAdd(acc64 + 12 * b + i, 0.0);
+    }
+  }
+}
+
 // d xyz / d viewdir / d z_vals of a ray's compact rows -> d (o, d, near, far) -> through the slab test -> d (rays_o, viewdir) ->
 // through get_rays -> this object's d cam_pose (12 fp64 sums per thread, one block reduction + one atomic each per block).
 // Two phases per group of 32 rays of a warp: (1) the warp walks its 32 rays one after the other, lanes over the ray's samples, and
@@ -442,11 +413,8 @@ __global__ void __launch_bounds__(256) rb_rays_bwd_kernel(const float* __restric
                                                          float* __restrict__ g_c2w) {
   const int b = blockIdx.y;
   const ObjCounts c = counts[b];
-  const float* Kb = K + 9 * b;
-  const float* P = c2w + 12 * b;
   const float half_diag = __ldg(box + 4 * b);
   const float half[3] = {__ldg(box + 4 * b + 1), __ldg(box + 4 * b + 2), __ldg(box + 4 * b + 3)};
-  const float cx = __ldg(Kb + 2), cy = __ldg(Kb + 5), fx = __ldg(Kb), fy = __ldg(Kb + 4);
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
   const float fstep = (float)(1.0 / (double)S);
   double acc[12];
@@ -472,48 +440,19 @@ __global__ void __launch_bounds__(256) rb_rays_bwd_kernel(const float* __restric
         const float dn = sqrtf(d[0] * d[0] + d[1] * d[1] + d[2] * d[2]);
         if (h) {
           for (int k = l8; k < S; k += 8) {
-            const float zs = __fadd_rn(__ldg(z_steps + k), __fmul_rn(__ldg(jitter + gi * S + k), fstep));
-            const float zc = __fadd_rn(__fmul_rn(near, __fsub_rn(1.f, zs)), __fmul_rn(far, zs));
             const int64_t gidx = c.row_start + (int64_t)p * S + k;
             // a row of a super tile the decoder skipped has d xyz = d viewdir = 0 (its scratch rows hold an older call's values);
             // d z comes from the compositing backward and is always read.  Per row: a ray can span two super tiles.
             const bool lv = __ldg(live + (gidx >> 8)) != 0;
-            const float gx[3] = {lv ? __ldg(g_xyz_c + 3 * gidx) : 0.f, lv ? __ldg(g_xyz_c + 3 * gidx + 1) : 0.f,
-                                 lv ? __ldg(g_xyz_c + 3 * gidx + 2) : 0.f};
-            float gz = gx[0] * d[0] + gx[1] * d[1] + gx[2] * d[2];
-#pragma unroll
-            for (int a = 0; a < 3; ++a) { v[a] += gx[a]; v[3 + a] += zc * gx[a]; }
-            if (lv) { v[3] += __ldg(g_vrep_c + 3 * gidx); v[4] += __ldg(g_vrep_c + 3 * gidx + 1); v[5] += __ldg(g_vrep_c + 3 * gidx + 2); }
-            if (g_z_c != nullptr) {
-              const float gv = __ldg(g_z_c + gidx);
-              const float sgn = (zc > 0.f) ? 1.f : ((zc < 0.f) ? -1.f : 0.f);
-              gz += gv * sgn * dn * half_diag;
-              v[6] += gv * fabsf(zc);
-            }
-            v[7] += gz * (1.f - zs);
-            v[8] += gz * zs;
+            fold_sample_grad(lv ? g_xyz_c + 3 * gidx : nullptr, lv ? g_vrep_c + 3 * gidx : nullptr, g_z_c ? g_z_c + gidx : nullptr,
+                             __ldg(z_steps + k), __ldg(jitter + gi * S + k), fstep, near, far, d, dn, half_diag, v);
           }
         } else if (l8 == 0) {
           // a miss ray's single row stands for all its samples and is credited to the last one (k = S - 1)
-          const int k = S - 1;
-          const float zs = __fadd_rn(__ldg(z_steps + k), __fmul_rn(__ldg(jitter + gi * S + k), fstep));
-          const float zc = __fadd_rn(__fmul_rn(near, __fsub_rn(1.f, zs)), __fmul_rn(far, zs));
           const int64_t gidx = c.row_start + c.n_hit * S + p;
           const bool lv = __ldg(live + (gidx >> 8)) != 0;
-          const float gx[3] = {lv ? __ldg(g_xyz_c + 3 * gidx) : 0.f, lv ? __ldg(g_xyz_c + 3 * gidx + 1) : 0.f,
-                               lv ? __ldg(g_xyz_c + 3 * gidx + 2) : 0.f};
-          float gz = gx[0] * d[0] + gx[1] * d[1] + gx[2] * d[2];
-#pragma unroll
-          for (int a = 0; a < 3; ++a) { v[a] = gx[a]; v[3 + a] = zc * gx[a]; }
-          if (lv) { v[3] += __ldg(g_vrep_c + 3 * gidx); v[4] += __ldg(g_vrep_c + 3 * gidx + 1); v[5] += __ldg(g_vrep_c + 3 * gidx + 2); }
-          if (g_z_c != nullptr) {
-            const float gv = __ldg(g_z_c + gidx);
-            const float sgn = (zc > 0.f) ? 1.f : ((zc < 0.f) ? -1.f : 0.f);
-            gz += gv * sgn * dn * half_diag;
-            v[6] = gv * fabsf(zc);
-          }
-          v[7] = gz * (1.f - zs);
-          v[8] = gz * zs;
+          fold_sample_grad(lv ? g_xyz_c + 3 * gidx : nullptr, lv ? g_vrep_c + 3 * gidx : nullptr, g_z_c ? g_z_c + gidx : nullptr,
+                           __ldg(z_steps + S - 1), __ldg(jitter + gi * S + S - 1), fstep, near, far, d, dn, half_diag, v);
         }
       }
       const int src = ((lane - jj) & 3) * 8;            // lanes jj .. jj+3 take their ray's sums from the group that walked it
@@ -550,49 +489,18 @@ __global__ void __launch_bounds__(256) rb_rays_bwd_kernel(const float* __restric
 #pragma unroll
         for (int a = 0; a < 3; ++a) { gon[a] += go2[a]; gd[a] += gd2[a]; }
       }
-      // through get_rays (sampler.cu: get_rays_bwd_kernel): g_r = (g_d - d (g_d . d)) / |r|
-      const float pp[3] = {(__ldg(px + gi) - cx) / fx, (__ldg(py + gi) - cy) / fy, 1.f};
-      float r[3];
-#pragma unroll
-      for (int a = 0; a < 3; ++a) r[a] = pp[0] * __ldg(P + 4 * a) + pp[1] * __ldg(P + 4 * a + 1) + pp[2] * __ldg(P + 4 * a + 2);
-      const float inv = 1.f / sqrtf(r[0] * r[0] + r[1] * r[1] + r[2] * r[2]);
-      float dd[3];
-#pragma unroll
-      for (int a = 0; a < 3; ++a) dd[a] = r[a] * inv;
-      const float dot = gd[0] * dd[0] + gd[1] * dd[1] + gd[2] * dd[2];
+      float pp[3], gr[3];
+      dir_grad_to_pose(K + 9 * b, c2w + 12 * b, __ldg(px + gi), __ldg(py + gi), gd, pp, gr);
 #pragma unroll
       for (int a = 0; a < 3; ++a) {
-        const float gr = (gd[a] - dd[a] * dot) * inv;
-        acc[4 * a + 0] += (double)(gr * pp[0]);
-        acc[4 * a + 1] += (double)(gr * pp[1]);
-        acc[4 * a + 2] += (double)(gr * pp[2]);
+        acc[4 * a + 0] += (double)(gr[a] * pp[0]);
+        acc[4 * a + 1] += (double)(gr[a] * pp[1]);
+        acc[4 * a + 2] += (double)(gr[a] * pp[2]);
         acc[4 * a + 3] += (double)(gon[a] / half_diag);
       }
     }
   }
-  __shared__ double red[8][12];
-#pragma unroll
-  for (int i = 0; i < 12; ++i) {
-    double v = acc[i];
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    if (lane == 0) red[wib][i] = v;
-  }
-  __syncthreads();
-  if (threadIdx.x < 12) {
-    double v = 0.0;
-    for (int k = 0; k < (int)(blockDim.x >> 5); ++k) v += red[k][threadIdx.x];
-    atomicAdd(acc64 + 12 * b + threadIdx.x, v);
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    __threadfence();
-    const unsigned t = atomicAdd(tickets + b, 1u);
-    if (t == gridDim.x - 1) {     // the object's last block: every partial is visible
-      __threadfence();
-      for (int i = 0; i < 12; ++i) g_c2w[12 * b + i] = (float)atomicAdd(acc64 + 12 * b + i, 0.0);
-    }
-  }
+  flush_pose_grad(acc, b, acc64, tickets, g_c2w);
 }
 
 // --------------------------------------------------------------------------------------------------------------- dataset-side ray prep
@@ -611,17 +519,11 @@ __global__ void __launch_bounds__(256) rb_shell_prep_kernel(const float* __restr
   const int64_t nwarps = (int64_t)gridDim.x * (blockDim.x >> 5);
   for (int64_t i = warp; i < total; i += nwarps) {
     const int64_t b = i / n;
-    const float* Kb = K + 9 * b;
     const float* P = c2w + 12 * b;
-    const float cx = __ldg(Kb + 2), cy = __ldg(Kb + 5), fx = __ldg(Kb), fy = __ldg(Kb + 4);
-    const float p0 = __fdiv_rn(__fsub_rn(__ldg(px + i), cx), fx), p1 = __fdiv_rn(__fsub_rn(__ldg(py + i), cy), fy), p2 = 1.f;
-    float r[3], o[3], d[3];
+    float o[3], d[3];
+    pixel_dir(K + 9 * b, P, __ldg(px + i), __ldg(py + i), d);
 #pragma unroll
-    for (int a = 0; a < 3; ++a)
-      r[a] = __fadd_rn(__fadd_rn(__fmul_rn(p0, __ldg(P + 4 * a)), __fmul_rn(p1, __ldg(P + 4 * a + 1))), __fmul_rn(p2, __ldg(P + 4 * a + 2)));
-    const float nrm = sqrtf(__fadd_rn(__fadd_rn(__fmul_rn(r[0], r[0]), __fmul_rn(r[1], r[1])), __fmul_rn(r[2], r[2])));
-#pragma unroll
-    for (int a = 0; a < 3; ++a) { d[a] = __fdiv_rn(r[a], nrm); o[a] = __ldg(P + 4 * a + 3); }
+    for (int a = 0; a < 3; ++a) o[a] = __ldg(P + 4 * a + 3);
     const float diag = __ldg(obj_diag + b);
     const float sy = (flip != nullptr && flip[b]) ? -1.f : 1.f;       // sym_aug: xyz[:, :, 1] *= -1, viewdir[:, :, 1] *= -1 (utils.py:474-477)
     const float* zb = z + b * S;
@@ -653,9 +555,6 @@ __global__ void __launch_bounds__(256) rb_shell_rays_bwd_kernel(const float* __r
                                                                const float* __restrict__ g_vrep, double* __restrict__ acc64,
                                                                unsigned int* __restrict__ tickets, float* __restrict__ g_c2w) {
   const int b = blockIdx.y;
-  const float* Kb = K + 9 * b;
-  const float* P = c2w + 12 * b;
-  const float cx = __ldg(Kb + 2), cy = __ldg(Kb + 5), fx = __ldg(Kb), fy = __ldg(Kb + 4);
   const float diag = __ldg(obj_diag + b);
   const float* zb = z + (int64_t)b * S;
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
@@ -682,123 +581,19 @@ __global__ void __launch_bounds__(256) rb_shell_rays_bwd_kernel(const float* __r
     }
 #pragma unroll
     for (int a = 0; a < 3; ++a) { go[a] = warp_sum(go[a]); gd[a] = warp_sum(gd[a]); }
-    if (lane == 0) {
-      const float pp[3] = {(__ldg(px + gi) - cx) / fx, (__ldg(py + gi) - cy) / fy, 1.f};
-      float r[3], dd[3];
-#pragma unroll
-      for (int a = 0; a < 3; ++a) r[a] = pp[0] * __ldg(P + 4 * a) + pp[1] * __ldg(P + 4 * a + 1) + pp[2] * __ldg(P + 4 * a + 2);
-      const float inv = 1.f / sqrtf(r[0] * r[0] + r[1] * r[1] + r[2] * r[2]);
-#pragma unroll
-      for (int a = 0; a < 3; ++a) dd[a] = r[a] * inv;
-      const float dot = gd[0] * dd[0] + gd[1] * dd[1] + gd[2] * dd[2];
+    if (lane == 0) {   // the other lanes' sums stay 0
+      float pp[3], gr[3];
+      dir_grad_to_pose(K + 9 * b, c2w + 12 * b, __ldg(px + gi), __ldg(py + gi), gd, pp, gr);
 #pragma unroll
       for (int a = 0; a < 3; ++a) {
-        const float gr = (gd[a] - dd[a] * dot) * inv;
-        acc[4 * a + 0] += (double)(gr * pp[0]);
-        acc[4 * a + 1] += (double)(gr * pp[1]);
-        acc[4 * a + 2] += (double)(gr * pp[2]);
+        acc[4 * a + 0] += (double)(gr[a] * pp[0]);
+        acc[4 * a + 1] += (double)(gr[a] * pp[1]);
+        acc[4 * a + 2] += (double)(gr[a] * pp[2]);
         acc[4 * a + 3] += (double)go[a];
       }
     }
   }
-  __shared__ double red[8][12];
-  if (lane == 0) {
-#pragma unroll
-    for (int i = 0; i < 12; ++i) red[wib][i] = acc[i];
-  }
-  __syncthreads();
-  if (threadIdx.x < 12) {
-    double v = 0.0;
-    for (int k = 0; k < 8; ++k) v += red[k][threadIdx.x];
-    atomicAdd(acc64 + 12 * b + threadIdx.x, v);
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    __threadfence();
-    const unsigned t = atomicAdd(tickets + b, 1u);
-    if (t == gridDim.x - 1) {
-      __threadfence();
-      for (int i = 0; i < 12; ++i) g_c2w[12 * b + i] = (float)atomicAdd(acc64 + 12 * b + i, 0.0);
-    }
-  }
-}
-
-// --------------------------------------------------------------------------------------------------------------- batched losses
-// optimizer_nuscenes.py:729-736 per object (see loss.cu): grid (chunks, B)
-struct LossAccB { double num_rgb, num_occ, den; unsigned int ticket, pad; double den_final; };
-
-__device__ __forceinline__ double block_sum_d(double v, double* sh) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  __syncthreads();
-  if (lane == 0) sh[warp] = v;
-  __syncthreads();
-  double t = 0.0;
-  if (warp == 0) {
-    t = lane < (int)(blockDim.x >> 5) ? sh[lane] : 0.0;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
-  }
-  return t;
-}
-
-__global__ void __launch_bounds__(256) rb_loss_fwd_kernel(const float* __restrict__ rgb, const float* __restrict__ acc,
-                                                         const float* __restrict__ tgt, const float* __restrict__ occ, int64_t N,
-                                                         float coef, LossAccB* __restrict__ accs, float* __restrict__ out3) {
-  __shared__ double sh[8];
-  const int b = blockIdx.y;
-  LossAccB* a = accs + b;
-  const int64_t base = (int64_t)b * N;
-  double s_rgb = 0.0, s_occ = 0.0, s_den = 0.0;
-  for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < N; j += (int64_t)gridDim.x * blockDim.x) {
-    const int64_t i = base + j;
-    const float o = __ldg(occ + i), ao = fabsf(o);
-    const float d0 = __ldg(rgb + 3 * i) - __ldg(tgt + 3 * i), d1 = __ldg(rgb + 3 * i + 1) - __ldg(tgt + 3 * i + 1),
-                d2 = __ldg(rgb + 3 * i + 2) - __ldg(tgt + 3 * i + 2);
-    s_rgb += (double)((d0 * d0) * ao) + (double)((d1 * d1) * ao) + (double)((d2 * d2) * ao);
-    s_occ += (double)(expf(-o * (0.5f - __ldg(acc + i))) * ao);
-    s_den += (double)ao;
-  }
-  s_rgb = block_sum_d(s_rgb, sh);
-  s_occ = block_sum_d(s_occ, sh);
-  s_den = block_sum_d(s_den, sh);
-  if (threadIdx.x == 0) {
-    atomicAdd(&a->num_rgb, s_rgb);
-    atomicAdd(&a->num_occ, s_occ);
-    atomicAdd(&a->den, s_den);
-    __threadfence();
-    const unsigned int t = atomicAdd(&a->ticket, 1u);
-    if (t == gridDim.x - 1) {
-      __threadfence();
-      const double nr = atomicAdd(&a->num_rgb, 0.0), no = atomicAdd(&a->num_occ, 0.0), dn = atomicAdd(&a->den, 0.0);
-      const float den = (float)dn + 1e-9f;
-      a->den_final = (double)den;
-      const float lr = (float)(nr / (double)den), lo = (float)(no / (double)den);
-      out3[3 * b] = lr + coef * lo;
-      out3[3 * b + 1] = lr;
-      out3[3 * b + 2] = lo;
-    }
-  }
-}
-
-__global__ void __launch_bounds__(256) rb_loss_bwd_kernel(const float* __restrict__ rgb, const float* __restrict__ acc,
-                                                         const float* __restrict__ tgt, const float* __restrict__ occ, int64_t N,
-                                                         float coef, const LossAccB* __restrict__ accs, const float* __restrict__ g_loss,
-                                                         float* __restrict__ g_rgb, float* __restrict__ g_acc) {
-  const int b = blockIdx.y;
-  const float g = g_loss ? __ldg(g_loss + b) : 1.f;
-  const float inv_den = (float)(1.0 / accs[b].den_final);
-  const int64_t base = (int64_t)b * N;
-  for (int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < N; j += (int64_t)gridDim.x * blockDim.x) {
-    const int64_t i = base + j;
-    const float o = __ldg(occ + i), ao = fabsf(o);
-    const float s = 2.f * ao * inv_den * g;
-    g_rgb[3 * i] = (__ldg(rgb + 3 * i) - __ldg(tgt + 3 * i)) * s;
-    g_rgb[3 * i + 1] = (__ldg(rgb + 3 * i + 1) - __ldg(tgt + 3 * i + 1)) * s;
-    g_rgb[3 * i + 2] = (__ldg(rgb + 3 * i + 2) - __ldg(tgt + 3 * i + 2)) * s;
-    g_acc[i] = g * coef * expf(-o * (0.5f - __ldg(acc + i))) * o * ao * inv_den;
-  }
+  flush_pose_grad(acc, b, acc64, tickets, g_c2w);
 }
 
 }  // namespace rb
@@ -888,13 +683,13 @@ int check_batch(snb_handle h, const snb_batch_desc* d, const char* who) {
 template <typename T> inline T* at(void* base, size_t off) { return reinterpret_cast<T*>(static_cast<uint8_t*>(base) + off); }
 template <typename T> inline const T* at(const void* base, size_t off) { return reinterpret_cast<const T*>(static_cast<const uint8_t*>(base) + off); }
 
-inline int ew_grid(int64_t n, int per_sm) {
-  const int sms = sm_count();
-  if (sms <= 0) return -1;
-  const int64_t blocks = ceil_div(n > 0 ? n : 1, 256);
-  const int64_t cap = (int64_t)sms * per_sm;
-  return (int)(blocks < cap ? blocks : cap);
-}
+// the compositing launches: LPR lanes per hit ray (4 samples each), 32 / LPR rays per warp, 8 warps per block; grid (x, objects)
+struct CompositeGrid {
+  int lpr;
+  dim3 grid;
+  CompositeGrid(int64_t N, int S, int B)
+      : lpr(S <= 32 ? 8 : (S <= 64 ? 16 : 32)), grid((unsigned)grid_1d(N, 8 * (32 / lpr), 8, B), (unsigned)B) {}
+};
 
 }  // namespace
 }  // namespace snb
@@ -925,10 +720,9 @@ extern "C" int snb_render_batch_fwd(snb_handle h, const snb_batch_desc* d, const
   void* ws = workspace;
   const int B = d->n_objs, S = d->n_samples;
   const int64_t N = d->rays_per_obj, BN = (int64_t)B * N;
-  const int sms = sm_count();
-  SNB_REQUIRE(sms > 0, "render_batch_fwd: no CUDA device (there is no CPU fallback)");
+  SNB_REQUIRE(sm_count() > 0, "render_batch_fwd: no CUDA device (there is no CPU fallback)");
   SNB_CHECK_CUDA(cudaMemsetAsync(at<uint8_t>(ws, L.meta), 0, sizeof(rb::Meta), st));
-  rb::rb_setup_kernel<<<ew_grid(BN, 8), 256, 0, st>>>(px, py, K, c2w, box, N, BN, at<float>(ws, L.rays8), at<uint8_t>(ws, L.hit));
+  rb::rb_setup_kernel<<<grid_1d(BN, 256, 8), 256, 0, st>>>(px, py, K, c2w, box, N, BN, at<float>(ws, L.rays8), at<uint8_t>(ws, L.hit));
   SNB_LAUNCH_CHECK();
   rb::rb_plan_kernel<<<B, 1024, 0, st>>>(at<uint8_t>(ws, L.hit), N, S, B, at<int32_t>(ws, L.order), at<int32_t>(ws, L.pos),
                                         at<rb::ObjCounts>(ws, L.counts), at<int32_t>(ws, L.tile_start), at<rb::Meta>(ws, L.meta));
@@ -949,7 +743,7 @@ extern "C" int snb_render_batch_fwd(snb_handle h, const snb_batch_desc* d, const
   } else {
     // default: the stratified samples of the EXECUTED rows are written once (28 B per row) and read back by the decoder -- measured
     // faster than the fused sampler: the extra ~150 instructions per row sit on the decoder's critical tile-boundary chain
-    rb::rb_gather_kernel<<<ew_grid(L.Mmax, 8), 256, 0, st>>>(at<float>(ws, L.rays8), box, z_steps, jitter, at<int32_t>(ws, L.order),
+    rb::rb_gather_kernel<<<grid_1d(L.Mmax, 256, 8), 256, 0, st>>>(at<float>(ws, L.rays8), box, z_steps, jitter, at<int32_t>(ws, L.order),
                                                             at<rb::ObjCounts>(ws, L.counts), at<rb::Meta>(ws, L.meta), B, N, S,
                                                             at<float>(ws, L.xyz_c), at<float>(ws, L.vrep_c), at<float>(ws, L.z_c));
     SNB_LAUNCH_CHECK();
@@ -959,15 +753,10 @@ extern "C" int snb_render_batch_fwd(snb_handle h, const snb_batch_desc* d, const
       return 1;
     zsrc.z_c = at<float>(ws, L.z_c);
   }
-  const int lpr = S <= 32 ? 8 : (S <= 64 ? 16 : 32);
-  int gx = (int)ceil_div(ceil_div(N, 32 / lpr), 8);
-  const int cap = (sms * 8 + B - 1) / B;
-  if (gx > cap) gx = cap;
-  if (gx < 1) gx = 1;
-  const dim3 grid((unsigned)gx, (unsigned)B);
-#define SNB_RBF(LL) rb::rb_composite_fwd_kernel<LL><<<grid, 256, 0, st>>>(at<float>(ws, L.sigma_c), at<float>(ws, L.rgb_c), zsrc, \
+  const CompositeGrid cg(N, S, B);
+#define SNB_RBF(LL) rb::rb_composite_fwd_kernel<LL><<<cg.grid, 256, 0, st>>>(at<float>(ws, L.sigma_c), at<float>(ws, L.rgb_c), zsrc, \
     at<int32_t>(ws, L.order), at<rb::ObjCounts>(ws, L.counts), N, S, d->flags, out_rgb, out_depth, out_acc)
-  if (lpr == 8) SNB_RBF(8); else if (lpr == 16) SNB_RBF(16); else SNB_RBF(32);
+  if (cg.lpr == 8) SNB_RBF(8); else if (cg.lpr == 16) SNB_RBF(16); else SNB_RBF(32);
 #undef SNB_RBF
   SNB_LAUNCH_CHECK();
   return 0;
@@ -989,20 +778,14 @@ extern "C" int snb_render_batch_bwd(snb_handle h, const snb_batch_desc* d, const
   void* sc = scratch;
   const int B = d->n_objs, S = d->n_samples;
   const int64_t N = d->rays_per_obj;
-  const int sms = sm_count();
-  SNB_REQUIRE(sms > 0, "render_batch_bwd: no CUDA device (there is no CPU fallback)");
+  SNB_REQUIRE(sm_count() > 0, "render_batch_bwd: no CUDA device (there is no CPU fallback)");
   const bool pose = g_c2w != nullptr;
-  const int lpr = S <= 32 ? 8 : (S <= 64 ? 16 : 32);
-  int gx = (int)ceil_div(ceil_div(N, 32 / lpr), 8);
-  const int cap = (sms * 8 + B - 1) / B;
-  if (gx > cap) gx = cap;
-  if (gx < 1) gx = 1;
-  const dim3 grid((unsigned)gx, (unsigned)B);
+  const CompositeGrid cg(N, S, B);
   float* gz = pose ? at<float>(sc, G.g_z_c) : nullptr;
   const bool fused = (d->flags & SNB_BATCH_FUSED_SAMPLER) != 0;
   const float *xyz_c = at<float>(ws, L.xyz_c), *vrep_c = at<float>(ws, L.vrep_c), *z_c = at<float>(ws, L.z_c);
   if (fused) {   // the executed rows' coordinates and depths for the backward (the forward kept none)
-    rb::rb_gather_kernel<<<ew_grid(L.Mmax, 8), 256, 0, st>>>(at<float>(ws, L.rays8), box, z_steps, jitter, at<int32_t>(ws, L.order),
+    rb::rb_gather_kernel<<<grid_1d(L.Mmax, 256, 8), 256, 0, st>>>(at<float>(ws, L.rays8), box, z_steps, jitter, at<int32_t>(ws, L.order),
                                                             at<rb::ObjCounts>(ws, L.counts), at<rb::Meta>(ws, L.meta), B, N, S,
                                                             at<float>(sc, G.xyz_c), at<float>(sc, G.vrep_c), at<float>(sc, G.z_c));
     SNB_LAUNCH_CHECK();
@@ -1010,10 +793,10 @@ extern "C" int snb_render_batch_bwd(snb_handle h, const snb_batch_desc* d, const
   }
   const int64_t* total_rows = &at<rb::Meta>(ws, L.meta)->total_rows;
   SNB_CHECK_CUDA(cudaMemsetAsync(at<uint8_t>(sc, G.live_hdr), 0, G.live_end - G.live_hdr, st));   // count, ticket, flags
-#define SNB_RBB(LL) rb::rb_composite_bwd_kernel<LL><<<grid, 256, 0, st>>>(at<float>(ws, L.sigma_c), at<float>(ws, L.rgb_c), z_c, \
+#define SNB_RBB(LL) rb::rb_composite_bwd_kernel<LL><<<cg.grid, 256, 0, st>>>(at<float>(ws, L.sigma_c), at<float>(ws, L.rgb_c), z_c, \
     at<int32_t>(ws, L.order), at<rb::ObjCounts>(ws, L.counts), N, S, d->flags, g_rgb, g_depth, g_acc, at<float>(sc, G.g_sigma_c), \
     at<float>(sc, G.g_rgb_c), gz, total_rows, at<uint8_t>(sc, G.live), at<int32_t>(sc, G.live_list), at<rb::LiveHdr>(sc, G.live_hdr))
-  if (lpr == 8) SNB_RBB(8); else if (lpr == 16) SNB_RBB(16); else SNB_RBB(32);
+  if (cg.lpr == 8) SNB_RBB(8); else if (cg.lpr == 16) SNB_RBB(16); else SNB_RBB(32);
 #undef SNB_RBB
   SNB_LAUNCH_CHECK();
   if (decoder_backward(h, batch_precision(*d), xyz_c, vrep_c, L.Mmax, B, shape_latent, texture_latent, at<float>(ws, L.sigma_c),
@@ -1024,47 +807,9 @@ extern "C" int snb_render_batch_bwd(snb_handle h, const snb_batch_desc* d, const
     return 1;
   if (!pose) return 0;
   SNB_CHECK_CUDA(cudaMemsetAsync(at<uint8_t>(sc, G.acc64), 0, G.mlp - G.acc64, st));   // fp64 sums + tickets
-  int gr = (int)ceil_div(N, 256);
-  if (gr > cap) gr = cap;
-  if (gr < 1) gr = 1;
-  rb::rb_rays_bwd_kernel<<<dim3((unsigned)gr, (unsigned)B), 256, 0, st>>>(px, py, K, c2w, box, at<float>(ws, L.rays8), at<uint8_t>(ws, L.hit),
+  rb::rb_rays_bwd_kernel<<<dim3((unsigned)grid_1d(N, 256, 8, B), (unsigned)B), 256, 0, st>>>(px, py, K, c2w, box, at<float>(ws, L.rays8), at<uint8_t>(ws, L.hit),
       at<int32_t>(ws, L.pos), at<rb::ObjCounts>(ws, L.counts), z_steps, jitter, N, S, at<float>(sc, G.g_xyz_c), at<float>(sc, G.g_vrep_c), gz,
       at<uint8_t>(sc, G.live), at<double>(sc, G.acc64), at<unsigned int>(sc, G.tickets), g_c2w);
-  SNB_LAUNCH_CHECK();
-  return 0;
-}
-
-extern "C" size_t snb_refine_loss_batch_scratch_bytes(int32_t n_objs) { return n_objs > 0 ? (size_t)n_objs * sizeof(rb::LossAccB) : 0; }
-
-extern "C" int snb_refine_loss_batch_fwd(const float* rgb, const float* acc, const float* tgt, const float* occ, int32_t n_objs,
-                                         int64_t rays_per_obj, float occ_coef, float* out3, void* scratch, void* stream) {
-  SNB_REQUIRE(n_objs >= 1 && rays_per_obj >= 1 && rgb && acc && tgt && occ && out3 && scratch, "refine_loss_batch_fwd: bad arguments");
-  const int sms = sm_count();
-  SNB_REQUIRE(sms > 0, "refine_loss_batch_fwd: no CUDA device (there is no CPU fallback)");
-  cudaStream_t st = (cudaStream_t)stream;
-  SNB_CHECK_CUDA(cudaMemsetAsync(scratch, 0, (size_t)n_objs * sizeof(rb::LossAccB), st));
-  int gx = (int)ceil_div(rays_per_obj, 256);
-  const int cap = (2 * sms + n_objs - 1) / n_objs;
-  if (gx > cap) gx = cap;
-  if (gx < 1) gx = 1;
-  rb::rb_loss_fwd_kernel<<<dim3((unsigned)gx, (unsigned)n_objs), 256, 0, st>>>(rgb, acc, tgt, occ, rays_per_obj, occ_coef,
-                                                                              (rb::LossAccB*)scratch, out3);
-  SNB_LAUNCH_CHECK();
-  return 0;
-}
-
-extern "C" int snb_refine_loss_batch_bwd(const float* rgb, const float* acc, const float* tgt, const float* occ, int32_t n_objs,
-                                         int64_t rays_per_obj, float occ_coef, const void* scratch, const float* g_loss, float* g_rgb,
-                                         float* g_acc, void* stream) {
-  SNB_REQUIRE(n_objs >= 1 && rays_per_obj >= 1 && rgb && acc && tgt && occ && scratch && g_rgb && g_acc, "refine_loss_batch_bwd: bad arguments");
-  const int sms = sm_count();
-  SNB_REQUIRE(sms > 0, "refine_loss_batch_bwd: no CUDA device (there is no CPU fallback)");
-  int gx = (int)ceil_div(rays_per_obj, 256);
-  const int cap = (8 * sms + n_objs - 1) / n_objs;
-  if (gx > cap) gx = cap;
-  if (gx < 1) gx = 1;
-  rb::rb_loss_bwd_kernel<<<dim3((unsigned)gx, (unsigned)n_objs), 256, 0, (cudaStream_t)stream>>>(rgb, acc, tgt, occ, rays_per_obj, occ_coef,
-                                                                                                (const rb::LossAccB*)scratch, g_loss, g_rgb, g_acc);
   SNB_LAUNCH_CHECK();
   return 0;
 }
@@ -1075,12 +820,10 @@ extern "C" int snb_prepare_samples_batch(const float* px, const float* py, const
   SNB_REQUIRE(n_objs >= 1 && rays_per_obj >= 0 && n_samples >= 1, "prepare_samples_batch: bad sizes");
   if (rays_per_obj == 0) return 0;
   SNB_REQUIRE(px && py && K && c2w && z && obj_diag && xyz && viewdir_rep, "prepare_samples_batch: null pointer");
-  const int sms = sm_count();
-  SNB_REQUIRE(sms > 0, "prepare_samples_batch: no CUDA device (there is no CPU fallback)");
   const int64_t total = (int64_t)n_objs * rays_per_obj;
-  int64_t grid = ceil_div(total, 8);
-  if (grid > (int64_t)sms * 8) grid = (int64_t)sms * 8;
-  rb::rb_shell_prep_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(px, py, K, c2w, z, obj_diag, flip, rays_per_obj, n_samples,
+  const int grid = grid_1d(total, 8, 8);
+  SNB_REQUIRE(grid > 0, "prepare_samples_batch: no CUDA device (there is no CPU fallback)");
+  rb::rb_shell_prep_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(px, py, K, c2w, z, obj_diag, flip, rays_per_obj, n_samples,
                                                                            shapenet_swap, total, xyz, viewdir_rep);
   SNB_LAUNCH_CHECK();
   return 0;
@@ -1184,13 +927,9 @@ extern "C" int snb_render_shell_batch_bwd(snb_handle h, const snb_shell_batch_de
                   pose ? at<float>(sc, G.g_xyz) : nullptr, pose ? at<float>(sc, G.g_vrep) : nullptr, g_shape_latent, g_texture_latent, nullptr,
                   stream)) return 1;
   if (!pose) return 0;
-  const int sms = sm_count();
-  SNB_REQUIRE(sms > 0, "render_shell_batch_bwd: no CUDA device (there is no CPU fallback)");
+  const int gx = grid_1d(N, 8, 8, B);
+  SNB_REQUIRE(gx > 0, "render_shell_batch_bwd: no CUDA device (there is no CPU fallback)");
   SNB_CHECK_CUDA(cudaMemsetAsync(at<uint8_t>(sc, G.acc64), 0, G.mlp - G.acc64, st));   // fp64 sums + tickets
-  int gx = (int)ceil_div(N, 8);
-  const int cap = (sms * 8 + B - 1) / B;
-  if (gx > cap) gx = cap;
-  if (gx < 1) gx = 1;
   rb::rb_shell_rays_bwd_kernel<<<dim3((unsigned)gx, (unsigned)B), 256, 0, st>>>(px, py, K, c2w, z, obj_diag, N, d->n_samples, d->shapenet_swap,
       at<float>(sc, G.g_xyz), at<float>(sc, G.g_vrep), at<double>(sc, G.acc64), at<unsigned int>(sc, G.tickets), g_c2w);
   SNB_LAUNCH_CHECK();

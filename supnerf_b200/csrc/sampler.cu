@@ -15,23 +15,13 @@ __global__ void __launch_bounds__(256) get_rays_fwd_kernel(const float* __restri
                                                           int64_t n, const float* __restrict__ K,
                                                           const float* __restrict__ c2w, float* __restrict__ rays_o,
                                                           float* __restrict__ viewdir) {
-  const float cx = K[2], cy = K[5], fx = K[0], fy = K[4];
-  float R[9], t[3];
-#pragma unroll
-  for (int i = 0; i < 3; ++i) {
-    R[3 * i] = c2w[4 * i]; R[3 * i + 1] = c2w[4 * i + 1]; R[3 * i + 2] = c2w[4 * i + 2]; t[i] = c2w[4 * i + 3];
-  }
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-    const float p0 = __fdiv_rn(__fsub_rn(px[i], cx), fx), p1 = __fdiv_rn(__fsub_rn(py[i], cy), fy), p2 = 1.f;
-    float r[3];
-#pragma unroll
-    for (int a = 0; a < 3; ++a)
-      r[a] = __fadd_rn(__fadd_rn(__fmul_rn(p0, R[3 * a]), __fmul_rn(p1, R[3 * a + 1])), __fmul_rn(p2, R[3 * a + 2]));
-    const float nrm = sqrtf(__fadd_rn(__fadd_rn(__fmul_rn(r[0], r[0]), __fmul_rn(r[1], r[1])), __fmul_rn(r[2], r[2])));
+    float d[3];
+    pixel_dir(K, c2w, px[i], py[i], d);
 #pragma unroll
     for (int a = 0; a < 3; ++a) {
-      viewdir[3 * i + a] = __fdiv_rn(r[a], nrm);
-      rays_o[3 * i + a] = t[a];
+      viewdir[3 * i + a] = d[a];
+      rays_o[3 * i + a] = __ldg(c2w + 4 * a + 3);
     }
   }
 }
@@ -42,30 +32,18 @@ __global__ void __launch_bounds__(256) get_rays_bwd_kernel(const float* __restri
                                                           const float* __restrict__ c2w,
                                                           const float* __restrict__ g_o, const float* __restrict__ g_d,
                                                           float* __restrict__ g_c2w) {
-  const float cx = K[2], cy = K[5], fx = K[0], fy = K[4];
-  float R[9];
-#pragma unroll
-  for (int i = 0; i < 3; ++i) { R[3 * i] = c2w[4 * i]; R[3 * i + 1] = c2w[4 * i + 1]; R[3 * i + 2] = c2w[4 * i + 2]; }
   float acc[12];
 #pragma unroll
   for (int i = 0; i < 12; ++i) acc[i] = 0.f;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-    const float p[3] = {(px[i] - cx) / fx, (py[i] - cy) / fy, 1.f};
-    float r[3], d[3];
-#pragma unroll
-    for (int a = 0; a < 3; ++a) r[a] = p[0] * R[3 * a] + p[1] * R[3 * a + 1] + p[2] * R[3 * a + 2];
-    const float nrm = sqrtf(r[0] * r[0] + r[1] * r[1] + r[2] * r[2]);
-    const float inv = 1.f / nrm;
-#pragma unroll
-    for (int a = 0; a < 3; ++a) d[a] = r[a] * inv;
     const float gd[3] = {g_d[3 * i], g_d[3 * i + 1], g_d[3 * i + 2]};
-    const float dot = gd[0] * d[0] + gd[1] * d[1] + gd[2] * d[2];
+    float p[3], gr[3];
+    dir_grad_to_pose(K, c2w, px[i], py[i], gd, p, gr);
 #pragma unroll
     for (int a = 0; a < 3; ++a) {
-      const float gr = (gd[a] - d[a] * dot) * inv;
-      acc[4 * a + 0] += gr * p[0];
-      acc[4 * a + 1] += gr * p[1];
-      acc[4 * a + 2] += gr * p[2];
+      acc[4 * a + 0] += gr[a] * p[0];
+      acc[4 * a + 1] += gr[a] * p[1];
+      acc[4 * a + 2] += gr[a] * p[2];
       acc[4 * a + 3] += g_o[3 * i + a];
     }
   }
@@ -183,32 +161,19 @@ __global__ void __launch_bounds__(256) sample_box_bwd_kernel(
     const Slab sl = slab_test(o, d, half);
     const float near = sl.hit ? sl.t_near : -1.f, far = sl.hit ? sl.t_far : -1.f;
     const float dn = sqrtf(d[0] * d[0] + d[1] * d[1] + d[2] * d[2]);
-    float gon[3] = {0.f, 0.f, 0.f}, gd[3] = {0.f, 0.f, 0.f}, gzabs = 0.f, gnear = 0.f, gfar = 0.f;
+    float g[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};   // d o (3), d d (3), d |z|, d near, d far
     for (int k = lane; k < S; k += 32) {
       const int64_t idx = ray * S + k;
-      const float zs = __fadd_rn(__ldg(z_steps + k), __fmul_rn(__ldg(jitter + idx), fstep));
-      const float zc = __fadd_rn(__fmul_rn(near, __fsub_rn(1.f, zs)), __fmul_rn(far, zs));
-      float gx[3] = {0.f, 0.f, 0.f};
       // compacted gradients: S rows per hit ray; a miss ray's single row stands for all its samples and is credited to the last one
       int64_t gidx = idx;
       if (cpos != nullptr) gidx = sl.hit ? (int64_t)cpos[ray] * S + k : (k == S - 1 ? ccounts[0] * S + cpos[ray] : -1);
-      if (g_xyz && gidx >= 0) { gx[0] = __ldg(g_xyz + 3 * gidx); gx[1] = __ldg(g_xyz + 3 * gidx + 1); gx[2] = __ldg(g_xyz + 3 * gidx + 2); }
-      float gz = gx[0] * d[0] + gx[1] * d[1] + gx[2] * d[2];
-#pragma unroll
-      for (int a = 0; a < 3; ++a) { gon[a] += gx[a]; gd[a] += zc * gx[a]; }
-      if (g_vrep && gidx >= 0) { gd[0] += __ldg(g_vrep + 3 * gidx); gd[1] += __ldg(g_vrep + 3 * gidx + 1); gd[2] += __ldg(g_vrep + 3 * gidx + 2); }
-      if (g_zv) {
-        const float gv = __ldg(g_zv + idx);
-        const float sgn = (zc > 0.f) ? 1.f : ((zc < 0.f) ? -1.f : 0.f);
-        gz += gv * sgn * dn * half_diag;
-        gzabs += gv * fabsf(zc);
-      }
-      gnear += gz * (1.f - zs);
-      gfar += gz * zs;
+      fold_sample_grad((g_xyz && gidx >= 0) ? g_xyz + 3 * gidx : nullptr, (g_vrep && gidx >= 0) ? g_vrep + 3 * gidx : nullptr,
+                       g_zv ? g_zv + idx : nullptr, __ldg(z_steps + k), __ldg(jitter + idx), fstep, near, far, d, dn, half_diag, g);
     }
 #pragma unroll
-    for (int a = 0; a < 3; ++a) { gon[a] = warp_sum(gon[a]); gd[a] = warp_sum(gd[a]); }
-    gzabs = warp_sum(gzabs); gnear = warp_sum(gnear); gfar = warp_sum(gfar);
+    for (int i = 0; i < 9; ++i) g[i] = warp_sum(g[i]);
+    float gon[3] = {g[0], g[1], g[2]}, gd[3] = {g[3], g[4], g[5]};
+    const float gzabs = g[6], gnear = g[7], gfar = g[8];
     if (lane == 0) {
       if (dn > 0.f) {
 #pragma unroll
@@ -291,14 +256,6 @@ __global__ void __launch_bounds__(256) sample_shell_bwd_kernel(
   }
 }
 
-static int ray_grid(int64_t n_rays, int per_block) {
-  int sms = sm_count();
-  if (sms <= 0) return -1;
-  int64_t blocks = ceil_div(n_rays, per_block);
-  int64_t cap = (int64_t)sms * 8;
-  return (int)(blocks < cap ? (blocks > 0 ? blocks : 1) : cap);
-}
-
 }  // namespace snb
 
 using namespace snb;
@@ -306,7 +263,7 @@ using namespace snb;
 extern "C" int snb_get_rays_fwd(const float* px, const float* py, int64_t n_rays, const float* K, const float* c2w,
                                 float* rays_o, float* viewdir, void* stream) {
   if (n_rays == 0) return 0;
-  int grid = ray_grid(n_rays, 256);
+  int grid = grid_1d(n_rays, 256, 8);
   SNB_REQUIRE(grid > 0, "get_rays_fwd: no CUDA device");
   get_rays_fwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(px, py, n_rays, K, c2w, rays_o, viewdir);
   SNB_LAUNCH_CHECK();
@@ -316,10 +273,8 @@ extern "C" int snb_get_rays_fwd(const float* px, const float* py, int64_t n_rays
 extern "C" int snb_get_rays_bwd(const float* px, const float* py, int64_t n_rays, const float* K, const float* c2w,
                                 const float* g_rays_o, const float* g_viewdir, float* g_c2w, void* stream) {
   if (n_rays == 0) return 0;
-  int sms = sm_count();
-  SNB_REQUIRE(sms > 0, "get_rays_bwd: no CUDA device");
-  int64_t blocks = ceil_div(n_rays, 256 * 4);
-  int grid = (int)(blocks < sms ? (blocks > 0 ? blocks : 1) : sms);
+  const int grid = grid_1d(n_rays, 256 * 4, 1);
+  SNB_REQUIRE(grid > 0, "get_rays_bwd: no CUDA device");
   get_rays_bwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(px, py, n_rays, K, c2w, g_rays_o, g_viewdir, g_c2w);
   SNB_LAUNCH_CHECK();
   return 0;
@@ -329,7 +284,7 @@ extern "C" int snb_ray_box_fwd(const float* ray_o, const float* ray_d, const flo
                                int64_t n_rays, float* t_near, float* t_far, uint8_t* hit, void* stream) {
   SNB_REQUIRE((aabb_min == nullptr) == (aabb_max == nullptr), "ray_box_fwd: give both aabb corners or neither");
   if (n_rays == 0) return 0;
-  int grid = ray_grid(n_rays, 256);
+  int grid = grid_1d(n_rays, 256, 8);
   SNB_REQUIRE(grid > 0, "ray_box_fwd: no CUDA device");
   ray_box_fwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(ray_o, ray_d, aabb_min, aabb_max, n_rays, t_near, t_far, hit);
   SNB_LAUNCH_CHECK();
@@ -341,7 +296,7 @@ extern "C" int snb_ray_box_bwd(const float* ray_o, const float* ray_d, const flo
                                float* g_aabb_min, float* g_aabb_max, void* stream) {
   SNB_REQUIRE((aabb_min == nullptr) == (aabb_max == nullptr), "ray_box_bwd: give both aabb corners or neither");
   if (n_rays == 0) return 0;
-  int grid = ray_grid(n_rays, 256);
+  int grid = grid_1d(n_rays, 256, 8);
   SNB_REQUIRE(grid > 0, "ray_box_bwd: no CUDA device");
   ray_box_bwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(ray_o, ray_d, aabb_min, aabb_max, n_rays, g_near, g_far,
                                                              g_ray_o, g_ray_d, g_aabb_min, g_aabb_max);
@@ -354,7 +309,7 @@ extern "C" int snb_sample_box_fwd(const float* rays_o, const float* viewdir, con
                                   float* xyz, float* viewdir_rep, float* z_vals, uint8_t* hit, void* stream) {
   SNB_REQUIRE(n_samples >= 1 && h != nullptr, "sample_box_fwd: bad arguments");
   if (n_rays == 0) return 0;
-  int grid = ray_grid(n_rays, 8);
+  int grid = grid_1d(n_rays, 8, 8);
   SNB_REQUIRE(grid > 0, "sample_box_fwd: no CUDA device");
   sample_box_fwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(rays_o, viewdir, z_steps, jitter, n_rays, n_samples,
                                                                 half_diag, h[0], h[1], h[2], xyz, viewdir_rep, z_vals, hit);
@@ -368,7 +323,7 @@ extern "C" int snb_sample_box_bwd(const float* rays_o, const float* viewdir, con
                                   float* g_rays_o, float* g_viewdir, int32_t detach_bounds, void* stream) {
   SNB_REQUIRE(n_samples >= 1 && h != nullptr, "sample_box_bwd: bad arguments");
   if (n_rays == 0) return 0;
-  int grid = ray_grid(n_rays, 8);
+  int grid = grid_1d(n_rays, 8, 8);
   SNB_REQUIRE(grid > 0, "sample_box_bwd: no CUDA device");
   sample_box_bwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(rays_o, viewdir, z_steps, jitter, n_rays, n_samples,
                                                                 half_diag, h[0], h[1], h[2], g_xyz, g_viewdir_rep, g_z_vals,
@@ -385,7 +340,7 @@ int sample_box_bwd_compact(const float* rays_o, const float* viewdir, const floa
                            const float* g_z_vals, const int32_t* pos, const int64_t* counts, float* g_rays_o, float* g_viewdir,
                            cudaStream_t st) {
   if (n_rays == 0) return 0;
-  int grid = ray_grid(n_rays, 8);
+  int grid = grid_1d(n_rays, 8, 8);
   SNB_REQUIRE(grid > 0, "sample_box_bwd: no CUDA device");
   sample_box_bwd_kernel<<<grid, 256, 0, st>>>(rays_o, viewdir, z_steps, jitter, n_rays, n_samples, half_diag, h[0], h[1], h[2],
                                               g_xyz_c, g_vrep_c, g_z_vals, g_rays_o, g_viewdir, pos, counts, 0);
@@ -398,7 +353,7 @@ extern "C" int snb_sample_shell_fwd(const float* rays_o, const float* viewdir, c
                                     int32_t n_samples, float obj_diag, int32_t shapenet_swap,
                                     float* xyz, float* viewdir_rep, void* stream) {
   if (n_rays == 0) return 0;
-  int grid = ray_grid(n_rays, 8);
+  int grid = grid_1d(n_rays, 8, 8);
   SNB_REQUIRE(grid > 0, "sample_shell_fwd: no CUDA device");
   sample_shell_fwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(rays_o, viewdir, z, n_rays, n_samples, obj_diag,
                                                                   shapenet_swap, xyz, viewdir_rep);
@@ -410,7 +365,7 @@ extern "C" int snb_sample_shell_bwd(const float* z, int64_t n_rays, int32_t n_sa
                                     const float* g_xyz, const float* g_viewdir_rep,
                                     float* g_rays_o, float* g_viewdir, void* stream) {
   if (n_rays == 0) return 0;
-  int grid = ray_grid(n_rays, 8);
+  int grid = grid_1d(n_rays, 8, 8);
   SNB_REQUIRE(grid > 0, "sample_shell_bwd: no CUDA device");
   sample_shell_bwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(z, n_rays, n_samples, obj_diag, shapenet_swap, g_xyz,
                                                                   g_viewdir_rep, g_rays_o, g_viewdir);
@@ -462,11 +417,9 @@ extern "C" int snb_stratified_z_fwd(const float* rays, int32_t row_floats, const
   SNB_REQUIRE(n_rays >= 0 && n_samples >= 1 && row_floats >= 2, "stratified_z_fwd: bad arguments");
   if (n_rays == 0) return 0;
   SNB_REQUIRE(rays && z_steps && jitter && z, "stratified_z_fwd: null pointer");
-  const int sms = sm_count();
-  SNB_REQUIRE(sms > 0, "stratified_z_fwd: no CUDA device");
-  int64_t grid = (n_rays * n_samples + 255) / 256;
-  if (grid > (int64_t)sms * 16) grid = (int64_t)sms * 16;
-  stratified_z_fwd_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(rays, row_floats, z_steps, jitter, n_rays, n_samples, z);
+  const int grid = grid_1d(n_rays * n_samples, 256, 16);
+  SNB_REQUIRE(grid > 0, "stratified_z_fwd: no CUDA device");
+  stratified_z_fwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(rays, row_floats, z_steps, jitter, n_rays, n_samples, z);
   SNB_LAUNCH_CHECK();
   return 0;
 }
@@ -476,7 +429,7 @@ extern "C" int snb_stratified_z_bwd(const float* z_steps, const float* jitter, i
   SNB_REQUIRE(n_rays >= 0 && n_samples >= 1, "stratified_z_bwd: bad arguments");
   if (n_rays == 0) return 0;
   SNB_REQUIRE(z_steps && jitter && g_z && g_near && g_far, "stratified_z_bwd: null pointer");
-  int grid = ray_grid(n_rays, 8);
+  int grid = grid_1d(n_rays, 8, 8);
   SNB_REQUIRE(grid > 0, "stratified_z_bwd: no CUDA device");
   stratified_z_bwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(z_steps, jitter, n_rays, n_samples, g_z, g_near, g_far);
   SNB_LAUNCH_CHECK();
@@ -527,11 +480,9 @@ extern "C" int snb_jitter_fill(uint64_t seed, const int64_t* ray_ids, int64_t n_
   SNB_REQUIRE(n_rays > 0 && n_samples >= 1 && out, "jitter_fill: bad arguments");
   SNB_REQUIRE((n_samples & 3) != 0 || ((uintptr_t)out & 15) == 0, "jitter_fill: out must be 16-byte aligned");
   const int64_t total = n_rays * ((n_samples + 3) / 4);
-  const int sms = sm_count();
-  SNB_REQUIRE(sms > 0, "jitter_fill: no CUDA device");
-  int64_t grid = (total + 255) / 256;
-  if (grid > (int64_t)sms * 16) grid = (int64_t)sms * 16;
-  jitter_fill_kernel<<<(unsigned)grid, 256, 0, (cudaStream_t)stream>>>(seed, ray_ids, n_rays, n_samples, out);
+  const int grid = grid_1d(total, 256, 16);
+  SNB_REQUIRE(grid > 0, "jitter_fill: no CUDA device");
+  jitter_fill_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(seed, ray_ids, n_rays, n_samples, out);
   SNB_LAUNCH_CHECK();
   return 0;
 }

@@ -1,4 +1,5 @@
-// Device helpers of the ray / box-sampler kernels (sampler.cu), shared with the batched render (render_batch.cu).
+// Device helpers of the ray / box-sampler kernels (sampler.cu), shared with the batched render (render_batch.cu): each is the one
+// copy of its arithmetic, so the per-object and the batched paths compute the same bits.
 #pragma once
 #include "common.cuh"
 #include <math.h>
@@ -78,6 +79,62 @@ __device__ __forceinline__ void slab_backward(const Slab& sl, const float o[3], 
     const float ginv = gmin_a * (lo[a] - o[a]) + gmax_a * (hi[a] - o[a]);
     gd[a] = -ginv * sl.inv[a] * sl.inv[a];
   }
+}
+
+// utils.get_rays for one pixel: dirs = ((px - cx) / fx, (py - cy) / fy, 1); rays_d = sum(dirs * R, -1); viewdir = rays_d / |rays_d|,
+// as separate round-to-nearest fp32 ops.  K (3,3) and c2w (3,4) row-major; the caller forms the origin.
+__device__ __forceinline__ void pixel_dir(const float* __restrict__ K, const float* __restrict__ c2w, float px, float py, float d[3]) {
+  const float cx = __ldg(K + 2), cy = __ldg(K + 5), fx = __ldg(K), fy = __ldg(K + 4);
+  const float p0 = __fdiv_rn(__fsub_rn(px, cx), fx), p1 = __fdiv_rn(__fsub_rn(py, cy), fy), p2 = 1.f;
+  float r[3];
+#pragma unroll
+  for (int a = 0; a < 3; ++a)
+    r[a] = __fadd_rn(__fadd_rn(__fmul_rn(p0, __ldg(c2w + 4 * a)), __fmul_rn(p1, __ldg(c2w + 4 * a + 1))), __fmul_rn(p2, __ldg(c2w + 4 * a + 2)));
+  const float nrm = sqrtf(__fadd_rn(__fadd_rn(__fmul_rn(r[0], r[0]), __fmul_rn(r[1], r[1])), __fmul_rn(r[2], r[2])));
+#pragma unroll
+  for (int a = 0; a < 3; ++a) d[a] = __fdiv_rn(r[a], nrm);
+}
+
+// Backward of the box sampler for one sample k of a ray (o, d, near, far):
+//   zs = z_steps[k] + jitter[k] / S;  z = near (1 - zs) + far zs;  xyz = o + z d;  z_vals = |z d| * half_diag
+// g_x, g_v, g_z point at the sample's d xyz (3), d viewdir (3) and d z_vals, or are NULL where those are zero.  Adds the sample's
+// share to g = {d o (3), d d (3, without the |z d| term), d |z| (the |z d| term's factor), d near, d far}; dn = |d|.
+__device__ __forceinline__ void fold_sample_grad(const float* __restrict__ g_x, const float* __restrict__ g_v, const float* __restrict__ g_z,
+                                                 float z_step, float jit, float fstep, float near, float far, const float d[3], float dn,
+                                                 float half_diag, float g[9]) {
+  const float zs = __fadd_rn(z_step, __fmul_rn(jit, fstep));
+  const float zc = __fadd_rn(__fmul_rn(near, __fsub_rn(1.f, zs)), __fmul_rn(far, zs));
+  float gx[3] = {0.f, 0.f, 0.f};
+  if (g_x != nullptr) { gx[0] = __ldg(g_x); gx[1] = __ldg(g_x + 1); gx[2] = __ldg(g_x + 2); }
+  float gz = gx[0] * d[0] + gx[1] * d[1] + gx[2] * d[2];
+#pragma unroll
+  for (int a = 0; a < 3; ++a) { g[a] += gx[a]; g[3 + a] += zc * gx[a]; }
+  if (g_v != nullptr) { g[3] += __ldg(g_v); g[4] += __ldg(g_v + 1); g[5] += __ldg(g_v + 2); }
+  if (g_z != nullptr) {
+    const float gv = __ldg(g_z);
+    const float sgn = (zc > 0.f) ? 1.f : ((zc < 0.f) ? -1.f : 0.f);
+    gz += gv * sgn * dn * half_diag;
+    g[6] += gv * fabsf(zc);
+  }
+  g[7] += gz * (1.f - zs);
+  g[8] += gz * zs;
+}
+
+// Backward of get_rays' direction for one pixel: r = R p, p = ((px - cx) / fx, (py - cy) / fy, 1), d = r / |r|.
+// g_r = (g_d - d (g_d . d)) / |r|; the pose gets d c2w[a][j < 3] = g_r[a] p[j], which the caller accumulates in its own precision.
+__device__ __forceinline__ void dir_grad_to_pose(const float* __restrict__ K, const float* __restrict__ c2w, float px, float py,
+                                                 const float g_d[3], float pp[3], float g_r[3]) {
+  const float cx = __ldg(K + 2), cy = __ldg(K + 5), fx = __ldg(K), fy = __ldg(K + 4);
+  pp[0] = (px - cx) / fx; pp[1] = (py - cy) / fy; pp[2] = 1.f;
+  float r[3], d[3];
+#pragma unroll
+  for (int a = 0; a < 3; ++a) r[a] = pp[0] * __ldg(c2w + 4 * a) + pp[1] * __ldg(c2w + 4 * a + 1) + pp[2] * __ldg(c2w + 4 * a + 2);
+  const float inv = 1.f / sqrtf(r[0] * r[0] + r[1] * r[1] + r[2] * r[2]);
+#pragma unroll
+  for (int a = 0; a < 3; ++a) d[a] = r[a] * inv;
+  const float dot = g_d[0] * d[0] + g_d[1] * d[1] + g_d[2] * d[2];
+#pragma unroll
+  for (int a = 0; a < 3; ++a) g_r[a] = (g_d[a] - d[a] * dot) * inv;
 }
 
 }  // namespace snb

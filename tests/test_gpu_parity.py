@@ -510,6 +510,22 @@ def test_refine_loss_kernel_vs_oracle(n):
     den = torch.tensor([2.0 * occ.abs().sum().item() + 1e-9], device=DEV)
     half = S.losses.refine_loss(rgb.to(DEV), acc.to(DEV), tgt.to(DEV), occ.to(DEV), 0.1, den=den)[0]
     assert parity_ok("half", half, 0.5 * l64[0], TOL)
+    # B objects in one launch per direction (refine_loss_batch) against the per-object entry point on the same rows: the fp64 sums
+    # may be added in another order, the gradients are the same arithmetic bit for bit
+    B = 3
+    rgb_b, tgt_b, acc_b = torch.rand(B, n, 3, generator=g), torch.rand(B, n, 3, generator=g), torch.rand(B, n, generator=g)
+    occ_b = torch.randint(-1, 2, (B, n, 1), generator=g).float()
+    if n == 1:
+        occ_b[:] = 1.0
+    rb, ab = rgb_b.to(DEV).requires_grad_(), acc_b.to(DEV).requires_grad_()
+    loss_b, parts_b = S.losses.refine_loss_batch(rb, ab, tgt_b.to(DEV), occ_b.to(DEV), 0.1)
+    (3.0 * loss_b).sum().backward()
+    for i in range(B):
+        ri, ai = rgb_b[i].to(DEV).requires_grad_(), acc_b[i].to(DEV).requires_grad_()
+        li, vec = S.losses.refine_loss_vec(ri, ai, tgt_b[i].to(DEV), occ_b[i].to(DEV), 0.1)
+        (3.0 * li).backward()
+        torch.testing.assert_close(parts_b[i], vec, rtol=1e-6, atol=0)
+        assert torch.equal(rb.grad[i], ri.grad) and torch.equal(ab.grad[i], ai.grad)
     with pytest.raises(S._lib.SnbError):
         S.losses.refine_loss(rgb, acc, tgt, occ)   # CPU tensors: no fallback
 
