@@ -347,6 +347,25 @@ int snb_refine_pose_batch_fwd(const float* rot_vec, const float* trans_vec, int3
                               const float* step_counter, int32_t table_rows, float* cam, float* z, float* z2, void* stream);
 int snb_refine_pose_batch_bwd(const float* rot_vec, const float* trans_vec, int32_t n_objs, int32_t opt_cam_pose,
                               const float* g_cam, float* g_rot, float* g_trans, void* stream);
+/* ---- the same glue for a stream of objects through C fixed slots (refine.SlotRefiner) ---------------------------------
+ * snb_refine_pose_slots_fwd: snb_refine_pose_batch_fwd with one step counter per slot: slot b reads row int(step_counters[b])
+ * of its jitter table(s) (C, table_rows, S).  active (C bytes, NULL = all active): an active slot whose counter lies outside
+ * [0, table_rows) gets NaN in its z / z2 and sets *err_flag to 1 (a device int32, NULL = not reported); an inactive slot
+ * reads a row inside the table and reports nothing.  The backward is snb_refine_pose_batch_bwd.
+ * snb_adamw_step_rows: snb_adamw_step on n_rows independent rows of every tensor (row r of tensor i: row_sizes[i] elements
+ * at r * row_sizes[i]).  steps (n_rows device floats): each row's step count -- its bias corrections -- incremented by the
+ * call; active (n_rows bytes, NULL = all active): an inactive row's parameters, moments and count stay bit-for-bit unchanged.
+ * snb_adamw_step is the one-row case.  loss_history (NULL = none): (n_rows, history_rows, 4); an active row r with
+ * 0 <= steps[r] < history_rows first writes {loss3[3r .. 3r+2], loss_rgb2[r * loss_rgb2_stride]} to row steps[r]. */
+int snb_refine_pose_slots_fwd(const float* rot_vec, const float* trans_vec, int32_t n_slots, int32_t opt_cam_pose,
+                              const float* obj_diag, int32_t n_samples, const float* jitter, const float* jitter2,
+                              const float* step_counters, int32_t table_rows, const uint8_t* active, int32_t* err_flag,
+                              float* cam, float* z, float* z2, void* stream);
+int snb_adamw_step_rows(int32_t n_groups, float* const* params, const float* const* grads, float* const* exp_avg,
+                        float* const* exp_avg_sq, const int32_t* row_sizes, const float* lrs, float beta1, float beta2,
+                        float eps, float weight_decay, int32_t n_rows, float* steps, const uint8_t* active,
+                        const float* loss3, const float* loss_rgb2, int32_t loss_rgb2_stride, float* loss_history,
+                        int32_t history_rows, void* stream);
 size_t snb_render_shell_batch_workspace_bytes(snb_handle h, const snb_shell_batch_desc* d);
 size_t snb_render_shell_batch_scratch_bytes(snb_handle h, const snb_shell_batch_desc* d);
 int snb_render_shell_batch_fwd(snb_handle h, const snb_shell_batch_desc* d, const float* px, const float* py, const float* K,

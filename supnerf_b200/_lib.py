@@ -92,6 +92,10 @@ SIGNATURES = {
     "snb_refine_loss_batch_bwd": (c_i32, [c_f, c_f, c_f, c_f, c_i32, c_i64, c_flt, c_f, c_f, c_f, c_f, c_f]),
     "snb_refine_pose_batch_fwd": (c_i32, [c_f, c_f, c_i32, c_i32, c_f, c_i32, c_f, c_f, c_f, c_i32, c_f, c_f, c_f, c_f]),
     "snb_refine_pose_batch_bwd": (c_i32, [c_f, c_f, c_i32, c_i32, c_f, c_f, c_f, c_f]),
+    "snb_refine_pose_slots_fwd": (c_i32, [c_f, c_f, c_i32, c_i32, c_f, c_i32, c_f, c_f, c_f, c_i32, c_f, c_f, c_f, c_f, c_f, c_f]),
+    "snb_adamw_step_rows": (c_i32, [c_i32, ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(ctypes.c_void_p),
+                                    ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(c_i32), ctypes.POINTER(c_flt), c_flt, c_flt, c_flt, c_flt,
+                                    c_i32, c_f, c_f, c_f, c_f, c_i32, c_f, c_i32, c_f]),
     "snb_render_shell_batch_workspace_bytes": (c_sz, [ctypes.c_void_p, ctypes.POINTER(SnbShellBatchDesc)]),
     "snb_render_shell_batch_scratch_bytes": (c_sz, [ctypes.c_void_p, ctypes.POINTER(SnbShellBatchDesc)]),
     "snb_render_shell_batch_fwd": (c_i32, [ctypes.c_void_p, ctypes.POINTER(SnbShellBatchDesc)] + [c_f] * 13),

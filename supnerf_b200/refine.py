@@ -102,6 +102,38 @@ class FusedAdamW:
                                      self.betas[0], self.betas[1], self.eps, self.weight_decay, ptr(self.step_t), stream_ptr()), "snb_adamw_step")
 
 
+class SlotAdamW(FusedAdamW):
+    """FusedAdamW on `rows` independent rows of every parameter (one per refine slot) in ONE launch (snb_adamw_step_rows): each row has its own
+    step counter (``step_t`` (rows,)) and active byte (``active`` (rows,) uint8); an inactive row is left bit-for-bit unchanged."""
+
+    def __init__(self, groups, rows, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2):
+        super().__init__(groups, betas=betas, eps=eps, weight_decay=weight_decay)
+        dev = self.params[0].device
+        self.rows = int(rows)
+        self.step_t = torch.zeros(self.rows, device=dev, dtype=torch.float32)
+        self.active = torch.ones(self.rows, device=dev, dtype=torch.uint8)
+        self._sizes = (ctypes.c_int32 * len(self.params))(*[p.numel() // self.rows for p in self.params])
+
+    def reset_row(self, r):
+        """Zero row r's moments and step counter (stream-ordered, no host synchronisation)."""
+        for t in self.m + self.v:
+            t[r].zero_()
+        self.step_t[r].zero_()
+
+    def step(self, loss3=None, loss_rgb2=None, history=None):
+        """One update of every active row.  history (rows, T, 4) (optional): an active row r first writes [loss3[r, 0:3], loss_rgb2[r]] to
+        history[r, step_t[r]] (loss3 (rows,3) contiguous, loss_rgb2 a (rows,) view with any row stride)."""
+        lib = _lib.load()
+        n = len(self.params)
+        arr = lambda ts: (ctypes.c_void_p * n)(*[t.data_ptr() for t in ts])  # noqa: E731
+        stride = int(loss_rgb2.stride(0)) if loss_rgb2 is not None else 0
+        t_rows = int(history.shape[1]) if history is not None else 0
+        with on_device(self.params[0].device):
+            check(lib.snb_adamw_step_rows(n, arr(self.params), arr([p.grad for p in self.params]), arr(self.m), arr(self.v), self._sizes, self._lrs,
+                                          self.betas[0], self.betas[1], self.eps, self.weight_decay, self.rows, ptr(self.step_t), ptr(self.active),
+                                          ptr(loss3), ptr(loss_rgb2), stride, ptr(history), t_rows, stream_ptr()), "snb_adamw_step_rows")
+
+
 def axis_angle_to_matrix(v):
     """Rodrigues' formula, R = I + sin(t)/t [v]x + (1-cos(t))/t^2 [v]x^2 -- what pytorch3d.transforms.axis_angle_to_matrix
     evaluates (via quaternions); pytorch3d itself is not part of the reference tree (SURVEY §8c: parity unpinned there)."""
@@ -351,10 +383,12 @@ class ObjectGroup:
 
 class _PoseAndSamplesBatch(torch.autograd.Function):
     """(B,3) rot_vec, trans_vec -> cam2opt (B,3,4) + every object's shared sample vector z (B,S) [+ a second one, z2, from another jitter
-    table] in ONE launch (csrc/refine.cu: snb_refine_pose_batch_fwd); the jitter row is picked on the device by the optimiser's step counter."""
+    table] in ONE launch (csrc/refine.cu); the jitter row is picked on the device by the optimiser's step counter: one shared scalar
+    (snb_refine_pose_batch_fwd), or -- with `active` (B,) uint8 -- one counter per slot (B,) whose out-of-table rows give NaN and set
+    `err` (snb_refine_pose_slots_fwd)."""
 
     @staticmethod
-    def forward(ctx, rot_vec, trans_vec, jitter, jitter2, step_t, obj_diag, opt_cam_pose, n_samples):
+    def forward(ctx, rot_vec, trans_vec, jitter, jitter2, step_t, obj_diag, opt_cam_pose, n_samples, active=None, err=None):
         lib = _lib.load()
         require_cuda(rot_vec, trans_vec, jitter, step_t, obj_diag)
         rot_vec, trans_vec = f32c(rot_vec), f32c(trans_vec)
@@ -364,9 +398,14 @@ class _PoseAndSamplesBatch(torch.autograd.Function):
         z = torch.empty(b, s, device=dev, dtype=torch.float32)
         z2 = torch.empty(b, s, device=dev, dtype=torch.float32) if jitter2 is not None else None
         with on_device(dev):
-            check(lib.snb_refine_pose_batch_fwd(ptr(rot_vec), ptr(trans_vec), int(b), int(bool(opt_cam_pose)), ptr(obj_diag), int(n_samples),
-                                                ptr(jitter), ptr(jitter2), ptr(step_t), int(t), ptr(cam), ptr(z), ptr(z2), stream_ptr()),
-                  "snb_refine_pose_batch_fwd")
+            if active is None:
+                check(lib.snb_refine_pose_batch_fwd(ptr(rot_vec), ptr(trans_vec), int(b), int(bool(opt_cam_pose)), ptr(obj_diag), int(n_samples),
+                                                    ptr(jitter), ptr(jitter2), ptr(step_t), int(t), ptr(cam), ptr(z), ptr(z2), stream_ptr()),
+                      "snb_refine_pose_batch_fwd")
+            else:
+                check(lib.snb_refine_pose_slots_fwd(ptr(rot_vec), ptr(trans_vec), int(b), int(bool(opt_cam_pose)), ptr(obj_diag), int(n_samples),
+                                                    ptr(jitter), ptr(jitter2), ptr(step_t), int(t), ptr(active), ptr(err), ptr(cam), ptr(z),
+                                                    ptr(z2), stream_ptr()), "snb_refine_pose_slots_fwd")
         ctx.save_for_backward(rot_vec, trans_vec)
         ctx.opt_cam_pose = int(bool(opt_cam_pose))
         ctx.set_materialize_grads(False)
@@ -381,16 +420,47 @@ class _PoseAndSamplesBatch(torch.autograd.Function):
         lib = _lib.load()
         rot_vec, trans_vec = ctx.saved_tensors
         if g_cam is None:
-            return (None,) * 8
+            return (None,) * 10
         g_cam = f32c(g_cam)
         g_rot, g_trans = torch.empty_like(rot_vec), torch.empty_like(trans_vec)
         with on_device(rot_vec.device):
             check(lib.snb_refine_pose_batch_bwd(ptr(rot_vec), ptr(trans_vec), int(rot_vec.shape[0]), ctx.opt_cam_pose, ptr(g_cam), ptr(g_rot),
                                                 ptr(g_trans), stream_ptr()), "snb_refine_pose_batch_bwd")
-        return (g_rot, g_trans) + (None,) * 6
+        return (g_rot, g_trans) + (None,) * 8
 
 
-class BatchRefiner:
+class _BatchStep:
+    """The per-iteration body of BatchRefiner and SlotRefiner: ObjectRefiner.step for every object (or slot) at once.  A subclass holds the
+    stacked state (codes, pose parameters, pixels, targets, jitter tables, lidar pixels) and supplies the two stages that differ: which
+    jitter row each object reads (`_pose_and_samples`) and the optimiser update (`_update`)."""
+
+    def _params(self):
+        return (self.shapecode, self.texturecode, self.rot_vec, self.trans_vec)
+
+    def step(self):
+        """One iteration of every object (no host synchronisation anywhere)."""
+        if self.shapecode.grad is not None:
+            self.opt.zero_grad()
+        out = self._pose_and_samples()
+        cam, z = out[0], out[1]
+        prec = self.model.precision or models.get_default_precision()
+        h, w = self.model._handle(self.device), self.model._weights()
+        rgb, _dep, acc = ops.render_shell_batch(h, prec, self.n_samples, self.swap, self.px, self.py, self.K, cam, z, self.obj_diag,
+                                                self.shapecode, self.texturecode, w)
+        loss, parts = losses.refine_loss_batch(rgb, acc, self.rgb_tgt, self.occ, self.coef)
+        torch.autograd.backward(loss, self._ones)
+        with torch.no_grad():       # the per-iteration evaluation (optimizer_nuscenes.py:740-769), before the parameter update as there
+            self.loss_rgb2 = losses.refine_loss_batch(rgb.detach(), acc.detach(), self.rgb_tgt, self.occ_pos, 0.0)[1][:, 1]
+            if self.lidar is not None:
+                _, dep2, _ = ops.render_shell_batch(h, prec, self.n_samples, self.swap, self.lidar[0], self.lidar[1], self.K, cam.detach(),
+                                                    out[2], self.obj_diag, self.shapecode.detach(), self.texturecode.detach(), w)
+                self.depth_pred = dep2           # (B, width): object b's lidar depths are depth_pred[b, :n_lidar[b]]
+        self.loss = parts           # (B,3) = [loss, loss_rgb, loss_occ] per object
+        self._update()
+        return self.loss
+
+
+class BatchRefiner(_BatchStep):
     """The refine loops of B INDEPENDENT objects (one GPU's share of config C3) as ONE launch set per iteration: every stage of
     ObjectRefiner.step -- pose map + sample vectors, the utils.py-stack render, the losses, their backward, the per-iteration
     evaluation (loss_rgb2, lidar-pixel depths) and the AdamW update -- runs once over all objects (ops.render_shell_batch,
@@ -459,31 +529,12 @@ class BatchRefiner:
         self.it = 0              # host-side count of issued iterations (the device-side row index is the optimiser's step counter)
         self.graph = None
 
-    def _params(self):
-        return (self.shapecode, self.texturecode, self.rot_vec, self.trans_vec)
+    def _pose_and_samples(self):
+        return _PoseAndSamplesBatch.apply(self.rot_vec, self.trans_vec, self.jitter, self.jitter_lidar, self.opt.step_t, self.obj_diag,
+                                          self.opt_cam_pose, self.n_samples)
 
-    def step(self):
-        """One iteration of every object (no host synchronisation anywhere)."""
-        if self.shapecode.grad is not None:
-            self.opt.zero_grad()
-        out = _PoseAndSamplesBatch.apply(self.rot_vec, self.trans_vec, self.jitter, self.jitter_lidar, self.opt.step_t, self.obj_diag,
-                                         self.opt_cam_pose, self.n_samples)
-        cam, z = out[0], out[1]
-        prec = self.model.precision or models.get_default_precision()
-        h, w = self.model._handle(self.device), self.model._weights()
-        rgb, _dep, acc = ops.render_shell_batch(h, prec, self.n_samples, self.swap, self.px, self.py, self.K, cam, z, self.obj_diag,
-                                                self.shapecode, self.texturecode, w)
-        loss, parts = losses.refine_loss_batch(rgb, acc, self.rgb_tgt, self.occ, self.coef)
-        torch.autograd.backward(loss, self._ones)
-        with torch.no_grad():       # the per-iteration evaluation (optimizer_nuscenes.py:740-769), before the parameter update as there
-            self.loss_rgb2 = losses.refine_loss_batch(rgb.detach(), acc.detach(), self.rgb_tgt, self.occ_pos, 0.0)[1][:, 1]
-            if self.lidar is not None:
-                _, dep2, _ = ops.render_shell_batch(h, prec, self.n_samples, self.swap, self.lidar[0], self.lidar[1], self.K, cam.detach(),
-                                                    out[2], self.obj_diag, self.shapecode.detach(), self.texturecode.detach(), w)
-                self.depth_pred = dep2           # (B, width): object b's lidar depths are depth_pred[b, :n_lidar[b]]
+    def _update(self):
         self.opt.step()
-        self.loss = parts           # (B,3) = [loss, loss_rgb, loss_occ] per object
-        return self.loss
 
     def capture(self, warmup=3):
         """Warm up on a side stream (allocator, weight packing), undo the warm-up updates, then capture one iteration."""
@@ -532,3 +583,227 @@ class BatchRefiner:
                 r.loss = self.loss[b]
                 r.loss_rgb2 = self.loss_rgb2[b]
         return self.refiners
+
+
+class SlotRefiner(_BatchStep):
+    """A stream of INDEPENDENT objects refined through C fixed slots (the reference's test-time refinement goes through the evaluation split
+    one object at a time: optimize_objs_w_pose_unified, optimizer_nuscenes.py:684-769).  Each slot holds one object's refine state; one
+    iteration of all C slots is BatchRefiner's launch set, captured ONCE as a CUDA graph.  Between replays the host ``admit``s an
+    ObjectRefiner into a free slot with its own iteration budget, and ``run`` retires every object whose budget is used up, copying its
+    results back into its ObjectRefiner -- all stream-ordered, without a host synchronisation.  The host knows every slot's remaining budget
+    without reading the device: each replay advances every active slot by exactly one iteration.
+
+    Every slot has its own AdamW step counter (SlotAdamW), which also picks its jitter row, and an active byte.  A free slot keeps running
+    on finite placeholder inputs (a fixed synthetic object at first, its last object's inputs with zero loss weights after a retirement):
+    it takes no AdamW step, writes no loss history and reports nothing, but its render is paid.  ``max_lidar`` is the per-slot capacity of
+    lidar pixels evaluated every iteration (0 = no lidar evaluation)."""
+
+    def __init__(self, model, device, slots=16, n_samples=64, im_sz=32, max_iters=100, max_lidar=0, lr_shape=0.02, lr_texture=0.02,
+                 lr_pose=0.01, loss_occ_coef=0.1, shapenet_obj_cood=True, opt_cam_pose=False):
+        if not isinstance(model, models._DecoderBase):
+            raise TypeError("SlotRefiner needs a supnerf_b200 decoder")
+        self.model, self.device = model, torch.device(device)
+        if self.device.type != "cuda":
+            raise RuntimeError("supnerf_b200 has no CPU path")
+        if int(slots) < 1 or int(max_iters) < 1 or int(max_lidar) < 0:
+            raise ValueError("SlotRefiner: slots >= 1, max_iters >= 1, max_lidar >= 0")
+        dev = self.device
+        c, s, n = int(slots), int(n_samples), int(im_sz) ** 2
+        self.slots, self.n_samples, self.im_sz, self.max_iters = c, s, int(im_sz), int(max_iters)
+        self.coef, self.swap, self.opt_cam_pose = float(loss_occ_coef), bool(shapenet_obj_cood), bool(opt_cam_pose)
+        d = model._latent_dim
+        # placeholder object (finite everywhere, zero loss weights): camera 2.5 units from the origin looking down +z, unit diagonal
+        px, py = U._pixel_grid_on(dev, [0, 0, int(im_sz), int(im_sz)], [int(im_sz), int(im_sz)])
+        self.px = px.reshape(1, -1).repeat(c, 1).contiguous()
+        self.py = py.reshape(1, -1).repeat(c, 1).contiguous()
+        f = float(im_sz)
+        self.K = torch.tensor([[f, 0.0, f / 2], [0.0, f, f / 2], [0.0, 0.0, 1.0]], device=dev).repeat(c, 1, 1).contiguous()
+        self.rgb_tgt = torch.zeros(c, n, 3, device=dev)
+        self.occ = torch.zeros(c, n, device=dev)
+        self.occ_pos = torch.zeros(c, n, device=dev)
+        self.obj_diag = torch.ones(c, device=dev)
+        self.shapecode = torch.zeros(c, d, device=dev).requires_grad_()
+        self.texturecode = torch.zeros(c, d, device=dev).requires_grad_()
+        self.rot_vec = torch.zeros(c, 3, device=dev).requires_grad_()
+        self.trans_vec = torch.tensor([0.0, 0.0, 2.5], device=dev).repeat(c, 1).contiguous().requires_grad_()
+        self.opt = SlotAdamW([{"params": self.shapecode, "lr": lr_shape}, {"params": self.texturecode, "lr": lr_texture},
+                              {"params": self.rot_vec, "lr": lr_pose}, {"params": self.trans_vec, "lr": lr_pose}], rows=c)
+        self.opt.active.zero_()
+        self.jitter = torch.zeros(c, self.max_iters, s, device=dev)
+        self.lidar, self.jitter_lidar, self.width = None, None, 0
+        if int(max_lidar) > 0:   # whole 256-row decoder super tiles per slot, as BatchRefiner pads them
+            q = 256 // math.gcd(256, s)
+            self.width = -(-int(max_lidar) // q) * q
+            self.lidar = (self.px[:, :1].repeat(1, self.width).contiguous(), self.py[:, :1].repeat(1, self.width).contiguous())
+            self.jitter_lidar = torch.zeros(c, self.max_iters, s, device=dev)
+        self.history = torch.zeros(c, self.max_iters, 4, device=dev)   # [loss, loss_rgb, loss_occ, loss_rgb2] per slot and iteration
+        self.err = torch.zeros(1, device=dev, dtype=torch.int32)       # set by the pose kernel if an active slot's counter leaves its table
+        self._ones = torch.ones(c, device=dev)
+        self.loss = torch.zeros(c, 3, device=dev)
+        self.loss_rgb2 = torch.zeros(c, device=dev)
+        self.depth_pred = None
+        self.owner = [None] * c          # the ObjectRefiner in each slot (None = free)
+        self.budget = [0] * c            # its iteration budget
+        self.remaining = [0] * c         # iterations it still has to run
+        self.n_lidar = [0] * c
+        self.replays = 0                 # host-side counts: slot-iterations issued, and those of occupied slots
+        self.busy_slot_iters = 0
+        self.graph = None
+
+    def _pose_and_samples(self):
+        return _PoseAndSamplesBatch.apply(self.rot_vec, self.trans_vec, self.jitter, self.jitter_lidar, self.opt.step_t, self.obj_diag,
+                                          self.opt_cam_pose, self.n_samples, self.opt.active, self.err)
+
+    def _update(self):
+        self.opt.step(self.loss, self.loss_rgb2, self.history)
+
+    def capture(self, warmup=3):
+        """Warm up on a side stream (allocator, weight packing) with every slot free -- nothing is updated, so nothing needs restoring -- then
+        capture one iteration of all slots.  Done once, before the first admission."""
+        if any(o is not None for o in self.owner):
+            raise RuntimeError("SlotRefiner.capture: capture before admitting objects")
+        s = torch.cuda.Stream(device=self.device)
+        s.wait_stream(torch.cuda.current_stream(self.device))
+        with torch.cuda.stream(s):
+            for _ in range(warmup):
+                self.step()
+        torch.cuda.current_stream(self.device).wait_stream(s)
+        self.graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(self.graph):
+            self.step()
+        return self
+
+    def free_slots(self):
+        return [b for b, o in enumerate(self.owner) if o is None]
+
+    def busy(self):
+        return any(o is not None for o in self.owner)
+
+    def admit(self, r, iters):
+        """Put ObjectRefiner `r` into a free slot with a budget of `iters` iterations (stream-ordered copies, no host synchronisation).
+        -> the slot index.  ValueError if its settings differ from this refiner's, there is no free slot, `iters` exceeds max_iters or the
+        object's jitter rows, or it has more lidar pixels than the slot capacity."""
+        iters = int(iters)
+        lrs = (float(self.opt.lrs[0]), float(self.opt.lrs[1]), float(self.opt.lrs[2]), float(self.opt.lrs[2]))
+        if not (r.model is self.model and r.device == self.device and r.fused and (r.n_samples, r.im_sz, r.coef, r.swap, r.opt_cam_pose)
+                == (self.n_samples, self.im_sz, self.coef, self.swap, self.opt_cam_pose) and tuple(r.opt.lrs) == lrs
+                and (tuple(r.opt.betas), r.opt.eps, r.opt.weight_decay) == (tuple(self.opt.betas), self.opt.eps, self.opt.weight_decay)):
+            raise ValueError("SlotRefiner.admit: the object must share the decoder, device, n_samples, crop size, loss and optimiser settings "
+                             "(and be a fused ObjectRefiner)")
+        if not 1 <= iters <= min(self.max_iters, r.jitter.shape[0]):
+            raise ValueError("SlotRefiner.admit: iters must be in 1 .. min(max_iters, the object's jitter rows)")
+        n_lidar = r.n_lidar if r.lidar is not None else 0
+        if n_lidar > self.width:
+            raise ValueError("SlotRefiner.admit: %d lidar pixels exceed the slot capacity (%d)" % (n_lidar, self.width))
+        free = self.free_slots()
+        if not free:
+            raise ValueError("SlotRefiner.admit: no free slot")
+        b = free[0]
+        k = min(self.max_iters, r.jitter.shape[0])
+        with torch.no_grad():
+            self.px[b].copy_(r.px.reshape(-1))
+            self.py[b].copy_(r.py.reshape(-1))
+            self.K[b].copy_(r.K)
+            self.rgb_tgt[b].copy_(r.rgb_tgt)
+            self.occ[b].copy_(r.occ.reshape(-1))
+            self.occ_pos[b].copy_(r.occ_pos.reshape(-1))
+            self.obj_diag[b].fill_(float(r.obj_diag))
+            self.shapecode[b].copy_(r.shapecode.detach().reshape(-1))
+            self.texturecode[b].copy_(r.texturecode.detach().reshape(-1))
+            self.rot_vec[b].copy_(r.rot_vec.detach())
+            self.trans_vec[b].copy_(r.trans_vec.detach())
+            self.jitter[b, :k].copy_(r.jitter[:k])
+            if self.lidar is not None:
+                if n_lidar:
+                    x, y = r.lidar[0][:n_lidar], r.lidar[1][:n_lidar]
+                    self.jitter_lidar[b, :k].copy_(r.jitter_lidar[:k])
+                else:   # no lidar pixels: a dummy pixel is rendered and nothing reported, as in BatchRefiner
+                    x, y = r.px.reshape(-1)[:1], r.py.reshape(-1)[:1]
+                    self.jitter_lidar[b].zero_()
+                self.lidar[0][b, :x.numel()].copy_(x)
+                self.lidar[0][b, x.numel():].copy_(x[-1:].expand(self.width - x.numel()))
+                self.lidar[1][b, :y.numel()].copy_(y)
+                self.lidar[1][b, y.numel():].copy_(y[-1:].expand(self.width - y.numel()))
+            self.opt.reset_row(b)
+            self.history[b].zero_()
+            self.opt.active[b].fill_(1)
+        self.owner[b], self.budget[b], self.remaining[b], self.n_lidar[b] = r, iters, iters, n_lidar
+        return b
+
+    def _retire(self, b):
+        """Copy slot b's results into its ObjectRefiner (as BatchRefiner.write_back does, plus loss_history (iters, 4)) and free the slot."""
+        r, n = self.owner[b], self.n_lidar[b]
+        with torch.no_grad():
+            r.shapecode.copy_(self.shapecode[b].reshape(r.shapecode.shape))
+            r.texturecode.copy_(self.texturecode[b].reshape(r.texturecode.shape))
+            r.rot_vec.copy_(self.rot_vec[b])
+            r.trans_vec.copy_(self.trans_vec[b])
+            r.loss = self.loss[b].clone()          # copies: the slot's buffers are rewritten by the next replay
+            r.loss_rgb2 = self.loss_rgb2[b].clone()
+            if n:
+                r.depth_pred = self.depth_pred[b, :n].clone()
+            r.loss_history = self.history[b, :self.budget[b]].clone()
+            self.opt.active[b].fill_(0)
+            # zero loss weights: the idle slot's upstream gradients are exactly zero, so the batched backward skips its decoder tiles
+            self.occ[b].zero_()
+            self.occ_pos[b].zero_()
+        self.owner[b], self.remaining[b] = None, 0
+
+    def run(self, iters):
+        """`iters` iterations of every slot (graph replays if captured); an object whose budget is used up is retired right after its last
+        iteration.  -> (C,3) last [loss, loss_rgb, loss_occ] per slot (device tensor)."""
+        for _ in range(int(iters)):
+            if self.graph is not None:
+                self.graph.replay()
+            else:
+                self.step()
+            self.replays += 1
+            for b in range(self.slots):
+                if self.owner[b] is not None:
+                    self.busy_slot_iters += 1
+                    self.remaining[b] -= 1
+                    if self.remaining[b] == 0:
+                        self._retire(b)
+        return self.loss
+
+    def stream(self, refiners, iters):
+        """Refine every ObjectRefiner of `refiners` (iters: one budget for all, or one per object), admitting the next one as soon as a slot
+        is free, so every slot stays busy while objects remain.  Ends with a synchronisation (raises if the kernels' error flag is set).
+        Returns the refiners in input order, their results written back (codes, pose parameters, last losses, lidar depths, loss_history)."""
+        refiners = list(refiners)
+        budgets = [int(i) for i in iters] if hasattr(iters, "__len__") else [int(iters)] * len(refiners)
+        if len(budgets) != len(refiners):
+            raise ValueError("SlotRefiner.stream: one budget per refiner")
+        todo = list(zip(refiners, budgets))[::-1]
+        while todo or self.busy():
+            for _ in self.free_slots():
+                if todo:
+                    self.admit(*todo.pop())
+            self.run(min(self.remaining[b] for b in range(self.slots) if self.owner[b] is not None))
+        self.synchronize()
+        return refiners
+
+    def idle_share(self):
+        """Share of the slot-iterations issued so far that ran on a free slot."""
+        total = self.replays * self.slots
+        return 1.0 - self.busy_slot_iters / total if total else 0.0
+
+    def synchronize(self):
+        """Wait for the device, then raise if an active slot read outside its jitter table (the kernels' error flag)."""
+        torch.cuda.current_stream(self.device).synchronize()
+        if int(self.err.item()):
+            raise RuntimeError("SlotRefiner: an active slot's step counter left its jitter table (its sample vectors are NaN)")
+
+
+def refine_stream(refiners, iters, slots=16):
+    """Refine ObjectRefiners through one SlotRefiner of min(slots, len(refiners)) slots with their settings (SlotRefiner.stream).
+    iters: one budget for all, or one per object.  Returns the refiners in input order, results written back."""
+    refiners = list(refiners)
+    if not refiners:
+        return []
+    budgets = [int(i) for i in iters] if hasattr(iters, "__len__") else [int(iters)] * len(refiners)
+    r0, lrs = refiners[0], refiners[0].opt.lrs
+    sr = SlotRefiner(r0.model, r0.device, slots=min(int(slots), len(refiners)), n_samples=r0.n_samples, im_sz=r0.im_sz, max_iters=max(budgets),
+                     max_lidar=max(r.n_lidar if r.lidar is not None else 0 for r in refiners), lr_shape=lrs[0], lr_texture=lrs[1],
+                     lr_pose=lrs[2], loss_occ_coef=r0.coef, shapenet_obj_cood=r0.swap, opt_cam_pose=r0.opt_cam_pose)
+    return sr.capture().stream(refiners, budgets)
