@@ -18,7 +18,7 @@
 extern "C" {
 #endif
 
-#define SNB_ABI_VERSION 1
+#define SNB_ABI_VERSION 2
 
 /* flags for the compositing kernels */
 #define SNB_WHITE_BKGD 1 /* renderer.py:60-63 */
@@ -307,28 +307,38 @@ int snb_refine_loss_bwd(const float* rgb, const float* acc, const float* tgt, co
 int snb_merge_sort_samples(const float* z, const float* sigma, const float* rgb, int64_t n_rays, int32_t n_per_ray,
                            float* z_sort, float* sigma_sort, float* rgb_sort, int64_t* z_args, void* stream);
 
-/* ---- refine-iteration glue around the render (SURVEY 8(f) rank 1) ----------------------------------------------------
- * snb_refine_pose_fwd/bwd: optimizer_nuscenes.py:684-699 -- rot_vec (3, axis-angle; Rodrigues = what
- * pytorch3d.transforms.axis_angle_to_matrix evaluates), trans_vec (3) -> cam2opt (3,4) = [R | t] (opt_cam_pose != 0) or
- * [R^T | -R^T t] (opt_cam_pose == 0, every shipped config), and -- if z != NULL -- the shared sample vector z (S) of
- * utils.sample_from_rays (utils.py:154-167) with near/far = ||cam2opt[:,3]|| -/+ obj_diag/2 (utils.py:468-469, detached) and
- * jitter (S) = the torch.rand(n_samples) draw.  Backward: g_cam (12) -> g_rot (3), g_trans (3).
- * snb_adamw_step: torch.optim.AdamW's update (optimizer_nuscenes.py:757-769, groups of :1762-1769) on up to 8 tensors with
- * their own learning rates; `step` is a device float holding the number of steps taken (incremented). */
-int snb_refine_pose_fwd(const float* rot_vec, const float* trans_vec, int32_t opt_cam_pose, float obj_diag, int32_t n_samples,
-                        const float* jitter, float* cam, float* z, void* stream);
-int snb_refine_pose_bwd(const float* rot_vec, const float* trans_vec, int32_t opt_cam_pose, const float* g_cam, float* g_rot,
-                        float* g_trans, void* stream);
-int snb_adamw_step(int32_t n_groups, float* const* params, const float* const* grads, float* const* exp_avg,
-                   float* const* exp_avg_sq, const int32_t* sizes, const float* lrs, float beta1, float beta2, float eps,
-                   float weight_decay, float* step, void* stream);
+/* ---- refine-iteration glue around the render (SURVEY 8(f) rank 1), for B objects side by side --------------------------
+ * (one object is B = 1; one GPU's share of config C3 -- 32 objects over 8 GPUs -- or C fixed slots of a stream of objects)
+ * snb_refine_pose_slots_fwd: optimizer_nuscenes.py:684-699 -- rot_vec (B,3, axis-angle; Rodrigues = what
+ * pytorch3d.transforms.axis_angle_to_matrix evaluates), trans_vec (B,3) -> cam2opt (B,3,4) = [R | t] (opt_cam_pose != 0) or
+ * [R^T | -R^T t] (opt_cam_pose == 0, every shipped config), and every object's shared sample vector z (B,S) of
+ * utils.sample_from_rays (utils.py:154-167) with near/far = ||cam2opt[:,3]|| -/+ obj_diag/2 (obj_diag (B), device;
+ * utils.py:468-469, detached).  Object b's jitter is row int(step_counters[b]) of its table (B, table_rows, S) -- the
+ * torch.rand(n_samples) draw of that iteration, picked by the object's AdamW step counter of snb_adamw_step_rows, so a
+ * captured iteration needs neither an index_select nor a counter launch.  z2 / jitter2: a second sample vector from the same
+ * pose and another draw (the lidar-pixel evaluation of optimizer_nuscenes.py:759-769); both NULL = not wanted.  active (B
+ * bytes): an active object whose counter lies outside [0, table_rows) gets NaN in its z / z2 and sets *err_flag to 1 (a
+ * device int32, NULL = not reported); an inactive one reads a row inside the table and reports nothing.
+ * snb_refine_pose_batch_bwd: g_cam (B,3,4) -> g_rot, g_trans (B,3).
+ * snb_adamw_step_rows: torch.optim.AdamW's update (optimizer_nuscenes.py:757-769, groups of :1762-1769) on n_rows independent
+ * rows of up to 8 tensors with their own learning rates (row r of tensor i: row_sizes[i] elements at r * row_sizes[i]).
+ * steps (n_rows device floats): each row's step count -- its bias corrections -- incremented by the call; active (n_rows
+ * bytes): an inactive row's parameters, moments and count stay bit-for-bit unchanged.  loss_history (NULL = none):
+ * (n_rows, history_rows, 4); an active row r with 0 <= steps[r] < history_rows first writes {loss3[3r .. 3r+2],
+ * loss_rgb2[r * loss_rgb2_stride]} to row steps[r]. */
+int snb_refine_pose_slots_fwd(const float* rot_vec, const float* trans_vec, int32_t n_slots, int32_t opt_cam_pose,
+                              const float* obj_diag, int32_t n_samples, const float* jitter, const float* jitter2,
+                              const float* step_counters, int32_t table_rows, const uint8_t* active, int32_t* err_flag,
+                              float* cam, float* z, float* z2, void* stream);
+int snb_refine_pose_batch_bwd(const float* rot_vec, const float* trans_vec, int32_t n_objs, int32_t opt_cam_pose,
+                              const float* g_cam, float* g_rot, float* g_trans, void* stream);
+int snb_adamw_step_rows(int32_t n_groups, float* const* params, const float* const* grads, float* const* exp_avg,
+                        float* const* exp_avg_sq, const int32_t* row_sizes, const float* lrs, float beta1, float beta2,
+                        float eps, float weight_decay, int32_t n_rows, float* steps, const uint8_t* active,
+                        const float* loss3, const float* loss_rgb2, int32_t loss_rgb2_stride, float* loss_history,
+                        int32_t history_rows, void* stream);
 
-/* ---- the same glue for B objects side by side (one GPU's share of config C3: 32 objects over 8 GPUs) ----------------
- * snb_refine_pose_batch_fwd/bwd: rot_vec, trans_vec (B,3) -> cam (B,3,4) and, if z != NULL, every object's shared sample
- * vector z (B,S) from obj_diag (B, device).  jitter: (B,S), or -- step_counter != NULL -- a table (B, table_rows, S) whose row
- * int(*step_counter) is used (the AdamW step counter of snb_adamw_step: a captured iteration then needs neither an
- * index_select nor a counter launch).  z2 / jitter2: a second sample vector from the same pose and another draw (the
- * lidar-pixel evaluation of optimizer_nuscenes.py:759-769); both NULL = not wanted.
+/* ---- the render for B objects side by side ---------------------------------------------------------------------------
  * snb_render_shell_batch_fwd/bwd: utils.render_rays_v2 (utils.py:435-502) for B objects in one launch set: px, py (B,N); K
  * (B,3,3); c2w (B,3,4); z (B,S); obj_diag (B); latents (B,D) -> rgb (B,N,3), depth, acc (B,N).  Frozen weights; bf16 needs
  * N * S to be a multiple of 128.  Backward: g_rgb (B,N,3), g_depth, g_acc (B,N) -> g_c2w (B,3,4; NULL = not wanted),
@@ -342,30 +352,6 @@ typedef struct snb_shell_batch_desc {
   int32_t shapenet_swap;
   int32_t reserved;
 } snb_shell_batch_desc;
-int snb_refine_pose_batch_fwd(const float* rot_vec, const float* trans_vec, int32_t n_objs, int32_t opt_cam_pose,
-                              const float* obj_diag, int32_t n_samples, const float* jitter, const float* jitter2,
-                              const float* step_counter, int32_t table_rows, float* cam, float* z, float* z2, void* stream);
-int snb_refine_pose_batch_bwd(const float* rot_vec, const float* trans_vec, int32_t n_objs, int32_t opt_cam_pose,
-                              const float* g_cam, float* g_rot, float* g_trans, void* stream);
-/* ---- the same glue for a stream of objects through C fixed slots (refine.SlotRefiner) ---------------------------------
- * snb_refine_pose_slots_fwd: snb_refine_pose_batch_fwd with one step counter per slot: slot b reads row int(step_counters[b])
- * of its jitter table(s) (C, table_rows, S).  active (C bytes, NULL = all active): an active slot whose counter lies outside
- * [0, table_rows) gets NaN in its z / z2 and sets *err_flag to 1 (a device int32, NULL = not reported); an inactive slot
- * reads a row inside the table and reports nothing.  The backward is snb_refine_pose_batch_bwd.
- * snb_adamw_step_rows: snb_adamw_step on n_rows independent rows of every tensor (row r of tensor i: row_sizes[i] elements
- * at r * row_sizes[i]).  steps (n_rows device floats): each row's step count -- its bias corrections -- incremented by the
- * call; active (n_rows bytes, NULL = all active): an inactive row's parameters, moments and count stay bit-for-bit unchanged.
- * snb_adamw_step is the one-row case.  loss_history (NULL = none): (n_rows, history_rows, 4); an active row r with
- * 0 <= steps[r] < history_rows first writes {loss3[3r .. 3r+2], loss_rgb2[r * loss_rgb2_stride]} to row steps[r]. */
-int snb_refine_pose_slots_fwd(const float* rot_vec, const float* trans_vec, int32_t n_slots, int32_t opt_cam_pose,
-                              const float* obj_diag, int32_t n_samples, const float* jitter, const float* jitter2,
-                              const float* step_counters, int32_t table_rows, const uint8_t* active, int32_t* err_flag,
-                              float* cam, float* z, float* z2, void* stream);
-int snb_adamw_step_rows(int32_t n_groups, float* const* params, const float* const* grads, float* const* exp_avg,
-                        float* const* exp_avg_sq, const int32_t* row_sizes, const float* lrs, float beta1, float beta2,
-                        float eps, float weight_decay, int32_t n_rows, float* steps, const uint8_t* active,
-                        const float* loss3, const float* loss_rgb2, int32_t loss_rgb2_stride, float* loss_history,
-                        int32_t history_rows, void* stream);
 size_t snb_render_shell_batch_workspace_bytes(snb_handle h, const snb_shell_batch_desc* d);
 size_t snb_render_shell_batch_scratch_bytes(snb_handle h, const snb_shell_batch_desc* d);
 int snb_render_shell_batch_fwd(snb_handle h, const snb_shell_batch_desc* d, const float* px, const float* py, const float* K,

@@ -72,11 +72,6 @@ SIGNATURES = {
     "snb_refine_loss_fwd": (c_i32, [c_f, c_f, c_f, c_f, c_i64, c_flt, c_f, c_f, c_f, c_f]),
     "snb_refine_loss_bwd": (c_i32, [c_f, c_f, c_f, c_f, c_i64, c_flt, c_f, c_f, c_f, c_f, c_f]),
     "snb_merge_sort_samples": (c_i32, [c_f, c_f, c_f, c_i64, c_i32, c_f, c_f, c_f, c_f, c_f]),
-    "snb_refine_pose_fwd": (c_i32, [c_f, c_f, c_i32, c_flt, c_i32, c_f, c_f, c_f, c_f]),
-    "snb_refine_pose_bwd": (c_i32, [c_f, c_f, c_i32, c_f, c_f, c_f, c_f]),
-    "snb_adamw_step": (c_i32, [c_i32, ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(ctypes.c_void_p),
-                               ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(c_i32), ctypes.POINTER(c_flt), c_flt, c_flt, c_flt, c_flt,
-                               c_f, c_f]),
     "snb_render_workspace_bytes": (c_sz, [ctypes.c_void_p, ctypes.POINTER(SnbRenderDesc)]),
     "snb_render_bwd_scratch_bytes": (c_sz, [ctypes.c_void_p, ctypes.POINTER(SnbRenderDesc)]),
     "snb_render_fwd": (c_i32, [ctypes.c_void_p, ctypes.POINTER(SnbRenderDesc)] + [c_f] * 14),
@@ -90,7 +85,6 @@ SIGNATURES = {
     "snb_refine_loss_batch_scratch_bytes": (c_sz, [c_i32]),
     "snb_refine_loss_batch_fwd": (c_i32, [c_f, c_f, c_f, c_f, c_i32, c_i64, c_flt, c_f, c_f, c_f]),
     "snb_refine_loss_batch_bwd": (c_i32, [c_f, c_f, c_f, c_f, c_i32, c_i64, c_flt, c_f, c_f, c_f, c_f, c_f]),
-    "snb_refine_pose_batch_fwd": (c_i32, [c_f, c_f, c_i32, c_i32, c_f, c_i32, c_f, c_f, c_f, c_i32, c_f, c_f, c_f, c_f]),
     "snb_refine_pose_batch_bwd": (c_i32, [c_f, c_f, c_i32, c_i32, c_f, c_f, c_f, c_f]),
     "snb_refine_pose_slots_fwd": (c_i32, [c_f, c_f, c_i32, c_i32, c_f, c_i32, c_f, c_f, c_f, c_i32, c_f, c_f, c_f, c_f, c_f, c_f]),
     "snb_adamw_step_rows": (c_i32, [c_i32, ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(ctypes.c_void_p),
@@ -119,7 +113,7 @@ def load():
         fn = getattr(lib, name)  # AttributeError if the .so does not export a declared symbol
         fn.restype = res
         fn.argtypes = args
-    if lib.snb_abi_version() != 1:
+    if lib.snb_abi_version() != 2:
         raise ImportError("libsupnerf_b200.so ABI version mismatch; rebuild")
     _lib = lib
     return lib

@@ -4,9 +4,8 @@
 //           evaluates), t2opt = trans_vec; with opt_cam_pose false (every shipped config) cam2opt = [R^T | -R^T t] (:695-697).
 //           The same launch builds the shared sample vector of utils.sample_from_rays (utils.py:154-167) from the DETACHED
 //           translation norm (utils.py:468-469), so nothing in an iteration needs the host.
-//   AdamW : torch.optim.AdamW's update (decoupled weight decay, bias correction) on up to 8 small tensors with their own
-//           learning rates, state and step counter on the device -- or on R independent rows of them (one per refine slot), each
-//           row with its own step counter and an active byte.
+//   AdamW : torch.optim.AdamW's update (decoupled weight decay, bias correction) on R independent rows (one per object) of up to 8
+//           small tensors with their own learning rates, state on the device, each row with its own step counter and active byte.
 // Scalar work: one thread does the 3x3 algebra in double, S threads the sample vector, one block per row the optimiser.
 #include "common.cuh"
 #include "../../include/supnerf_b200.h"
@@ -47,19 +46,17 @@ __device__ __forceinline__ void rodrigues(const double v[3], const Rod& r, doubl
   for (int i = 0; i < 9; ++i) R[i] = (i % 4 == 0 ? 1.0 : 0.0) + r.a * K[i] + r.b * K2[i];
 }
 
-// One block per object.  obj_diag: a host scalar (obj_diag_dev null) or one value per object on the device.  The sample-vector jitter is
-// either the vector itself (it == nullptr: jitter (B,S)) or row int(it[b * it_stride]) of a per-object table (B, T, S) -- `it` being the
-// optimiser's device-side step counter (it_stride 0: one counter shared by every object, 1: one per object), so a captured iteration needs
-// neither an index_select nor a counter-increment launch.  z2 / jitter2: a second sample vector from the same pose and another draw (the
-// per-iteration lidar-pixel evaluation, optimizer_nuscenes.py:759-769).
-// Every table read is guarded: an active object (active null = all active) whose counter lies outside [0, T) gets NaN in z / z2 and sets
-// *err (if given); an inactive one reads row 0 instead and reports nothing (its render runs on placeholder inputs and is ignored).
+// One block per object.  Object b reads row int(it[b]) of its jitter table (B, T, S) -- `it` being its optimiser's device-side step
+// counter, so a captured iteration needs neither an index_select nor a counter-increment launch.  z2 / jitter2 (optional): a second
+// sample vector from the same pose and another draw (the per-iteration lidar-pixel evaluation, optimizer_nuscenes.py:759-769).
+// Every table read is guarded: an active object whose counter lies outside [0, T) gets NaN in z / z2 and sets *err (if given); an
+// inactive one reads row 0 instead and reports nothing (its render runs on placeholder inputs and is ignored).
 __global__ void __launch_bounds__(1024) refine_pose_fwd_kernel(const float* __restrict__ rot_vec, const float* __restrict__ trans_vec,
-                                                              int opt_cam_pose, float obj_diag_host, const float* __restrict__ obj_diag_dev,
-                                                              int S, const float* __restrict__ jitter, const float* __restrict__ jitter2,
-                                                              const float* __restrict__ it, int it_stride, int T,
-                                                              const uint8_t* __restrict__ active, int* __restrict__ err,
-                                                              float* __restrict__ cam, float* __restrict__ z, float* __restrict__ z2) {
+                                                              int opt_cam_pose, const float* __restrict__ obj_diag, int S,
+                                                              const float* __restrict__ jitter, const float* __restrict__ jitter2,
+                                                              const float* __restrict__ it, int T, const uint8_t* __restrict__ active,
+                                                              int* __restrict__ err, float* __restrict__ cam, float* __restrict__ z,
+                                                              float* __restrict__ z2) {
   __shared__ double tn;
   const int b = blockIdx.x;
   rot_vec += 3 * b; trans_vec += 3 * b; cam += 12 * b;
@@ -80,27 +77,20 @@ __global__ void __launch_bounds__(1024) refine_pose_fwd_kernel(const float* __re
     tn = sqrt((double)c[3] * c[3] + (double)c[7] * c[7] + (double)c[11] * c[11]);   // norm of the fp32 translation, in double
   }
   __syncthreads();
-  if (z != nullptr) {
-    // utils.py:468-469 + :154-167: near/far python floats (double), torch.linspace's fp32 formula, jitter scaled by (far-near)/(2S)
-    const float obj_diag = obj_diag_dev ? obj_diag_dev[b] : obj_diag_host;
-    const double half = (double)obj_diag / 2.0, near = tn - half, far = tn + half, dist = (far - near) / (2.0 * S);
-    const float start = (float)(near + dist), end = (float)(far - dist);
-    const float step = S > 1 ? (end - start) / (float)(S - 1) : 0.f;
-    const float scale = (float)((far - near) / (2.0 * S));
-    int64_t row = b;
-    bool bad = false;
-    if (it) {
-      const float c = it[(int64_t)b * it_stride];
-      const bool in_table = c >= 0.f && c < (float)T;    // false for NaN too
-      bad = !in_table && (active == nullptr || active[b] != 0);
-      row = (int64_t)b * T + (in_table ? (int64_t)c : 0);
-      if (bad && err != nullptr && threadIdx.x == 0) *err = 1;
-    }
-    for (int i = threadIdx.x; i < S; i += blockDim.x) {
-      const float lin = i < S / 2 ? __fadd_rn(start, __fmul_rn(step, (float)i)) : __fsub_rn(end, __fmul_rn(step, (float)(S - 1 - i)));
-      z[(int64_t)b * S + i] = bad ? __int_as_float(0x7fffffff) : __fadd_rn(lin, __fmul_rn(jitter[row * S + i], scale));
-      if (z2 != nullptr) z2[(int64_t)b * S + i] = bad ? __int_as_float(0x7fffffff) : __fadd_rn(lin, __fmul_rn(jitter2[row * S + i], scale));
-    }
+  // utils.py:468-469 + :154-167: near/far python floats (double), torch.linspace's fp32 formula, jitter scaled by (far-near)/(2S)
+  const double half = (double)obj_diag[b] / 2.0, near = tn - half, far = tn + half, dist = (far - near) / (2.0 * S);
+  const float start = (float)(near + dist), end = (float)(far - dist);
+  const float step = S > 1 ? (end - start) / (float)(S - 1) : 0.f;
+  const float scale = (float)((far - near) / (2.0 * S));
+  const float c = it[b];
+  const bool in_table = c >= 0.f && c < (float)T;    // false for NaN too
+  const bool bad = !in_table && active[b] != 0;
+  const int64_t row = (int64_t)b * T + (in_table ? (int64_t)c : 0);
+  if (bad && err != nullptr && threadIdx.x == 0) *err = 1;
+  for (int i = threadIdx.x; i < S; i += blockDim.x) {
+    const float lin = i < S / 2 ? __fadd_rn(start, __fmul_rn(step, (float)i)) : __fsub_rn(end, __fmul_rn(step, (float)(S - 1 - i)));
+    z[(int64_t)b * S + i] = bad ? __int_as_float(0x7fffffff) : __fadd_rn(lin, __fmul_rn(jitter[row * S + i], scale));
+    if (z2 != nullptr) z2[(int64_t)b * S + i] = bad ? __int_as_float(0x7fffffff) : __fadd_rn(lin, __fmul_rn(jitter2[row * S + i], scale));
   }
 }
 
@@ -149,7 +139,7 @@ struct AdamGroups {
   int n[kMaxAdamGroups]; float lr[kMaxAdamGroups];   // n: elements of ONE row of the tensor (row r starts at r * n)
   float beta1, beta2, eps, weight_decay;
   float* step;             // device: steps taken so far, one counter per row (incremented here)
-  const uint8_t* active;   // per row, or null = every row active; an inactive row is left bit-for-bit unchanged
+  const uint8_t* active;   // per row; an inactive row is left bit-for-bit unchanged
   // loss history (hist null = none): an active row r writes {loss3[r][0..2], loss_rgb2[r * rgb2_stride]} to hist[r][step[r]][0..3]
   const float* loss3; const float* loss_rgb2; int rgb2_stride; float* hist; int hist_rows;
 };
@@ -158,7 +148,7 @@ struct AdamGroups {
 // One block per row; each row's bias corrections come from its own step counter.
 __global__ void __launch_bounds__(1024) adamw_step_kernel(const __grid_constant__ AdamGroups A) {
   const int r = blockIdx.x;
-  if (A.active != nullptr && A.active[r] == 0) return;
+  if (A.active[r] == 0) return;
   __shared__ float s_s;
   if (threadIdx.x == 0) s_s = A.step[r];
   __syncthreads();
@@ -194,45 +184,17 @@ __global__ void __launch_bounds__(1024) adamw_step_kernel(const __grid_constant_
 
 using namespace snb;
 
-extern "C" int snb_refine_pose_fwd(const float* rot_vec, const float* trans_vec, int32_t opt_cam_pose, float obj_diag,
-                                   int32_t n_samples, const float* jitter, float* cam, float* z, void* stream) {
-  SNB_REQUIRE(rot_vec && trans_vec && cam, "refine_pose_fwd: null pointer");
-  SNB_REQUIRE(z == nullptr || (jitter != nullptr && n_samples >= 1), "refine_pose_fwd: the sample vector needs jitter and n_samples >= 1");
-  SNB_REQUIRE(sm_count() > 0, "refine_pose_fwd: no CUDA device (there is no CPU fallback)");
-  const int threads = z ? ((n_samples + 31) / 32 * 32 < 1024 ? (n_samples + 31) / 32 * 32 : 1024) : 32;
-  refine_pose_fwd_kernel<<<1, threads, 0, (cudaStream_t)stream>>>(rot_vec, trans_vec, opt_cam_pose, obj_diag, nullptr, n_samples, jitter, nullptr,
-                                                                  nullptr, 0, 0, nullptr, nullptr, cam, z, nullptr);
-  SNB_LAUNCH_CHECK();
-  return 0;
-}
-
-extern "C" int snb_refine_pose_batch_fwd(const float* rot_vec, const float* trans_vec, int32_t n_objs, int32_t opt_cam_pose,
-                                         const float* obj_diag, int32_t n_samples, const float* jitter, const float* jitter2,
-                                         const float* step_counter, int32_t table_rows, float* cam, float* z, float* z2, void* stream) {
-  SNB_REQUIRE(n_objs >= 1 && rot_vec && trans_vec && cam, "refine_pose_batch_fwd: bad arguments");
-  SNB_REQUIRE(z == nullptr || (jitter != nullptr && obj_diag != nullptr && n_samples >= 1),
-              "refine_pose_batch_fwd: the sample vectors need jitter, obj_diag and n_samples >= 1");
-  SNB_REQUIRE(z2 == nullptr || (z != nullptr && jitter2 != nullptr), "refine_pose_batch_fwd: z2 needs z and jitter2");
-  SNB_REQUIRE(step_counter == nullptr || table_rows >= 1, "refine_pose_batch_fwd: a jitter table needs its row count");
-  SNB_REQUIRE(sm_count() > 0, "refine_pose_batch_fwd: no CUDA device (there is no CPU fallback)");
-  const int threads = z ? ((n_samples + 31) / 32 * 32 < 1024 ? (n_samples + 31) / 32 * 32 : 1024) : 32;
-  refine_pose_fwd_kernel<<<n_objs, threads, 0, (cudaStream_t)stream>>>(rot_vec, trans_vec, opt_cam_pose, 0.f, obj_diag, n_samples, jitter, jitter2,
-                                                                       step_counter, 0, table_rows, nullptr, nullptr, cam, z, z2);
-  SNB_LAUNCH_CHECK();
-  return 0;
-}
-
 extern "C" int snb_refine_pose_slots_fwd(const float* rot_vec, const float* trans_vec, int32_t n_slots, int32_t opt_cam_pose,
                                          const float* obj_diag, int32_t n_samples, const float* jitter, const float* jitter2,
                                          const float* step_counters, int32_t table_rows, const uint8_t* active, int32_t* err_flag,
                                          float* cam, float* z, float* z2, void* stream) {
-  SNB_REQUIRE(n_slots >= 1 && rot_vec && trans_vec && cam && z && jitter && obj_diag && step_counters && n_samples >= 1 && table_rows >= 1,
-              "refine_pose_slots_fwd: bad arguments");
+  SNB_REQUIRE(n_slots >= 1 && rot_vec && trans_vec && cam && z && jitter && obj_diag && step_counters && active && n_samples >= 1 &&
+              table_rows >= 1, "refine_pose_slots_fwd: bad arguments");
   SNB_REQUIRE(z2 == nullptr || jitter2 != nullptr, "refine_pose_slots_fwd: z2 needs jitter2");
   SNB_REQUIRE(sm_count() > 0, "refine_pose_slots_fwd: no CUDA device (there is no CPU fallback)");
   const int threads = (n_samples + 31) / 32 * 32 < 1024 ? (n_samples + 31) / 32 * 32 : 1024;
-  refine_pose_fwd_kernel<<<n_slots, threads, 0, (cudaStream_t)stream>>>(rot_vec, trans_vec, opt_cam_pose, 0.f, obj_diag, n_samples, jitter, jitter2,
-                                                                        step_counters, 1, table_rows, active, err_flag, cam, z, z2);
+  refine_pose_fwd_kernel<<<n_slots, threads, 0, (cudaStream_t)stream>>>(rot_vec, trans_vec, opt_cam_pose, obj_diag, n_samples, jitter, jitter2,
+                                                                        step_counters, table_rows, active, err_flag, cam, z, z2);
   SNB_LAUNCH_CHECK();
   return 0;
 }
@@ -246,55 +208,29 @@ extern "C" int snb_refine_pose_batch_bwd(const float* rot_vec, const float* tran
   return 0;
 }
 
-extern "C" int snb_refine_pose_bwd(const float* rot_vec, const float* trans_vec, int32_t opt_cam_pose, const float* g_cam,
-                                   float* g_rot, float* g_trans, void* stream) {
-  SNB_REQUIRE(rot_vec && trans_vec && g_cam && g_rot && g_trans, "refine_pose_bwd: null pointer");
-  SNB_REQUIRE(sm_count() > 0, "refine_pose_bwd: no CUDA device (there is no CPU fallback)");
-  refine_pose_bwd_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(rot_vec, trans_vec, opt_cam_pose, g_cam, g_rot, g_trans);
-  SNB_LAUNCH_CHECK();
-  return 0;
-}
-
-static int adamw_launch(const char* what, int32_t n_groups, float* const* params, const float* const* grads, float* const* exp_avg,
-                        float* const* exp_avg_sq, const int32_t* sizes, const float* lrs, float beta1, float beta2, float eps,
-                        float weight_decay, int32_t n_rows, int threads, AdamGroups& A, cudaStream_t stream) {
-  SNB_REQUIRE(n_groups >= 1 && n_groups <= kMaxAdamGroups, "%s: 1..%d tensors", what, kMaxAdamGroups);
-  SNB_REQUIRE(params && grads && exp_avg && exp_avg_sq && sizes && lrs && A.step, "%s: null pointer", what);
-  SNB_REQUIRE(sm_count() > 0, "%s: no CUDA device (there is no CPU fallback)", what);
-  A.n_groups = n_groups;
-  for (int i = 0; i < n_groups; ++i) {
-    SNB_REQUIRE(params[i] && grads[i] && exp_avg[i] && exp_avg_sq[i] && sizes[i] >= 0, "%s: bad tensor %d", what, i);
-    A.p[i] = params[i]; A.g[i] = grads[i]; A.m[i] = exp_avg[i]; A.v[i] = exp_avg_sq[i]; A.n[i] = sizes[i]; A.lr[i] = lrs[i];
-  }
-  A.beta1 = beta1; A.beta2 = beta2; A.eps = eps; A.weight_decay = weight_decay;
-  adamw_step_kernel<<<n_rows, threads, 0, stream>>>(A);
-  SNB_LAUNCH_CHECK();
-  return 0;
-}
-
-extern "C" int snb_adamw_step(int32_t n_groups, float* const* params, const float* const* grads, float* const* exp_avg,
-                              float* const* exp_avg_sq, const int32_t* sizes, const float* lrs, float beta1, float beta2, float eps,
-                              float weight_decay, float* step, void* stream) {
-  AdamGroups A{};
-  A.step = step;
-  return adamw_launch("adamw_step", n_groups, params, grads, exp_avg, exp_avg_sq, sizes, lrs, beta1, beta2, eps, weight_decay, 1, 1024, A,
-                      (cudaStream_t)stream);
-}
-
 extern "C" int snb_adamw_step_rows(int32_t n_groups, float* const* params, const float* const* grads, float* const* exp_avg,
                                    float* const* exp_avg_sq, const int32_t* row_sizes, const float* lrs, float beta1, float beta2,
                                    float eps, float weight_decay, int32_t n_rows, float* steps, const uint8_t* active,
                                    const float* loss3, const float* loss_rgb2, int32_t loss_rgb2_stride, float* loss_history,
                                    int32_t history_rows, void* stream) {
+  SNB_REQUIRE(n_groups >= 1 && n_groups <= kMaxAdamGroups, "adamw_step_rows: 1..%d tensors", kMaxAdamGroups);
   SNB_REQUIRE(n_rows >= 1, "adamw_step_rows: n_rows >= 1");
+  SNB_REQUIRE(params && grads && exp_avg && exp_avg_sq && row_sizes && lrs && steps && active, "adamw_step_rows: null pointer");
   SNB_REQUIRE(loss_history == nullptr || (loss3 && loss_rgb2 && history_rows >= 1), "adamw_step_rows: the loss history needs its sources");
-  SNB_REQUIRE(row_sizes != nullptr, "adamw_step_rows: null pointer");
-  int widest = 1;
-  for (int i = 0; i < n_groups && i < kMaxAdamGroups; ++i) widest = row_sizes[i] > widest ? row_sizes[i] : widest;
-  const int threads = (widest + 31) / 32 * 32 < 1024 ? (widest + 31) / 32 * 32 : 1024;
+  SNB_REQUIRE(sm_count() > 0, "adamw_step_rows: no CUDA device (there is no CPU fallback)");
   AdamGroups A{};
+  A.n_groups = n_groups;
+  int widest = 1;
+  for (int i = 0; i < n_groups; ++i) {
+    SNB_REQUIRE(params[i] && grads[i] && exp_avg[i] && exp_avg_sq[i] && row_sizes[i] >= 0, "adamw_step_rows: bad tensor %d", i);
+    A.p[i] = params[i]; A.g[i] = grads[i]; A.m[i] = exp_avg[i]; A.v[i] = exp_avg_sq[i]; A.n[i] = row_sizes[i]; A.lr[i] = lrs[i];
+    widest = row_sizes[i] > widest ? row_sizes[i] : widest;
+  }
+  A.beta1 = beta1; A.beta2 = beta2; A.eps = eps; A.weight_decay = weight_decay;
   A.step = steps; A.active = active;
   A.loss3 = loss3; A.loss_rgb2 = loss_rgb2; A.rgb2_stride = loss_rgb2_stride; A.hist = loss_history; A.hist_rows = history_rows;
-  return adamw_launch("adamw_step_rows", n_groups, params, grads, exp_avg, exp_avg_sq, row_sizes, lrs, beta1, beta2, eps, weight_decay,
-                      n_rows, threads, A, (cudaStream_t)stream);
+  const int threads = (widest + 31) / 32 * 32 < 1024 ? (widest + 31) / 32 * 32 : 1024;
+  adamw_step_kernel<<<n_rows, threads, 0, (cudaStream_t)stream>>>(A);
+  SNB_LAUNCH_CHECK();
+  return 0;
 }

@@ -15,9 +15,10 @@ then is kernel time (~25 launches replayed from one graph: 0.21 ms at 32x32 rays
 Python / launch latency.
 
 The render, loss and their backward are the package's fused kernels (ops.render_shell, losses.refine_loss); with
-``fused=True`` (default) the pose map + sample vector and the AdamW update are single launches too (csrc/refine.cu:
-snb_refine_pose_fwd/bwd, snb_adamw_step); ``fused=False`` keeps them as torch ops (torch.optim.AdamW(capturable=True)) --
-the tests check both against the loop written with the reference-shaped API.  CUDA only."""
+``fused=True`` (default) the pose map + sample vectors and the AdamW update are single launches too (csrc/refine.cu:
+snb_refine_pose_slots_fwd / snb_refine_pose_batch_bwd, snb_adamw_step_rows -- the same launches BatchRefiner and SlotRefiner issue
+for many objects, here with one row); ``fused=False`` keeps them as torch ops (torch.optim.AdamW(capturable=True)) -- the tests
+check both against the loop written with the reference-shaped API.  CUDA only."""
 import ctypes
 import math
 
@@ -29,53 +30,23 @@ from . import utils as U
 from ._lib import check, f32c, on_device, ptr, require_cuda, stream_ptr
 
 
-class _PoseAndSamples(torch.autograd.Function):
-    """rot_vec, trans_vec -> cam2opt (3,4) and the shared sample vector z (S) in ONE launch (csrc/refine.cu); backward in one."""
+class SlotAdamW:
+    """torch.optim.AdamW's update on `rows` independent rows of a handful of small tensors (one row per object or refine slot) in ONE
+    launch (snb_adamw_step_rows); state lives on the device.  Each row has its own step counter (``step_t`` (rows,)), which also picks
+    its jitter row in the pose map, and active byte (``active`` (rows,) uint8); an inactive row is left bit-for-bit unchanged."""
 
-    @staticmethod
-    def forward(ctx, rot_vec, trans_vec, jitter, opt_cam_pose, obj_diag, n_samples):
-        lib = _lib.load()
-        require_cuda(rot_vec, trans_vec, jitter)
-        rot_vec, trans_vec, jitter = f32c(rot_vec), f32c(trans_vec), f32c(jitter)
-        dev = rot_vec.device
-        cam = torch.empty(3, 4, device=dev, dtype=torch.float32)
-        z = torch.empty(int(n_samples), device=dev, dtype=torch.float32)
-        with on_device(dev):
-            check(lib.snb_refine_pose_fwd(ptr(rot_vec), ptr(trans_vec), int(bool(opt_cam_pose)), float(obj_diag), int(n_samples), ptr(jitter),
-                                          ptr(cam), ptr(z), stream_ptr()), "snb_refine_pose_fwd")
-        ctx.save_for_backward(rot_vec, trans_vec)
-        ctx.opt_cam_pose = int(bool(opt_cam_pose))
-        ctx.mark_non_differentiable(z)
-        ctx.set_materialize_grads(False)
-        return cam, z
-
-    @staticmethod
-    def backward(ctx, g_cam, _g_z):
-        lib = _lib.load()
-        rot_vec, trans_vec = ctx.saved_tensors
-        if g_cam is None:
-            return None, None, None, None, None, None
-        g_cam = f32c(g_cam)
-        g_rot, g_trans = torch.empty_like(rot_vec), torch.empty_like(trans_vec)
-        with on_device(rot_vec.device):
-            check(lib.snb_refine_pose_bwd(ptr(rot_vec), ptr(trans_vec), ctx.opt_cam_pose, ptr(g_cam), ptr(g_rot), ptr(g_trans), stream_ptr()),
-                  "snb_refine_pose_bwd")
-        return g_rot, g_trans, None, None, None, None
-
-
-class FusedAdamW:
-    """torch.optim.AdamW's update for a handful of small tensors in ONE launch (snb_adamw_step); state lives on the device."""
-
-    def __init__(self, groups, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2):
+    def __init__(self, groups, rows, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2):
         self.params = [g["params"] for g in groups]
         self.lrs = [float(g["lr"]) for g in groups]
         self.betas, self.eps, self.weight_decay = betas, eps, weight_decay
         dev = self.params[0].device
+        self.rows = int(rows)
         self.m = [torch.zeros_like(p) for p in self.params]
         self.v = [torch.zeros_like(p) for p in self.params]
-        self.step_t = torch.zeros((), device=dev, dtype=torch.float32)
+        self.step_t = torch.zeros(self.rows, device=dev, dtype=torch.float32)
+        self.active = torch.ones(self.rows, device=dev, dtype=torch.uint8)
         n = len(self.params)
-        self._sizes = (ctypes.c_int32 * n)(*[p.numel() for p in self.params])
+        self._sizes = (ctypes.c_int32 * n)(*[p.numel() // self.rows for p in self.params])
         self._lrs = (ctypes.c_float * n)(*self.lrs)
 
     def zero_grad(self, set_to_none=True):
@@ -87,32 +58,6 @@ class FusedAdamW:
                     p.grad = None
                 else:
                     p.grad.zero_()
-
-    def reset(self):
-        for t in self.m + self.v:
-            t.zero_()
-        self.step_t.zero_()
-
-    def step(self):
-        lib = _lib.load()
-        n = len(self.params)
-        arr = lambda ts: (ctypes.c_void_p * n)(*[t.data_ptr() for t in ts])  # noqa: E731
-        with on_device(self.params[0].device):
-            check(lib.snb_adamw_step(n, arr(self.params), arr([p.grad for p in self.params]), arr(self.m), arr(self.v), self._sizes, self._lrs,
-                                     self.betas[0], self.betas[1], self.eps, self.weight_decay, ptr(self.step_t), stream_ptr()), "snb_adamw_step")
-
-
-class SlotAdamW(FusedAdamW):
-    """FusedAdamW on `rows` independent rows of every parameter (one per refine slot) in ONE launch (snb_adamw_step_rows): each row has its own
-    step counter (``step_t`` (rows,)) and active byte (``active`` (rows,) uint8); an inactive row is left bit-for-bit unchanged."""
-
-    def __init__(self, groups, rows, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-2):
-        super().__init__(groups, betas=betas, eps=eps, weight_decay=weight_decay)
-        dev = self.params[0].device
-        self.rows = int(rows)
-        self.step_t = torch.zeros(self.rows, device=dev, dtype=torch.float32)
-        self.active = torch.ones(self.rows, device=dev, dtype=torch.uint8)
-        self._sizes = (ctypes.c_int32 * len(self.params))(*[p.numel() // self.rows for p in self.params])
 
     def reset_row(self, r):
         """Zero row r's moments and step counter (stream-ordered, no host synchronisation)."""
@@ -132,6 +77,73 @@ class SlotAdamW(FusedAdamW):
             check(lib.snb_adamw_step_rows(n, arr(self.params), arr([p.grad for p in self.params]), arr(self.m), arr(self.v), self._sizes, self._lrs,
                                           self.betas[0], self.betas[1], self.eps, self.weight_decay, self.rows, ptr(self.step_t), ptr(self.active),
                                           ptr(loss3), ptr(loss_rgb2), stride, ptr(history), t_rows, stream_ptr()), "snb_adamw_step_rows")
+
+
+class _PoseAndSamplesBatch(torch.autograd.Function):
+    """(B,3) rot_vec, trans_vec -> cam2opt (B,3,4) + every object's shared sample vector z (B,S) [+ a second one, z2, from another jitter
+    table] in ONE launch (snb_refine_pose_slots_fwd).  Object b reads row step_t[b] of its jitter tables (B, T, S) -- its optimiser's step
+    counter; an active object (`active` (B,) uint8) whose counter lies outside the table gets NaN samples and sets `err` (optional)."""
+
+    @staticmethod
+    def forward(ctx, rot_vec, trans_vec, jitter, jitter2, step_t, obj_diag, opt_cam_pose, n_samples, active, err=None):
+        lib = _lib.load()
+        require_cuda(rot_vec, trans_vec, jitter, step_t, obj_diag, active)
+        rot_vec, trans_vec = f32c(rot_vec), f32c(trans_vec)
+        b, t, s = jitter.shape
+        dev = rot_vec.device
+        cam = torch.empty(b, 3, 4, device=dev, dtype=torch.float32)
+        z = torch.empty(b, s, device=dev, dtype=torch.float32)
+        z2 = torch.empty(b, s, device=dev, dtype=torch.float32) if jitter2 is not None else None
+        with on_device(dev):
+            check(lib.snb_refine_pose_slots_fwd(ptr(rot_vec), ptr(trans_vec), int(b), int(bool(opt_cam_pose)), ptr(obj_diag), int(n_samples),
+                                                ptr(jitter), ptr(jitter2), ptr(step_t), int(t), ptr(active), ptr(err), ptr(cam), ptr(z),
+                                                ptr(z2), stream_ptr()), "snb_refine_pose_slots_fwd")
+        ctx.save_for_backward(rot_vec, trans_vec)
+        ctx.opt_cam_pose = int(bool(opt_cam_pose))
+        ctx.set_materialize_grads(False)
+        if z2 is None:
+            ctx.mark_non_differentiable(z)
+            return cam, z
+        ctx.mark_non_differentiable(z, z2)
+        return cam, z, z2
+
+    @staticmethod
+    def backward(ctx, g_cam, *_):
+        lib = _lib.load()
+        rot_vec, trans_vec = ctx.saved_tensors
+        if g_cam is None:
+            return (None,) * 10
+        g_cam = f32c(g_cam)
+        g_rot, g_trans = torch.empty_like(rot_vec), torch.empty_like(trans_vec)
+        with on_device(rot_vec.device):
+            check(lib.snb_refine_pose_batch_bwd(ptr(rot_vec), ptr(trans_vec), int(rot_vec.shape[0]), ctx.opt_cam_pose, ptr(g_cam), ptr(g_rot),
+                                                ptr(g_trans), stream_ptr()), "snb_refine_pose_batch_bwd")
+        return (g_rot, g_trans) + (None,) * 8
+
+
+def _capture(device, warm_up, body):
+    """Run warm_up() on a side stream (allocator, weight packing, AdamW state), then record body() into a CUDA graph.  The capture
+    itself does not execute: the state after it is the one warm_up() left."""
+    s = torch.cuda.Stream(device=device)
+    s.wait_stream(torch.cuda.current_stream(device))
+    with torch.cuda.stream(s):
+        warm_up()
+    torch.cuda.current_stream(device).wait_stream(s)
+    graph = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(graph):
+        body()
+    return graph
+
+
+def _reserve(refiners, iters):
+    """Count `iters` more iterations of every ObjectRefiner against its pre-drawn jitter tables, before any of them is issued.
+    -> iters.  ValueError, counting nothing, if one of them would read past its tables."""
+    iters = int(iters)
+    if iters < 0 or any(iters > r.remaining for r in refiners):
+        raise ValueError("iters exceeds the pre-drawn jitter table (max_iters)")
+    for r in refiners:
+        r.remaining -= iters
+    return iters
 
 
 def axis_angle_to_matrix(v):
@@ -184,11 +196,11 @@ class ObjectRefiner:
         self.texturecode = texturecode.detach().to(dev).clone().requires_grad_()
         self.rot_vec = rot_vec.detach().to(dev).reshape(3).clone().requires_grad_()
         self.trans_vec = trans_vec.detach().to(dev).reshape(3).clone().requires_grad_()
-        # fused = True: pose map + sample vector and the AdamW update as single launches (csrc/refine.cu); False: torch ops
+        # fused = True: pose map + sample vectors and the AdamW update as single launches (csrc/refine.cu, one row); False: torch ops
         self.fused = bool(fused)
         if self.fused:
-            self.opt = FusedAdamW([{"params": self.shapecode, "lr": lr_shape}, {"params": self.texturecode, "lr": lr_texture},
-                                   {"params": self.rot_vec, "lr": lr_pose}, {"params": self.trans_vec, "lr": lr_pose}])
+            self.opt = SlotAdamW([{"params": self.shapecode, "lr": lr_shape}, {"params": self.texturecode, "lr": lr_texture},
+                                  {"params": self.rot_vec, "lr": lr_pose}, {"params": self.trans_vec, "lr": lr_pose}], rows=1)
         else:
             self.opt = torch.optim.AdamW([{"params": [self.shapecode], "lr": lr_shape}, {"params": [self.texturecode], "lr": lr_texture},
                                           {"params": [self.rot_vec], "lr": lr_pose}, {"params": [self.trans_vec], "lr": lr_pose}],
@@ -196,7 +208,7 @@ class ObjectRefiner:
         # Per-iteration evaluation the reference interleaves with the optimisation (optimizer_nuscenes.py:740-769): the PSNR loss over
         # the object mask only (loss_rgb2) and a no-grad depth render of the pixels that carry a lidar return (render_rays_specified).
         # lidar_xy = (x_vec, y_vec): integer pixel offsets inside the crop (np.where of the depth map, :759); None = not evaluated.
-        self.lidar = None
+        self.lidar, self.n_lidar = None, 0
         if lidar_xy is not None:
             x_vec, y_vec = np.asarray(lidar_xy[0]), np.asarray(lidar_xy[1])
             self.n_lidar = int(x_vec.shape[0])
@@ -216,7 +228,11 @@ class ObjectRefiner:
         draws = torch.stack([torch.rand(self.n_samples) for _ in range(max_iters * per_it)]).to(dev)
         self.jitter = draws[0::per_it].contiguous()
         self.jitter_lidar = draws[1::per_it].contiguous() if self.lidar is not None else None
-        self.it = torch.zeros((), dtype=torch.long, device=dev)
+        self.remaining = int(max_iters)   # host-side count of the iterations left in the jitter tables (eager steps and replays alike)
+        if self.fused:                     # the jitter row is the optimiser's step counter
+            self.obj_diag_dev = torch.tensor([float(self.obj_diag)], device=dev)
+        else:                              # the jitter row of the next iteration
+            self.it = torch.zeros((), dtype=torch.long, device=dev)
         self.loss = torch.zeros(3, device=dev)
         self.graph = None
 
@@ -229,13 +245,20 @@ class ObjectRefiner:
         return torch.cat((rot, t), dim=-1)
 
     def step(self):
-        """One iteration (no host synchronisation anywhere)."""
+        """One iteration, eagerly (no host synchronisation anywhere)."""
+        _reserve([self], 1)
+        return self._iteration()
+
+    def _iteration(self):
         if self.shapecode.grad is not None:
             self.opt.zero_grad() if self.fused else self.opt.zero_grad(set_to_none=False)
-        jit = self.jitter.index_select(0, self.it.reshape(1)).reshape(-1)
-        if self.fused:
-            cam, z = _PoseAndSamples.apply(self.rot_vec, self.trans_vec, jit, self.opt_cam_pose, self.obj_diag, self.n_samples)
+        if self.fused:   # (1, 3) views of the pose parameters, (1, T, S) views of the jitter tables
+            out = _PoseAndSamplesBatch.apply(self.rot_vec.view(1, 3), self.trans_vec.view(1, 3), self.jitter[None],
+                                             None if self.lidar is None else self.jitter_lidar[None], self.opt.step_t, self.obj_diag_dev,
+                                             self.opt_cam_pose, self.n_samples, self.opt.active)
+            cam, z = out[0].view(3, 4), out[1].view(-1)
         else:
+            jit = self.jitter.index_select(0, self.it.reshape(1)).reshape(-1)
             cam = self.cam2opt()
             z = shell_samples_on_device(cam, self.obj_diag, self.n_samples, jit)
         prec = self.model.precision or models.get_default_precision()
@@ -246,57 +269,56 @@ class ObjectRefiner:
         with torch.no_grad():       # the per-iteration evaluation (optimizer_nuscenes.py:740-769), before the parameter update as there
             self.loss_rgb2 = losses.refine_loss(rgb.detach(), acc.detach(), self.rgb_tgt, self.occ_pos, 0.0)[1]
             if self.lidar is not None:
-                jit2 = self.jitter_lidar.index_select(0, self.it.reshape(1)).reshape(-1)
                 if self.fused:
-                    cam2, z2 = _PoseAndSamples.apply(self.rot_vec.detach(), self.trans_vec.detach(), jit2, self.opt_cam_pose, self.obj_diag, self.n_samples)
+                    z2 = out[2].view(-1)
                 else:
-                    cam2 = cam.detach()
-                    z2 = shell_samples_on_device(cam2, self.obj_diag, self.n_samples, jit2)
+                    jit2 = self.jitter_lidar.index_select(0, self.it.reshape(1)).reshape(-1)
+                    z2 = shell_samples_on_device(cam.detach(), self.obj_diag, self.n_samples, jit2)
                 _, dep2, _ = ops.render_shell(self.model._handle(self.device), prec, self.n_samples, float(self.obj_diag), self.swap,
-                                              self.lidar[0], self.lidar[1], self.K, cam2, z2, self.shapecode.detach(), self.texturecode.detach(),
-                                              self.model._weights())
+                                              self.lidar[0], self.lidar[1], self.K, cam.detach(), z2, self.shapecode.detach(),
+                                              self.texturecode.detach(), self.model._weights())
                 self.depth_pred = dep2[:self.n_lidar]
         self.opt.step()
         self.loss = vec   # [loss, loss_rgb, loss_occ] as the loss kernel wrote them (graph mode: a static tensor of the graph's pool)
-        self.it += 1
+        if not self.fused:
+            self.it += 1
         return self.loss
 
+    def _warm_up(self, steps):
+        """`steps` iterations on the current stream that leave the refine state as it was.  Fused: with the active byte cleared, so
+        nothing is updated or counted and the jitter row stays inside the table; else: undone from a snapshot, each from row 0."""
+        if self.fused:
+            self.opt.active.zero_()
+            for _ in range(steps):
+                self._iteration()
+            self.opt.active.fill_(1)
+            return
+        state = (self.shapecode, self.texturecode, self.rot_vec, self.trans_vec, self.it)
+        snapshot = [t.detach().clone() for t in state]
+        for _ in range(steps):
+            self.it.zero_()
+            self._iteration()
+        with torch.no_grad():       # parameters, iteration counter, AdamW moments and step counters
+            for t, v in zip(state, snapshot):
+                t.copy_(v)
+            for st in self.opt.state.values():
+                for v in st.values():
+                    if torch.is_tensor(v):
+                        v.zero_()
+
     def capture(self, warmup=3):
-        """Warm up on a side stream (allocator, weight packing, AdamW state), then capture one iteration."""
-        s = torch.cuda.Stream(device=self.device)
-        s.wait_stream(torch.cuda.current_stream(self.device))
-        with torch.cuda.stream(s):
-            snapshot = [t.detach().clone() for t in (self.shapecode, self.texturecode, self.rot_vec, self.trans_vec)]
-            for _ in range(warmup):
-                self.step()
-            # undo the warm-up updates: parameters, AdamW moments and step counters, iteration counter
-            with torch.no_grad():
-                for t, v in zip((self.shapecode, self.texturecode, self.rot_vec, self.trans_vec), snapshot):
-                    t.copy_(v)
-                if self.fused:
-                    self.opt.reset()
-                else:
-                    for st in self.opt.state.values():
-                        for v in st.values():
-                            if torch.is_tensor(v):
-                                v.zero_()
-                self.it.zero_()
-        torch.cuda.current_stream(self.device).wait_stream(s)
-        self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph):
-            self.step()
-        # the capture itself does not execute: state is still the pre-capture one
+        """Warm up on a side stream, then capture one iteration."""
+        self.graph = _capture(self.device, lambda: self._warm_up(warmup), self._iteration)
         return self
 
     def run(self, iters):
-        """Run `iters` iterations (graph replays if captured).  Returns the last [loss, loss_rgb, loss_occ] (device tensor)."""
-        if int(iters) > self.jitter.shape[0]:
-            raise ValueError("iters exceeds the pre-drawn jitter table (max_iters)")
-        for _ in range(int(iters)):
+        """Run `iters` iterations (graph replays if captured).  Returns the last [loss, loss_rgb, loss_occ] (device tensor).
+        ValueError, issuing nothing, if they would run past the pre-drawn jitter table (max_iters iterations in all)."""
+        for _ in range(_reserve([self], iters)):
             if self.graph is not None:
                 self.graph.replay()
             else:
-                self.step()
+                self._iteration()
         return self.loss
 
 
@@ -336,267 +358,49 @@ class ObjectGroup:
         self.graph = None
 
     def capture(self, warmup=3):
+        """Warm up every object on a side stream (ObjectRefiner's warm-up), then capture one iteration of all of them."""
         dev = self.device
-        side = torch.cuda.Stream(device=dev)
-        side.wait_stream(torch.cuda.current_stream(dev))
-        with torch.cuda.stream(side):   # warm-up (allocator, weight packing, AdamW state), then undo it -- as ObjectRefiner.capture does
-            for r in self.refiners:
-                snapshot = [t.detach().clone() for t in (r.shapecode, r.texturecode, r.rot_vec, r.trans_vec)]
-                for _ in range(warmup):
-                    r.step()
-                with torch.no_grad():
-                    for t, v in zip((r.shapecode, r.texturecode, r.rot_vec, r.trans_vec), snapshot):
-                        t.copy_(v)
-                    if r.fused:
-                        r.opt.reset()
-                    else:
-                        for st in r.opt.state.values():
-                            for v in st.values():
-                                if torch.is_tensor(v):
-                                    v.zero_()
-                    r.it.zero_()
-        torch.cuda.current_stream(dev).wait_stream(side)
         streams = [torch.cuda.Stream(device=dev) for _ in self.refiners]
-        self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph):
+
+        def iteration():
             main = torch.cuda.current_stream(dev)
             for s_, r in zip(streams, self.refiners):
                 s_.wait_stream(main)                 # fork
                 with torch.cuda.stream(s_):
-                    r.step()
+                    r._iteration()
             for s_ in streams:
                 main.wait_stream(s_)                 # join
+
+        def warm_up():
+            for r in self.refiners:
+                r._warm_up(warmup)
+        self.graph = _capture(dev, warm_up, iteration)
         return self
 
     def run(self, iters):
-        """`iters` iterations of every object.  -> the objects' last [loss, loss_rgb, loss_occ] tensors."""
-        if any(int(iters) > r.jitter.shape[0] for r in self.refiners):
-            raise ValueError("iters exceeds the pre-drawn jitter table (max_iters)")
-        for _ in range(int(iters)):
+        """`iters` iterations of every object.  -> the objects' last [loss, loss_rgb, loss_occ] tensors.  ValueError, issuing nothing, if
+        one object would run past its pre-drawn jitter table."""
+        for _ in range(_reserve(self.refiners, iters)):
             if self.graph is not None:
                 self.graph.replay()
             else:
                 for r in self.refiners:
-                    r.step()
+                    r._iteration()
         return [r.loss for r in self.refiners]
 
 
-class _PoseAndSamplesBatch(torch.autograd.Function):
-    """(B,3) rot_vec, trans_vec -> cam2opt (B,3,4) + every object's shared sample vector z (B,S) [+ a second one, z2, from another jitter
-    table] in ONE launch (csrc/refine.cu); the jitter row is picked on the device by the optimiser's step counter: one shared scalar
-    (snb_refine_pose_batch_fwd), or -- with `active` (B,) uint8 -- one counter per slot (B,) whose out-of-table rows give NaN and set
-    `err` (snb_refine_pose_slots_fwd)."""
-
-    @staticmethod
-    def forward(ctx, rot_vec, trans_vec, jitter, jitter2, step_t, obj_diag, opt_cam_pose, n_samples, active=None, err=None):
-        lib = _lib.load()
-        require_cuda(rot_vec, trans_vec, jitter, step_t, obj_diag)
-        rot_vec, trans_vec = f32c(rot_vec), f32c(trans_vec)
-        b, t, s = jitter.shape
-        dev = rot_vec.device
-        cam = torch.empty(b, 3, 4, device=dev, dtype=torch.float32)
-        z = torch.empty(b, s, device=dev, dtype=torch.float32)
-        z2 = torch.empty(b, s, device=dev, dtype=torch.float32) if jitter2 is not None else None
-        with on_device(dev):
-            if active is None:
-                check(lib.snb_refine_pose_batch_fwd(ptr(rot_vec), ptr(trans_vec), int(b), int(bool(opt_cam_pose)), ptr(obj_diag), int(n_samples),
-                                                    ptr(jitter), ptr(jitter2), ptr(step_t), int(t), ptr(cam), ptr(z), ptr(z2), stream_ptr()),
-                      "snb_refine_pose_batch_fwd")
-            else:
-                check(lib.snb_refine_pose_slots_fwd(ptr(rot_vec), ptr(trans_vec), int(b), int(bool(opt_cam_pose)), ptr(obj_diag), int(n_samples),
-                                                    ptr(jitter), ptr(jitter2), ptr(step_t), int(t), ptr(active), ptr(err), ptr(cam), ptr(z),
-                                                    ptr(z2), stream_ptr()), "snb_refine_pose_slots_fwd")
-        ctx.save_for_backward(rot_vec, trans_vec)
-        ctx.opt_cam_pose = int(bool(opt_cam_pose))
-        ctx.set_materialize_grads(False)
-        if z2 is None:
-            ctx.mark_non_differentiable(z)
-            return cam, z
-        ctx.mark_non_differentiable(z, z2)
-        return cam, z, z2
-
-    @staticmethod
-    def backward(ctx, g_cam, *_):
-        lib = _lib.load()
-        rot_vec, trans_vec = ctx.saved_tensors
-        if g_cam is None:
-            return (None,) * 10
-        g_cam = f32c(g_cam)
-        g_rot, g_trans = torch.empty_like(rot_vec), torch.empty_like(trans_vec)
-        with on_device(rot_vec.device):
-            check(lib.snb_refine_pose_batch_bwd(ptr(rot_vec), ptr(trans_vec), int(rot_vec.shape[0]), ctx.opt_cam_pose, ptr(g_cam), ptr(g_rot),
-                                                ptr(g_trans), stream_ptr()), "snb_refine_pose_batch_bwd")
-        return (g_rot, g_trans) + (None,) * 8
-
-
-class _BatchStep:
-    """The per-iteration body of BatchRefiner and SlotRefiner: ObjectRefiner.step for every object (or slot) at once.  A subclass holds the
-    stacked state (codes, pose parameters, pixels, targets, jitter tables, lidar pixels) and supplies the two stages that differ: which
-    jitter row each object reads (`_pose_and_samples`) and the optimiser update (`_update`)."""
-
-    def _params(self):
-        return (self.shapecode, self.texturecode, self.rot_vec, self.trans_vec)
-
-    def step(self):
-        """One iteration of every object (no host synchronisation anywhere)."""
-        if self.shapecode.grad is not None:
-            self.opt.zero_grad()
-        out = self._pose_and_samples()
-        cam, z = out[0], out[1]
-        prec = self.model.precision or models.get_default_precision()
-        h, w = self.model._handle(self.device), self.model._weights()
-        rgb, _dep, acc = ops.render_shell_batch(h, prec, self.n_samples, self.swap, self.px, self.py, self.K, cam, z, self.obj_diag,
-                                                self.shapecode, self.texturecode, w)
-        loss, parts = losses.refine_loss_batch(rgb, acc, self.rgb_tgt, self.occ, self.coef)
-        torch.autograd.backward(loss, self._ones)
-        with torch.no_grad():       # the per-iteration evaluation (optimizer_nuscenes.py:740-769), before the parameter update as there
-            self.loss_rgb2 = losses.refine_loss_batch(rgb.detach(), acc.detach(), self.rgb_tgt, self.occ_pos, 0.0)[1][:, 1]
-            if self.lidar is not None:
-                _, dep2, _ = ops.render_shell_batch(h, prec, self.n_samples, self.swap, self.lidar[0], self.lidar[1], self.K, cam.detach(),
-                                                    out[2], self.obj_diag, self.shapecode.detach(), self.texturecode.detach(), w)
-                self.depth_pred = dep2           # (B, width): object b's lidar depths are depth_pred[b, :n_lidar[b]]
-        self.loss = parts           # (B,3) = [loss, loss_rgb, loss_occ] per object
-        self._update()
-        return self.loss
-
-
-class BatchRefiner(_BatchStep):
-    """The refine loops of B INDEPENDENT objects (one GPU's share of config C3) as ONE launch set per iteration: every stage of
-    ObjectRefiner.step -- pose map + sample vectors, the utils.py-stack render, the losses, their backward, the per-iteration
-    evaluation (loss_rgb2, lidar-pixel depths) and the AdamW update -- runs once over all objects (ops.render_shell_batch,
-    losses.refine_loss_batch, snb_refine_pose_batch_*), ~25 launches per iteration whatever B is instead of ~30 per object.  The objects
-    stay independent: per-object pose, codes, rays, targets, jitter draws, losses (the summed loss has block-diagonal gradients) and
-    elementwise AdamW state with one shared step count.
-
-    Built from ObjectRefiners (which hold the per-object inputs and the jitter tables drawn in the reference's order); they must agree on
-    n_samples, crop size, learning rates, loss coefficient, axis convention and decoder.  ``write_back()`` copies the optimised
-    state into them."""
-
-    def __init__(self, refiners):
-        if not refiners:
-            raise ValueError("BatchRefiner needs at least one refiner")
-        r0 = refiners[0]
-        same = lambda f: all(f(r) == f(r0) for r in refiners)   # noqa: E731
-        if not (same(lambda r: (r.n_samples, r.im_sz, r.coef, r.swap, r.opt_cam_pose, r.fused, tuple(r.opt.lrs) if r.fused else None,
-                                r.jitter.shape[0])) and all(r.model is r0.model and r.device == r0.device for r in refiners)):
-            raise ValueError("BatchRefiner: the objects must share the decoder, device, n_samples, crop size, loss and optimiser settings")
-        if not r0.fused:
-            raise ValueError("BatchRefiner builds on the fused refiners (fused=True)")
-        self.refiners = list(refiners)
-        self.model, self.device = r0.model, r0.device
-        dev = self.device
-        self.n_samples, self.coef, self.swap, self.opt_cam_pose = r0.n_samples, r0.coef, r0.swap, r0.opt_cam_pose
-        st = lambda f: torch.stack([f(r) for r in refiners]).contiguous()   # noqa: E731
-        self.px, self.py = st(lambda r: r.px.reshape(-1)), st(lambda r: r.py.reshape(-1))
-        self.K = st(lambda r: r.K)
-        self.rgb_tgt, self.occ = st(lambda r: r.rgb_tgt), st(lambda r: r.occ.reshape(-1))
-        self.occ_pos = self.occ.clamp_min(0.0)
-        self.obj_diag = torch.tensor([float(r.obj_diag) for r in refiners], device=dev, dtype=torch.float32)
-        self.shapecode = st(lambda r: r.shapecode.detach().reshape(-1)).requires_grad_()
-        self.texturecode = st(lambda r: r.texturecode.detach().reshape(-1)).requires_grad_()
-        self.rot_vec = st(lambda r: r.rot_vec.detach()).requires_grad_()
-        self.trans_vec = st(lambda r: r.trans_vec.detach()).requires_grad_()
-        lrs = r0.opt.lrs
-        self.opt = FusedAdamW([{"params": self.shapecode, "lr": lrs[0]}, {"params": self.texturecode, "lr": lrs[1]},
-                               {"params": self.rot_vec, "lr": lrs[2]}, {"params": self.trans_vec, "lr": lrs[3]}],
-                              betas=r0.opt.betas, eps=r0.opt.eps, weight_decay=r0.opt.weight_decay)
-        self.jitter = st(lambda r: r.jitter)                                  # (B, T, S)
-        self.max_iters = int(self.jitter.shape[1])
-        # lidar pixels: every object's list padded to one length (a whole number of 256-row decoder super tiles: 4 rays at 64 samples) with copies of
-        # its last pixel; the copies' depths are sliced off again.  Objects without lidar pixels render a dummy pixel and report nothing.
-        self.n_lidar = [r.n_lidar if r.lidar is not None else 0 for r in refiners]
-        self.lidar, self.jitter_lidar = None, None
-        if any(self.n_lidar):
-            q = 256 // math.gcd(256, self.n_samples)          # rays per 256 decoder rows (4 at 64 samples)
-            width = -(-max(self.n_lidar) // q) * q
-            lx, ly, jl = [], [], []
-            for r, n in zip(refiners, self.n_lidar):
-                if n:
-                    x, y = r.lidar[0][:n], r.lidar[1][:n]
-                    jl.append(r.jitter_lidar)
-                else:
-                    x, y = r.px.reshape(-1)[:1], r.py.reshape(-1)[:1]
-                    jl.append(torch.zeros_like(r.jitter))
-                lx.append(torch.cat([x, x[-1:].expand(width - x.numel())]))
-                ly.append(torch.cat([y, y[-1:].expand(width - y.numel())]))
-            self.lidar = (torch.stack(lx).contiguous(), torch.stack(ly).contiguous())
-            self.jitter_lidar = torch.stack(jl).contiguous()
-        b = len(refiners)
-        self._ones = torch.ones(b, device=dev)
-        self.loss = torch.zeros(b, 3, device=dev)
-        self.loss_rgb2 = torch.zeros(b, device=dev)
-        self.depth_pred = None
-        self.it = 0              # host-side count of issued iterations (the device-side row index is the optimiser's step counter)
-        self.graph = None
-
-    def _pose_and_samples(self):
-        return _PoseAndSamplesBatch.apply(self.rot_vec, self.trans_vec, self.jitter, self.jitter_lidar, self.opt.step_t, self.obj_diag,
-                                          self.opt_cam_pose, self.n_samples)
-
-    def _update(self):
-        self.opt.step()
-
-    def capture(self, warmup=3):
-        """Warm up on a side stream (allocator, weight packing), undo the warm-up updates, then capture one iteration."""
-        s = torch.cuda.Stream(device=self.device)
-        s.wait_stream(torch.cuda.current_stream(self.device))
-        with torch.cuda.stream(s):
-            snapshot = [t.detach().clone() for t in self._params()]
-            for _ in range(warmup):
-                self.step()
-            with torch.no_grad():
-                for t, v in zip(self._params(), snapshot):
-                    t.copy_(v)
-                self.opt.reset()
-        torch.cuda.current_stream(self.device).wait_stream(s)
-        self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph):
-            self.step()
-        return self
-
-    def run(self, iters):
-        """`iters` iterations of every object (graph replays if captured).  -> (B,3) last [loss, loss_rgb, loss_occ] per object."""
-        if self.it + int(iters) > self.max_iters:
-            raise ValueError("iters exceeds the pre-drawn jitter tables (max_iters)")
-        for _ in range(int(iters)):
-            if self.graph is not None:
-                self.graph.replay()
-            else:
-                self.step()
-        self.it += int(iters)
-        return self.loss
-
-    def lidar_depths(self):
-        """Per object: the depths at its lidar pixels from the last iteration's evaluation (None for an object without lidar pixels)."""
-        if self.depth_pred is None:
-            return [None] * len(self.refiners)
-        return [self.depth_pred[b, :n] if n else None for b, n in enumerate(self.n_lidar)]
-
-    def write_back(self):
-        """Copy the optimised codes and pose parameters into the ObjectRefiners this batch was built from."""
-        with torch.no_grad():
-            for b, r in enumerate(self.refiners):
-                r.shapecode.copy_(self.shapecode[b].reshape(r.shapecode.shape))
-                r.texturecode.copy_(self.texturecode[b].reshape(r.texturecode.shape))
-                r.rot_vec.copy_(self.rot_vec[b])
-                r.trans_vec.copy_(self.trans_vec[b])
-                r.loss = self.loss[b]
-                r.loss_rgb2 = self.loss_rgb2[b]
-        return self.refiners
-
-
-class SlotRefiner(_BatchStep):
+class SlotRefiner:
     """A stream of INDEPENDENT objects refined through C fixed slots (the reference's test-time refinement goes through the evaluation split
     one object at a time: optimize_objs_w_pose_unified, optimizer_nuscenes.py:684-769).  Each slot holds one object's refine state; one
-    iteration of all C slots is BatchRefiner's launch set, captured ONCE as a CUDA graph.  Between replays the host ``admit``s an
-    ObjectRefiner into a free slot with its own iteration budget, and ``run`` retires every object whose budget is used up, copying its
-    results back into its ObjectRefiner -- all stream-ordered, without a host synchronisation.  The host knows every slot's remaining budget
-    without reading the device: each replay advances every active slot by exactly one iteration.
+    iteration of all C slots is ONE launch set (ObjectRefiner's iteration over every slot at once), captured ONCE as a CUDA graph.
+    Between replays the host ``admit``s an ObjectRefiner into a free slot with its own iteration budget, and ``run`` retires every object
+    whose budget is used up, copying its results back into its ObjectRefiner -- all stream-ordered, without a host synchronisation.  The
+    host knows every slot's remaining budget without reading the device: each replay advances every active slot by exactly one iteration.
 
     Every slot has its own AdamW step counter (SlotAdamW), which also picks its jitter row, and an active byte.  A free slot keeps running
     on finite placeholder inputs (a fixed synthetic object at first, its last object's inputs with zero loss weights after a retirement):
     it takes no AdamW step, writes no loss history and reports nothing, but its render is paid.  ``max_lidar`` is the per-slot capacity of
-    lidar pixels evaluated every iteration (0 = no lidar evaluation)."""
+    lidar pixels evaluated every iteration (0 = no lidar evaluation).  ``capture()`` may come before or after admissions."""
 
     def __init__(self, model, device, slots=16, n_samples=64, im_sz=32, max_iters=100, max_lidar=0, lr_shape=0.02, lr_texture=0.02,
                  lr_pose=0.01, loss_occ_coef=0.1, shapenet_obj_cood=True, opt_cam_pose=False):
@@ -631,7 +435,7 @@ class SlotRefiner(_BatchStep):
         self.opt.active.zero_()
         self.jitter = torch.zeros(c, self.max_iters, s, device=dev)
         self.lidar, self.jitter_lidar, self.width = None, None, 0
-        if int(max_lidar) > 0:   # whole 256-row decoder super tiles per slot, as BatchRefiner pads them
+        if int(max_lidar) > 0:   # whole 256-row decoder super tiles per slot: 4 rays at 64 samples
             q = 256 // math.gcd(256, s)
             self.width = -(-int(max_lidar) // q) * q
             self.lidar = (self.px[:, :1].repeat(1, self.width).contiguous(), self.py[:, :1].repeat(1, self.width).contiguous())
@@ -650,27 +454,41 @@ class SlotRefiner(_BatchStep):
         self.busy_slot_iters = 0
         self.graph = None
 
-    def _pose_and_samples(self):
-        return _PoseAndSamplesBatch.apply(self.rot_vec, self.trans_vec, self.jitter, self.jitter_lidar, self.opt.step_t, self.obj_diag,
-                                          self.opt_cam_pose, self.n_samples, self.opt.active, self.err)
-
-    def _update(self):
+    def _iteration(self):
+        """ObjectRefiner's iteration for every slot at once (no host synchronisation anywhere)."""
+        if self.shapecode.grad is not None:
+            self.opt.zero_grad()
+        out = _PoseAndSamplesBatch.apply(self.rot_vec, self.trans_vec, self.jitter, self.jitter_lidar, self.opt.step_t, self.obj_diag,
+                                         self.opt_cam_pose, self.n_samples, self.opt.active, self.err)
+        cam, z = out[0], out[1]
+        prec = self.model.precision or models.get_default_precision()
+        h, w = self.model._handle(self.device), self.model._weights()
+        rgb, _dep, acc = ops.render_shell_batch(h, prec, self.n_samples, self.swap, self.px, self.py, self.K, cam, z, self.obj_diag,
+                                                self.shapecode, self.texturecode, w)
+        loss, parts = losses.refine_loss_batch(rgb, acc, self.rgb_tgt, self.occ, self.coef)
+        torch.autograd.backward(loss, self._ones)
+        with torch.no_grad():       # the per-iteration evaluation (optimizer_nuscenes.py:740-769), before the parameter update as there
+            self.loss_rgb2 = losses.refine_loss_batch(rgb.detach(), acc.detach(), self.rgb_tgt, self.occ_pos, 0.0)[1][:, 1]
+            if self.lidar is not None:
+                _, dep2, _ = ops.render_shell_batch(h, prec, self.n_samples, self.swap, self.lidar[0], self.lidar[1], self.K, cam.detach(),
+                                                    out[2], self.obj_diag, self.shapecode.detach(), self.texturecode.detach(), w)
+                self.depth_pred = dep2           # (C, width): slot b's lidar depths are depth_pred[b, :n_lidar[b]]
+        self.loss = parts           # (C,3) = [loss, loss_rgb, loss_occ] per slot
         self.opt.step(self.loss, self.loss_rgb2, self.history)
+        return self.loss
+
+    def _warm_up(self, steps):
+        """`steps` iterations with every active byte cleared: nothing is updated or counted and every slot reads a row inside its jitter
+        tables, so nothing needs restoring."""
+        active = self.opt.active.clone()
+        self.opt.active.zero_()
+        for _ in range(steps):
+            self._iteration()
+        self.opt.active.copy_(active)
 
     def capture(self, warmup=3):
-        """Warm up on a side stream (allocator, weight packing) with every slot free -- nothing is updated, so nothing needs restoring -- then
-        capture one iteration of all slots.  Done once, before the first admission."""
-        if any(o is not None for o in self.owner):
-            raise RuntimeError("SlotRefiner.capture: capture before admitting objects")
-        s = torch.cuda.Stream(device=self.device)
-        s.wait_stream(torch.cuda.current_stream(self.device))
-        with torch.cuda.stream(s):
-            for _ in range(warmup):
-                self.step()
-        torch.cuda.current_stream(self.device).wait_stream(s)
-        self.graph = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(self.graph):
-            self.step()
+        """Warm up on a side stream (allocator, weight packing), then capture one iteration of all slots, occupied or free."""
+        self.graph = _capture(self.device, lambda: self._warm_up(warmup), self._iteration)
         return self
 
     def free_slots(self):
@@ -692,7 +510,7 @@ class SlotRefiner(_BatchStep):
                              "(and be a fused ObjectRefiner)")
         if not 1 <= iters <= min(self.max_iters, r.jitter.shape[0]):
             raise ValueError("SlotRefiner.admit: iters must be in 1 .. min(max_iters, the object's jitter rows)")
-        n_lidar = r.n_lidar if r.lidar is not None else 0
+        n_lidar = r.n_lidar
         if n_lidar > self.width:
             raise ValueError("SlotRefiner.admit: %d lidar pixels exceed the slot capacity (%d)" % (n_lidar, self.width))
         free = self.free_slots()
@@ -717,7 +535,7 @@ class SlotRefiner(_BatchStep):
                 if n_lidar:
                     x, y = r.lidar[0][:n_lidar], r.lidar[1][:n_lidar]
                     self.jitter_lidar[b, :k].copy_(r.jitter_lidar[:k])
-                else:   # no lidar pixels: a dummy pixel is rendered and nothing reported, as in BatchRefiner
+                else:   # no lidar pixels: a dummy pixel is rendered and nothing reported
                     x, y = r.px.reshape(-1)[:1], r.py.reshape(-1)[:1]
                     self.jitter_lidar[b].zero_()
                 self.lidar[0][b, :x.numel()].copy_(x)
@@ -730,8 +548,9 @@ class SlotRefiner(_BatchStep):
         self.owner[b], self.budget[b], self.remaining[b], self.n_lidar[b] = r, iters, iters, n_lidar
         return b
 
-    def _retire(self, b):
-        """Copy slot b's results into its ObjectRefiner (as BatchRefiner.write_back does, plus loss_history (iters, 4)) and free the slot."""
+    def _copy_out(self, b):
+        """Copy slot b's results into its ObjectRefiner: codes, pose parameters, last losses, lidar depths and loss_history (iterations
+        run, 4)."""
         r, n = self.owner[b], self.n_lidar[b]
         with torch.no_grad():
             r.shapecode.copy_(self.shapecode[b].reshape(r.shapecode.shape))
@@ -740,23 +559,36 @@ class SlotRefiner(_BatchStep):
             r.trans_vec.copy_(self.trans_vec[b])
             r.loss = self.loss[b].clone()          # copies: the slot's buffers are rewritten by the next replay
             r.loss_rgb2 = self.loss_rgb2[b].clone()
-            if n:
+            if n and self.depth_pred is not None:
                 r.depth_pred = self.depth_pred[b, :n].clone()
-            r.loss_history = self.history[b, :self.budget[b]].clone()
+            r.loss_history = self.history[b, :self.budget[b] - self.remaining[b]].clone()
+
+    def _retire(self, b):
+        """Copy slot b's results into its ObjectRefiner and free the slot."""
+        self._copy_out(b)
+        with torch.no_grad():
             self.opt.active[b].fill_(0)
             # zero loss weights: the idle slot's upstream gradients are exactly zero, so the batched backward skips its decoder tiles
             self.occ[b].zero_()
             self.occ_pos[b].zero_()
         self.owner[b], self.remaining[b] = None, 0
 
+    def step(self):
+        """One iteration of every slot, eagerly; counted and retired as a replay is."""
+        return self._advance(1, eager=True)
+
     def run(self, iters):
         """`iters` iterations of every slot (graph replays if captured); an object whose budget is used up is retired right after its last
         iteration.  -> (C,3) last [loss, loss_rgb, loss_occ] per slot (device tensor)."""
-        for _ in range(int(iters)):
-            if self.graph is not None:
-                self.graph.replay()
+        return self._advance(int(iters))
+
+    def _advance(self, iters, eager=False):
+        """Issue `iters` iterations (graph replays unless eager or not captured) and count them on the host, slot by slot."""
+        for _ in range(iters):
+            if self.graph is None or eager:
+                self._iteration()
             else:
-                self.step()
+                self.graph.replay()
             self.replays += 1
             for b in range(self.slots):
                 if self.owner[b] is not None:
@@ -802,8 +634,74 @@ def refine_stream(refiners, iters, slots=16):
     if not refiners:
         return []
     budgets = [int(i) for i in iters] if hasattr(iters, "__len__") else [int(iters)] * len(refiners)
-    r0, lrs = refiners[0], refiners[0].opt.lrs
-    sr = SlotRefiner(r0.model, r0.device, slots=min(int(slots), len(refiners)), n_samples=r0.n_samples, im_sz=r0.im_sz, max_iters=max(budgets),
-                     max_lidar=max(r.n_lidar if r.lidar is not None else 0 for r in refiners), lr_shape=lrs[0], lr_texture=lrs[1],
-                     lr_pose=lrs[2], loss_occ_coef=r0.coef, shapenet_obj_cood=r0.swap, opt_cam_pose=r0.opt_cam_pose)
+    sr = SlotRefiner(refiners[0].model, refiners[0].device, slots=min(int(slots), len(refiners)), max_iters=max(budgets),
+                     max_lidar=max(r.n_lidar for r in refiners), **_settings(refiners[0]))
     return sr.capture().stream(refiners, budgets)
+
+
+def _settings(r):
+    """SlotRefiner's sample count, crop size, learning rates, loss coefficient and axis conventions from ObjectRefiner r's."""
+    lrs = r.opt.lrs
+    return dict(n_samples=r.n_samples, im_sz=r.im_sz, lr_shape=lrs[0], lr_texture=lrs[1], lr_pose=lrs[2], loss_occ_coef=r.coef,
+                shapenet_obj_cood=r.swap, opt_cam_pose=r.opt_cam_pose)
+
+
+class BatchRefiner(SlotRefiner):
+    """The refine loops of B INDEPENDENT objects (one GPU's share of config C3) as ONE launch set per iteration: every stage of
+    ObjectRefiner.step -- pose map + sample vectors, the utils.py-stack render, the losses, their backward, the per-iteration
+    evaluation (loss_rgb2, lidar-pixel depths) and the AdamW update -- runs once over all objects (ops.render_shell_batch,
+    losses.refine_loss_batch, snb_refine_pose_slots_fwd / snb_refine_pose_batch_bwd, snb_adamw_step_rows), ~25 launches per iteration
+    whatever B is instead of ~30 per object.  The objects stay independent: per-object pose, codes, rays, targets, jitter draws, losses
+    (the summed loss has block-diagonal gradients) and elementwise AdamW state.
+
+    A SlotRefiner with one slot per object, every slot admitted for the objects' whole jitter tables and never retired.  Built from
+    ObjectRefiners (which hold the per-object inputs and the jitter tables drawn in the reference's order); they must agree on n_samples,
+    crop size, learning rates, loss coefficient, axis convention, decoder and jitter rows.  ``write_back()`` copies the optimised state
+    into them."""
+
+    def __init__(self, refiners):
+        if not refiners:
+            raise ValueError("BatchRefiner needs at least one refiner")
+        r0 = refiners[0]
+        same = lambda f: all(f(r) == f(r0) for r in refiners)   # noqa: E731
+        if not (same(lambda r: (r.n_samples, r.im_sz, r.coef, r.swap, r.opt_cam_pose, r.fused, tuple(r.opt.lrs) if r.fused else None,
+                                r.jitter.shape[0])) and all(r.model is r0.model and r.device == r0.device for r in refiners)):
+            raise ValueError("BatchRefiner: the objects must share the decoder, device, n_samples, crop size, loss and optimiser settings")
+        if not r0.fused:
+            raise ValueError("BatchRefiner builds on the fused refiners (fused=True)")
+        super().__init__(r0.model, r0.device, slots=len(refiners), max_iters=r0.jitter.shape[0], max_lidar=max(r.n_lidar for r in refiners),
+                         **_settings(r0))
+        self.refiners = list(refiners)
+        for r in self.refiners:
+            self.admit(r, self.max_iters)
+
+    def step(self):
+        """One iteration of every object, eagerly.  ValueError if the jitter tables are used up."""
+        self._check(1)
+        return self._advance(1, eager=True)
+
+    def run(self, iters):
+        """`iters` iterations of every object (graph replays if captured).  -> (B,3) last [loss, loss_rgb, loss_occ] per object.
+        ValueError, issuing nothing, if they would run past the pre-drawn jitter tables (max_iters iterations in all)."""
+        self._check(iters)
+        return self._advance(int(iters))
+
+    def _check(self, iters):
+        if int(iters) < 0 or int(iters) > min(self.remaining):
+            raise ValueError("iters exceeds the pre-drawn jitter tables (max_iters)")
+
+    def _retire(self, b):
+        """Objects stay in their slots when their tables are used up: write_back() copies their state out."""
+
+    def lidar_depths(self):
+        """Per object: the depths at its lidar pixels from the last iteration's evaluation (None for an object without lidar pixels)."""
+        if self.depth_pred is None:
+            return [None] * len(self.refiners)
+        return [self.depth_pred[b, :n] if n else None for b, n in enumerate(self.n_lidar)]
+
+    def write_back(self):
+        """Copy the optimised codes, pose parameters and last results into the ObjectRefiners this batch was built from; the objects
+        stay in their slots."""
+        for b in range(self.slots):
+            self._copy_out(b)
+        return self.refiners

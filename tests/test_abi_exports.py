@@ -16,7 +16,7 @@ def _header_symbols():
     return sorted(set(re.findall(r"\b(snb_[a-z0-9_]+)\s*\(", src)))
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_exports_every_declared_symbol_at_abi_2():
     from supnerf_b200 import _lib
     from supnerf_b200.build import build
     build()
@@ -26,7 +26,7 @@ def test_library_exports_every_declared_symbol():
     for s in syms:
         assert hasattr(lib, s), f"{s} declared in include/supnerf_b200.h but not exported"
     assert set(_lib.SIGNATURES) == set(syms), set(_lib.SIGNATURES) ^ set(syms)
-    assert _lib.load().snb_abi_version() == 1
+    assert _lib.load().snb_abi_version() == 2
 
 
 def test_no_gpu_means_loud_failure():

@@ -777,7 +777,7 @@ def test_scene_merge_kernel_golden_and_random():
         S.scene.merge_objects(z, sig, col)     # CPU tensors: no fallback
 
 
-def test_refine_pose_and_adamw_kernels_vs_torch():
+def test_one_row_refine_pose_and_adamw_kernels_vs_torch():
     """csrc/refine.cu: the Rodrigues pose map (both conventions) + its backward against torch autograd in float64, the fused
     sample vector against refine.shell_samples_on_device, and the fused AdamW against torch.optim.AdamW over 5 steps."""
     S = snb()
@@ -797,7 +797,10 @@ def test_refine_pose_and_adamw_kernels_vs_torch():
             cam64 = torch.cat((rot, tt), -1)
             (cam64 * up.double()).sum().backward()
             rg, tg = rv.to(DEV).requires_grad_(), tv.to(DEV).requires_grad_()
-            cam, z = S.refine._PoseAndSamples.apply(rg, tg, jit.to(DEV), opt_cam, np.float32(4.7), 64)
+            one = torch.ones(1, device=DEV, dtype=torch.uint8)
+            cam, z = S.refine._PoseAndSamplesBatch.apply(rg.view(1, 3), tg.view(1, 3), jit.to(DEV).view(1, 1, 64), None,
+                                                         torch.zeros(1, device=DEV), torch.tensor([4.7], device=DEV), opt_cam, 64, one)
+            cam, z = cam.view(3, 4), z.view(64)
             (cam * up.to(DEV)).sum().backward()
             assert parity_ok("cam", cam, cam64, 1e-6)
             assert parity_ok("rg_grad", rg.grad, r64.grad, 1e-5) and parity_ok("tg_grad", tg.grad, t64.grad, 1e-5)
@@ -808,7 +811,7 @@ def test_refine_pose_and_adamw_kernels_vs_torch():
     ref = [p.clone().requires_grad_() for p in ps]
     opt = torch.optim.AdamW([{"params": [p], "lr": lr} for p, lr in zip(ref, lrs)])
     mine = [p.to(DEV).clone().requires_grad_() for p in ps]
-    fo = S.refine.FusedAdamW([{"params": p, "lr": lr} for p, lr in zip(mine, lrs)])
+    fo = S.refine.SlotAdamW([{"params": p, "lr": lr} for p, lr in zip(mine, lrs)], rows=1)
     for it in range(5):
         gs = [torch.randn(p.shape, generator=gen) for p in ps]
         for p, q, g in zip(ref, mine, gs):

@@ -124,8 +124,8 @@ def test_admit_run_retire_without_host_synchronisation():
 
 
 @pytest.mark.gpu
-def test_adamw_rows_match_one_row_calls_and_torch():
-    """Rows with different step counts and one inactive row: each active row is bit-identical to snb_adamw_step on that row alone and
+def test_adamw_rows_match_one_row_optimiser_and_torch():
+    """Rows with different step counts and one inactive row: each active row is bit-identical to a one-row SlotAdamW on that row alone and
     within 1e-6 of torch.optim.AdamW on the CPU; the inactive row and its counter are bit-unchanged; the loss history row is written."""
     R = snb().refine
     g = torch.Generator().manual_seed(5)
@@ -155,7 +155,7 @@ def test_adamw_rows_match_one_row_calls_and_torch():
             assert opt.step_t[r].item() == steps[r] and bool((history[r] == -1).all())
             continue
         one = [P[i][r].clone().to(DEV) for i in range(2)]
-        ref = R.FusedAdamW([{"params": p, "lr": lr} for p, lr in zip(one, lrs)])
+        ref = R.SlotAdamW([{"params": p, "lr": lr} for p, lr in zip(one, lrs)], rows=1)
         for i in range(2):
             one[i].grad = G[i][r].to(DEV)
             ref.m[i].copy_(M[i][r])
@@ -178,29 +178,24 @@ def test_adamw_rows_match_one_row_calls_and_torch():
 
 
 def _pose_fwd(rot, trans, jitter, jitter2, T, steps, active, err, obj_diag):
-    """snb_refine_pose_slots_fwd (steps (C,)) or, with `steps` a 0-d tensor, the shared-counter snb_refine_pose_batch_fwd."""
+    """snb_refine_pose_slots_fwd with steps (C,)."""
     from supnerf_b200 import _lib
     from supnerf_b200._lib import ptr, stream_ptr
     lib = _lib.load()
     c, s = rot.shape[0], jitter.shape[-1]
     cam = torch.empty(c, 3, 4, device=DEV)
     z, z2 = torch.empty(c, s, device=DEV), torch.empty(c, s, device=DEV)
-    if steps.dim() == 0:
-        rc = lib.snb_refine_pose_batch_fwd(ptr(rot), ptr(trans), c, 0, ptr(obj_diag), s, ptr(jitter), ptr(jitter2), ptr(steps), T, ptr(cam),
-                                           ptr(z), ptr(z2), stream_ptr())
-    else:
-        rc = lib.snb_refine_pose_slots_fwd(ptr(rot), ptr(trans), c, 0, ptr(obj_diag), s, ptr(jitter), ptr(jitter2), ptr(steps), T, ptr(active),
-                                           ptr(err), ptr(cam), ptr(z), ptr(z2), stream_ptr())
+    rc = lib.snb_refine_pose_slots_fwd(ptr(rot), ptr(trans), c, 0, ptr(obj_diag), s, ptr(jitter), ptr(jitter2), ptr(steps), T, ptr(active),
+                                       ptr(err), ptr(cam), ptr(z), ptr(z2), stream_ptr())
     assert rc == 0
     torch.cuda.synchronize()
     return cam, z, z2
 
 
 @pytest.mark.gpu
-def test_counter_guard():
+def test_slot_counter_guard():
     """The jitter tables hold T + 1 rows per slot but are passed as T rows, so an unguarded read at row T would read valid memory: an
-    active slot at counter T (or -1) gets NaN z / z2 and sets the flag; inactive, the same slot gives finite z and no flag; and the
-    shared-counter path is bit-identical to the per-slot path with equal in-range counters."""
+    active slot at counter T (or -1) gets NaN z / z2 and sets the flag; inactive, the same slot gives finite z and no flag."""
     snb()
     g = torch.Generator().manual_seed(9)
     c, T, s = 4, 5, 64
@@ -219,9 +214,6 @@ def test_counter_guard():
     err.zero_()
     _, z, z2 = _pose_fwd(rot, trans, jit, jit2, T, steps, torch.tensor([1, 0, 1, 0], dtype=torch.uint8, device=DEV), err, obj_diag)
     assert int(err.item()) == 0 and bool(torch.isfinite(z).all() and torch.isfinite(z2).all())
-    shared = _pose_fwd(rot, trans, jit, jit2, T, torch.tensor(2.0, device=DEV), None, None, obj_diag)
-    per_slot = _pose_fwd(rot, trans, jit, jit2, T, torch.full((c,), 2.0, device=DEV), None, err, obj_diag)
-    assert int(err.item()) == 0 and all(torch.equal(a, b) for a, b in zip(shared, per_slot))
 
 
 @pytest.mark.gpu
