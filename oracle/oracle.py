@@ -12,6 +12,10 @@ Parity status: PINNED.  Every function here is checked against outputs of the un
 ``tests/test_oracle_golden.py`` (runs on CPU, does not need ``/root/reference``).
 
 Citations are ``file:line`` into ``/root/reference/src``.
+
+Stated divergence: ``composite`` at S = 1.  The reference builds the last sample's 1e10 delta from ``deltas[..., :1]``, which is
+empty when a ray has one sample, so it cannot composite S = 1 at all; here the single sample is the last one (delta 1e10), as in
+the library's compositing (composite.cuh) and in ``composite_backward_closed_form``.  Every S >= 2 is unchanged.
 """
 from __future__ import annotations
 
@@ -329,7 +333,8 @@ def composite(sigmas: Tensor, rgbs: Tensor, z_vals: Tensor, white_bkgd: bool, us
     else:
         z = z_vals
     deltas = z[..., 1:] - z[..., :-1]
-    deltas = torch.cat([deltas, torch.ones_like(deltas[..., :1]) * 1e10], -1)
+    # (z[..., :1], not the reference's deltas[..., :1]: the same column for S >= 2, and S = 1 works -- see the module docstring)
+    deltas = torch.cat([deltas, torch.ones_like(z[..., :1]) * 1e10], -1)
     s = torch.relu(sigmas) if use_relu else sigmas
     alphas = 1 - torch.exp(-s * deltas)
     trans = 1 - alphas + 1e-10
@@ -380,22 +385,22 @@ def composite_backward_closed_form(sigmas, rgbs, z_vals, g_rgb, g_depth, g_acc, 
 # a9. drivers (one object / view)
 # --------------------------------------------------------------------------------------------------
 def render_rays_box(sd, K, cam_pose, obj_sz, roi, im_sz, n_samples, shapecode, texturecode, jitter,
-                    white_bkgd=True, ray_ids=None):
+                    white_bkgd=True, ray_ids=None, decoder=codenerf_decoder):
     """NeRFRenderer.render_rays, renderer.py:117-167, minus the target resize (targets are inputs,
     not renders).  ``jitter`` (N,S) replaces torch.rand_like; ``ray_ids`` replaces the numpy
-    permutation (renderer.py:139-146)."""
+    permutation (renderer.py:139-146).  ``decoder``: codenerf_decoder, or codenerf_decoder_bf16 for the bf16 mode's rounding."""
     rays_o, viewdir = get_rays(K, cam_pose, roi, uv_steps=[im_sz, im_sz])
     if ray_ids is not None:
         rays_o, viewdir = rays_o[ray_ids], viewdir[ray_ids]
     xyz, vd, z_vals, hit = prepare_sampled_rays(rays_o, viewdir, obj_sz, n_samples, jitter)
-    sigmas, rgbs = codenerf_decoder(sd, xyz, vd, shapecode, texturecode)
+    sigmas, rgbs = decoder(sd, xyz, vd, shapecode, texturecode)
     rgb, depth, acc = composite(sigmas.squeeze(-1), rgbs, z_vals, white_bkgd)
     return rgb, depth, acc, hit
 
 
 def render_rays_shell(sd, K, cam_pose, obj_diag, roi, im_sz, n_samples, shapecode, texturecode, jitter,
-                      shapenet_obj_cood=True, ray_ids=None):
-    """utils.render_rays_v2, utils.py:435-502 (sym_aug / kitti2nusc off), targets excluded."""
+                      shapenet_obj_cood=True, ray_ids=None, decoder=codenerf_decoder):
+    """utils.render_rays_v2, utils.py:435-502 (sym_aug / kitti2nusc off), targets excluded.  ``decoder`` as in render_rays_box."""
     rays_o, viewdir = get_rays(K, cam_pose, roi, uv_steps=[im_sz, im_sz])
     if ray_ids is not None:
         rays_o, viewdir = rays_o[ray_ids], viewdir[ray_ids]
@@ -406,7 +411,7 @@ def render_rays_shell(sd, K, cam_pose, obj_diag, roi, im_sz, n_samples, shapecod
     if shapenet_obj_cood:
         xyz = shapenet_swap(xyz)
         vd = shapenet_swap(vd)
-    sigmas, rgbs = codenerf_decoder(sd, xyz, vd, shapecode, texturecode)
+    sigmas, rgbs = decoder(sd, xyz, vd, shapecode, texturecode)
     rgb, depth, acc = composite(sigmas.squeeze(-1), rgbs, z_vals, white_bkgd=False)
     return rgb, depth, acc
 

@@ -47,7 +47,9 @@ def model_from_state(cls, sd, *args, **kw):
 
 
 # ------------------------------------------------------------------------------------------- compositing
-@pytest.mark.parametrize("N,S", [(1, 2), (5, 7), (1000, 37), (4096, 64), (3000, 128), (257, 200)])
+@pytest.mark.parametrize("N,S", [(1, 2), (5, 7), (1000, 37), (4096, 64), (3000, 128), (257, 200),
+                                 # the fast path with lanes left empty (8 / 16 / 32 lanes per ray) and a last warp the rays do not fill
+                                 (37, 4), (77, 12), (5, 20), (1001, 36), (133, 100), (45, 124)])
 @pytest.mark.parametrize("white", [False, True])
 def test_composite_vs_oracle(N, S, white):
     g = torch.Generator().manual_seed(N * 131 + S)
@@ -1123,3 +1125,56 @@ def test_fp32_tensor_core_mode_steps_aside_for_weights_outside_fp16_range():
     with torch.no_grad():
         m.get_parameter("shape_layer_1.0.weight")[3, 5] = 0.01      # an in-place update bumps the version: re-checked, back on the tensor cores
     assert h.weights_in_fp16_range(m._weights())
+
+
+# ------------------------------------------------------------------------------------------- counter-based jitter
+_M32 = np.uint64(0xFFFFFFFF)
+
+
+def _philox4x32_10(ctr, key):
+    """Philox4x32-10 (Salmon et al., SC'11; Random123), vectorised over numpy uint64 arrays that hold 32-bit words."""
+    c0, c1, c2, c3 = (np.asarray(c, dtype=np.uint64) for c in ctr)
+    k0, k1 = (np.asarray(k, dtype=np.uint64) for k in key)
+    for _ in range(10):
+        p0, p1 = np.uint64(0xD2511F53) * c0, np.uint64(0xCD9E8D57) * c2      # < 2^64: exact
+        c0, c1, c2, c3 = (p1 >> np.uint64(32)) ^ c1 ^ k0, p1 & _M32, (p0 >> np.uint64(32)) ^ c3 ^ k1, p0 & _M32
+        k0, k1 = (k0 + np.uint64(0x9E3779B9)) & _M32, (k1 + np.uint64(0xBB67AE85)) & _M32
+    return c0, c1, c2, c3
+
+
+def _jitter_reference(seed, ray_ids, n_samples):
+    """u[r][k] = word k % 4 of Philox4x32-10(counter (id low, id high, k / 4, 0), key (seed low, seed high)), as (x >> 8) * 2^-24."""
+    ids = np.asarray(ray_ids, dtype=np.uint64)[:, None]
+    k = np.arange(n_samples, dtype=np.uint64)[None, :]
+    seed = np.uint64(seed)
+    words = np.stack(np.broadcast_arrays(*_philox4x32_10((ids & _M32, ids >> np.uint64(32), k // np.uint64(4), np.uint64(0)),
+                                                         (seed & _M32, seed >> np.uint64(32)))), -1)
+    x = np.take_along_axis(words, np.broadcast_to((k % np.uint64(4)).astype(np.int64)[..., None], words.shape[:2] + (1,)), -1)[..., 0]
+    return torch.from_numpy(((x >> np.uint64(8)).astype(np.float64) * 2.0 ** -24).astype(np.float32))
+
+
+@pytest.mark.parametrize("S_", [1, 3, 4, 7, 64])
+def test_jitter_fill_is_philox4x32_10_bit_for_bit(S_):
+    """ops.jitter_fill (snb_jitter_fill, the ray-sharded modes' stratified jitter) against a Python Philox4x32-10 that reproduces the
+    Random123 known-answer vectors: every value bit for bit, seeds and ray ids past 2^32, and shards given by ray ids whose union is the
+    full draw."""
+    hexw = lambda ws: ["%08x" % int(w) for w in ws]   # noqa: E731
+    assert hexw(_philox4x32_10([0] * 4, [0, 0])) == ["6627e8d5", "e169c58d", "bc57ac4c", "9b00dbd8"]
+    assert hexw(_philox4x32_10([0xFFFFFFFF] * 4, [0xFFFFFFFF] * 2)) == ["408f276d", "41c83b0e", "a20bc7c6", "6d5451fd"]
+    assert hexw(_philox4x32_10([0x243f6a88, 0x85a308d3, 0x13198a2e, 0x03707344], [0xa4093822, 0x299f31d0])) == \
+        ["d16cfe09", "94fdcceb", "5001e420", "24126ea1"]
+    S = snb()
+    n = 777
+    for seed in (0, 20240611, (1 << 32) + 5, (1 << 64) - 3):
+        full = S.ops.jitter_fill(seed, n, S_, DEV)
+        assert full.shape == (n, S_) and torch.equal(full.cpu(), _jitter_reference(seed, np.arange(n), S_))
+        ids = torch.arange(n, dtype=torch.int64) + (1 << 32) - 300          # both sides of 2^32
+        ids[-5:] = torch.tensor([(1 << 40) + 1, (1 << 48) + 77, (1 << 62) + 3, (1 << 63) - 1, 12345])
+        big = S.ops.jitter_fill(seed, 0, S_, DEV, ray_ids=ids.to(DEV))
+        assert torch.equal(big.cpu(), _jitter_reference(seed, ids.numpy(), S_))
+        assert float(big.min()) >= 0.0 and float(big.max()) < 1.0
+        perm = torch.randperm(n, generator=torch.Generator().manual_seed(S_))
+        union = torch.full((n, S_), -1.0)
+        for shard in (perm[:100], perm[100:101], perm[101:]):
+            union[shard] = S.ops.jitter_fill(seed, 0, S_, DEV, ray_ids=ids[shard].to(DEV)).cpu()
+        assert torch.equal(union, big.cpu())
